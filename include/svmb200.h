@@ -171,6 +171,21 @@ int svmb200_pg_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
 int svmb200_fw_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                       int hessian, const double* q_host, const double* lb_host, const double* ub_host,
                       const double* x0_host, double eps, int64_t max_iter, double t, svmb200_pg** out);
+/* K11: SMO on the same handle type -- libsvm's solver without shrinking (working-set selection WSS2; Fan, Chen & Lin
+ * 2005) for the SVM dual WITH its equality constraint (an unregularised intercept, sklearn's SVC / SVR):
+ *     min a'Qa/2 + q'a   s.t.  sign'a = 0,  0 <= a <= ub
+ * Replaces optiml/ml/svm/smo.py (SMOClassifier, SMORegression; selection rules restated, not copied).  Starts at a = 0,
+ * stops with OPTIMAL when the maximal violating pair's gap m - M is below `tol` (or no pair is left), with STOPPED at
+ * max_iter.  sign_host: nvars values of +-1 (SVC: the labels; SVR: e = [1 (n times), -1 (n times)]); with the PLAIN
+ * layout dQ holds Q itself (SVC: y_s y_t K_st), with SVR it holds K and Q = [[K,-K],[-K,K]].  The matrix must be the
+ * whole problem on this rank (row0 = 0, nrows = n; otherwise SVMB200_ERR_ARG): there is no sharded SMO.  Then
+ * svmb200_pg_run (chunks of at most 65 536 iterations per launch, history storage grown with the iterations run),
+ * _state (x = a, g = G = Qa + q, f = objective tracked per step, ng = gap), _history (f and gap per state), _scalars
+ * ({f, gap, 0, 0, 0, 0}), _stats (passes = 0: an iteration reads two rows of Q) and _destroy apply; lockstep batches
+ * and single-process groups do not.                                                                                 */
+int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
+                       int hessian, const double* sign_host, const double* q_host, const double* ub_host, double tol,
+                       int64_t max_iter, svmb200_pg** out);
 /* Advance by at most `max_new` iterations (< 0: run to termination; 0: only evaluate the state at
  * the current callback point, i.e. f, |d| and the stopping tests).  The callback point of the
  * reference (projected_gradient.py:95-98) is reached once per iteration; the state visible after

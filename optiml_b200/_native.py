@@ -66,6 +66,7 @@ PROTOTYPES = {
     'svmb200_al_create_signed': [c_vp, c_vp, i64, i64, i64, i64, C.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, C.c_double,
                                  C.c_double, C.c_int, C.c_int, c_vp, c_vp, C.c_double, C.c_double, C.c_double,
                                  C.c_double, C.c_double, i64, C.POINTER(c_vp)],
+    'svmb200_smo_create': [c_vp, c_vp, i64, i64, i64, i64, C.c_int, c_vp, c_vp, c_vp, C.c_double, i64, C.POINTER(c_vp)],
     'svmb200_pg_run_batch': [C.POINTER(c_vp), C.c_int, C.POINTER(i64), C.POINTER(C.c_int)],
     'svmb200_matvec_multi': [c_vp, c_vp, i64, i64, C.POINTER(c_vp), C.POINTER(c_vp), C.c_int],
     'svmb200_al_multipliers': [c_vp, C.POINTER(C.c_double), c_vp, c_vp],

@@ -1,0 +1,330 @@
+// K11: SMO for the SVM dual with an unregularised intercept -- device code (included by pg.cu only).
+//
+//     min  a'Qa/2 + q'a   s.t.  y'a = 0,  0 <= a <= C          (libsvm's problem; y = label signs, or e = [1, -1] for SVR)
+//
+// libsvm's solver without shrinking (Fan, Chen & Lin 2005, working-set selection WSS2), one pair of variables per
+// iteration:
+//   i = argmax_{t in I_up} -y_t G_t  (= m),   j = argmin_{t in I_low, b_t > 0} -b_t^2 / a_t,   M = min_{t in I_low} -y_t G_t
+//   b_t = m + y_t G_t,  a_t = Q_ii + Q_tt - 2 y_i y_t Q_it (TAU if <= 0);  ties go to the larger index (libsvm's >= / <=)
+//   stop (optimal) when m - M < tol or no j exists; (stopped) at iter == max_iter
+//   two-variable step with clipping, then  G_t += Q_it da_i + Q_jt da_j  for every t.
+// An iteration needs two rows of Q (16 n bytes) and two arg-reductions over all variables: it is bound by latency, not by
+// bandwidth -- the regime of the persistent PG loop (k_persistent.cuh).  So ONE cooperative launch runs many iterations:
+//   CTA b owns the contiguous slice [b S, (b+1) S) of the variables; its alpha, G, sign, Q_tt, C and its part of row i
+//   live in shared memory for the whole launch (Q_tt read once per launch from the diagonal).
+//   phase 1  apply the previous step to the own G (Q_it from the cached row i, Q_jt streamed from row j); local
+//            candidate for i -> partial slot
+//   grid barrier
+//   phase 2  (every CTA) reduce the partials to i and m; stream the own part of row i (cached for the next phase 1);
+//            local candidate for j and local M -> partial slot
+//   grid barrier
+//   phase 3  (every CTA) reduce to j and M, stopping test (identical everywhere: all CTAs leave together), the step from
+//            the published scalars and Q_ij; the owners of i and j write their alpha; CTA 0 records history and state.
+// A published candidate carries every scalar another CTA needs (alpha, G, sign, Q_tt, C of the winner), so no CTA reads
+// another's live alpha or G; the slots are double-buffered by iteration parity (as K8's partials).  The reductions are
+// max / min under a total order (value, then index), so the result does not depend on arrival order: the solve is
+// reproducible run to run.
+// Q_st is always the element read from ROW s (Q[s][t]); the Gram matrix is not assumed to be bitwise symmetric.  Every
+// operation of the step, of G's update and of the objective is an explicit _rn intrinsic (the library is built with
+// --fmad=true): no contraction, so a NumPy restatement of the algorithm replays the whole trajectory bit for bit.
+// Layouts: PLAIN, Q itself resident (SVC: y_s y_t K_st);  SVR, M = K resident (n x n) and Q_st = e_s e_t M[s mod n][t mod n].
+#pragma once
+#include "k_persistent.cuh"   // pk_grid_barrier
+
+constexpr int SMO_NT = 256;
+constexpr int SMO_ARRAYS = 6;        // doubles of shared memory per owned variable: alpha, G, sign, Q_tt, C, Q_it
+constexpr double SMO_TAU = 1e-12;
+
+struct SmoCand {      // the winner of one CTA's slice (64 bytes)
+    double key;       // i pass: -y_t G_t;  j pass: b_t^2 / a_t  (the larger wins, ties to the larger index)
+    double idx;       // variable index (exact in a double), -1: no candidate
+    double alpha, g, y, qd, c;
+    double mlow;      // j pass: min of -y_t G_t over the slice's part of I_low (+inf if empty)
+};
+
+struct SmoArgs {
+    const double* Q;        // resident matrix, n x ld
+    long long ld, n, nvars;
+    int svr;
+    int slice;              // variables per CTA
+    double *x, *g;          // alpha and G (nvars): read at the start of a launch, written back at its end
+    const double *sgn, *ub; // sign vector and upper bounds (nvars)
+    SmoCand* cand;          // [2 parities][2 passes][grid]
+    unsigned* gbar;         // grid barrier (k_persistent.cuh)
+    PGDeviceState* st;      // f, ng = gap, iter, done, status of the last evaluated state
+    double *hist_f, *hist_gap;
+    long long hist_cap;
+    double tol;
+    long long max_iter;
+    long long k0;           // first state this launch evaluates
+    long long niter;        // steps to take unless the stopping test fires first (states k0 .. k0 + niter are evaluated)
+};
+
+// Q[s][t] as read from row s
+__device__ __forceinline__ double smo_q(const SmoArgs& a, long long s, long long t) {
+    if (!a.svr) return __ldg(a.Q + s * a.ld + t);
+    const bool s_lo = s < a.n, t_lo = t < a.n;
+    const double v = __ldg(a.Q + (s_lo ? s : s - a.n) * a.ld + (t_lo ? t : t - a.n));
+    return s_lo == t_lo ? v : -v;
+}
+
+__device__ __forceinline__ bool smo_wins(double k, double i, double bk, double bi) { return k > bk || (k == bk && i > bi); }
+
+// block-wide arg-max of (key, idx) and min of `low`; the result lands in thread 0
+__device__ __forceinline__ void smo_block_reduce(double& key, double& idx, double& low, double (*red)[SMO_NT / 32]) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ok = __shfl_xor_sync(0xffffffffu, key, o), oi = __shfl_xor_sync(0xffffffffu, idx, o);
+        const double ol = __shfl_xor_sync(0xffffffffu, low, o);
+        if (smo_wins(ok, oi, key, idx)) {
+            key = ok;
+            idx = oi;
+        }
+        low = fmin(low, ol);
+    }
+    if (lane == 0) {
+        red[0][wid] = key;
+        red[1][wid] = idx;
+        red[2][wid] = low;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < SMO_NT / 32; ++w) {
+            if (smo_wins(red[0][w], red[1][w], key, idx)) {
+                key = red[0][w];
+                idx = red[1][w];
+            }
+            low = fmin(low, red[2][w]);
+        }
+    }
+}
+
+// reduce the grid's partial slots of one pass; thread 0 copies the winner's slot (the owner of the winning index: slices
+// are contiguous, S variables each) to *out with mlow = the grid's minimum
+__device__ __forceinline__ void smo_grid_reduce(const SmoCand* slots, unsigned grid, int S, double (*red)[SMO_NT / 32],
+                                                SmoCand* out) {
+    double key = -INFINITY, idx = -1.0, low = INFINITY;
+    for (unsigned s = threadIdx.x; s < grid; s += SMO_NT) {
+        const double k = __ldcg(&slots[s].key), i = __ldcg(&slots[s].idx), l = __ldcg(&slots[s].mlow);
+        if (smo_wins(k, i, key, idx)) {
+            key = k;
+            idx = i;
+        }
+        low = fmin(low, l);
+    }
+    smo_block_reduce(key, idx, low, red);
+    if (threadIdx.x == 0) {
+        SmoCand w = {-INFINITY, -1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+        if (idx >= 0.0) {
+            const SmoCand* s = slots + (long long)idx / S;
+            w.key = key;
+            w.idx = idx;
+            w.alpha = __ldcg(&s->alpha);
+            w.g = __ldcg(&s->g);
+            w.y = __ldcg(&s->y);
+            w.qd = __ldcg(&s->qd);
+            w.c = __ldcg(&s->c);
+        }
+        w.mlow = __dadd_rn(low, 0.0);   // -0 -> +0: fmin may return either zero
+        *out = w;
+    }
+    __syncthreads();
+}
+
+__global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs a) {
+#ifndef SVMB200_HOST_EMULATION
+    extern __shared__ __align__(16) unsigned char smo_smem_raw[];
+    double* sm = reinterpret_cast<double*>(smo_smem_raw);
+#else
+    double* sm = reinterpret_cast<double*>(emu::dynamic_smem());
+#endif
+    __shared__ double red[3][SMO_NT / 32];
+    __shared__ SmoCand win_i, win_j;
+    const int tid = threadIdx.x;
+    const unsigned grid = gridDim.x;
+    const int S = a.slice;
+    double *s_alpha = sm, *s_g = sm + S, *s_y = sm + 2 * S, *s_qd = sm + 3 * S, *s_c = sm + 4 * S, *s_qi = sm + 5 * S;
+    const long long t0 = (long long)blockIdx.x * S;
+    const int len = t0 >= a.nvars ? 0 : (int)(a.nvars - t0 < S ? a.nvars - t0 : S);
+
+    for (int l = tid; l < len; l += SMO_NT) {
+        const long long t = t0 + l;
+        s_alpha[l] = a.x[t];
+        s_g[l] = a.g[t];
+        s_y[l] = a.sgn[t];
+        s_c[l] = a.ub[t];
+        s_qd[l] = smo_q(a, t, t);
+        s_qi[l] = 0.0;
+    }
+    double f = a.st->f;   // objective at state k0 (CTA 0 rewrites it only after the first grid barrier)
+    __syncthreads();
+
+    bool pending = false;          // a step whose G update phase 1 still has to apply
+    long long pj = 0;
+    double dai = 0.0, daj = 0.0;
+    for (long long e = 0;; ++e) {
+        const long long k = a.k0 + e;
+        SmoCand* slots_i = a.cand + (size_t)((k & 1) * 2) * grid;
+        SmoCand* slots_j = slots_i + grid;
+        // ================= phase 1: previous step on the own G, local candidate for i
+        double key = -INFINITY, idx = -1.0, low = INFINITY;
+        for (int l = tid; l < len; l += SMO_NT) {
+            const long long t = t0 + l;
+            double gt = s_g[l];
+            if (pending) {
+                gt = __dadd_rn(gt, __dadd_rn(__dmul_rn(s_qi[l], dai), __dmul_rn(smo_q(a, pj, t), daj)));
+                s_g[l] = gt;
+            }
+            const double y = s_y[l], al = s_alpha[l];
+            const bool up = y > 0.0 ? al < s_c[l] : al > 0.0;
+            const double v = -__dmul_rn(y, gt);
+            if (up && v >= key) {   // own indices ascend: >= keeps the larger one on ties
+                key = v;
+                idx = (double)t;
+            }
+        }
+        smo_block_reduce(key, idx, low, red);
+        if (tid == 0) {
+            SmoCand c = {key, idx, 0.0, 0.0, 0.0, 0.0, 0.0, INFINITY};
+            if (idx >= 0.0) {
+                const int l = (int)((long long)idx - t0);
+                c.alpha = s_alpha[l];
+                c.g = s_g[l];
+                c.y = s_y[l];
+                c.qd = s_qd[l];
+                c.c = s_c[l];
+            }
+            slots_i[blockIdx.x] = c;
+        }
+        pk_grid_barrier(a.gbar, grid);
+
+        // ================= phase 2: i and m; own part of row i; local candidate for j, local M
+        smo_grid_reduce(slots_i, grid, S, red, &win_i);
+        const double m = win_i.key, yi = win_i.y, qii = win_i.qd;
+        const long long i = (long long)win_i.idx;
+        key = -INFINITY;
+        idx = -1.0;
+        low = INFINITY;
+        for (int l = tid; l < len; l += SMO_NT) {
+            const long long t = t0 + l;
+            const double qit = i >= 0 ? smo_q(a, i, t) : 0.0;
+            s_qi[l] = qit;
+            const double y = s_y[l], al = s_alpha[l];
+            const bool lowset = y > 0.0 ? al > 0.0 : al < s_c[l];
+            if (lowset) {
+                const double ygt = __dmul_rn(y, s_g[l]);
+                low = fmin(low, -ygt);
+                const double b = __dadd_rn(m, ygt);
+                if (b > 0.0) {
+                    double at = __dsub_rn(__dadd_rn(qii, s_qd[l]), __dmul_rn(2.0 * yi * y, qit));
+                    if (at <= 0.0) at = SMO_TAU;
+                    const double v = __ddiv_rn(__dmul_rn(b, b), at);   // -(objective): -b^2/a is exact negation
+                    if (v >= key) {
+                        key = v;
+                        idx = (double)t;
+                    }
+                }
+            }
+        }
+        smo_block_reduce(key, idx, low, red);
+        if (tid == 0) {
+            SmoCand c = {key, idx, 0.0, 0.0, 0.0, 0.0, 0.0, low};
+            if (idx >= 0.0) {
+                const int l = (int)((long long)idx - t0);
+                c.alpha = s_alpha[l];
+                c.g = s_g[l];
+                c.y = s_y[l];
+                c.qd = s_qd[l];
+                c.c = s_c[l];
+            }
+            slots_j[blockIdx.x] = c;
+        }
+        pk_grid_barrier(a.gbar, grid);
+
+        // ================= phase 3: j and M, stopping test, the step
+        smo_grid_reduce(slots_j, grid, S, red, &win_j);
+        const long long j = (long long)win_j.idx;
+        const double gap = __dsub_rn(m, win_j.mlow);
+        if (blockIdx.x == 0 && tid == 0) {
+            if (k < a.hist_cap) {
+                a.hist_f[k] = f;
+                a.hist_gap[k] = gap;
+            }
+            a.st->f = f;
+            a.st->ng = gap;
+            a.st->iter = k;
+        }
+        int stop = 0;
+        if (j < 0 || gap < a.tol) stop = SVMB200_STATUS_OPTIMAL;
+        else if (k >= a.max_iter) stop = SVMB200_STATUS_STOPPED;
+        if (stop) {
+            if (blockIdx.x == 0 && tid == 0) {
+                a.st->status = stop;
+                __threadfence();
+                a.st->done = 1;
+            }
+            break;
+        }
+        if (e == a.niter) break;   // the budget ends at an evaluated state
+        // libsvm's two-variable step on the signed Q (Q_ij = y_i y_j K_ij for SVC).  y_i != y_j: the step keeps
+        // a_i - a_j, quad = Q_ii + Q_jj + 2 Q_ij;  y_i == y_j: it keeps a_i + a_j, quad = Q_ii + Q_jj - 2 Q_ij.  With
+        // Q_ij = y_i y_j K_ij both are K_ii + K_jj - 2 K_ij, the curvature along the feasible direction.
+        const double qjj = win_j.qd, gi = win_i.g, gj = win_j.g, ci = win_i.c, cj = win_j.c;
+        const double qij = smo_q(a, i, j);
+        const double ai0 = win_i.alpha, aj0 = win_j.alpha;
+        double ai = ai0, aj = aj0;
+        if (yi != win_j.y) {
+            double quad = __dadd_rn(__dadd_rn(qii, qjj), __dmul_rn(2.0, qij));
+            if (quad <= 0.0) quad = SMO_TAU;
+            const double delta = __ddiv_rn(__dsub_rn(-gi, gj), quad);
+            const double diff = __dsub_rn(ai, aj);
+            ai = __dadd_rn(ai, delta);
+            aj = __dadd_rn(aj, delta);
+            if (diff > 0.0) {
+                if (aj < 0.0) { aj = 0.0; ai = diff; }
+            } else {
+                if (ai < 0.0) { ai = 0.0; aj = -diff; }
+            }
+            if (diff > __dsub_rn(ci, cj)) {
+                if (ai > ci) { ai = ci; aj = __dsub_rn(ci, diff); }
+            } else {
+                if (aj > cj) { aj = cj; ai = __dadd_rn(cj, diff); }
+            }
+        } else {
+            double quad = __dsub_rn(__dadd_rn(qii, qjj), __dmul_rn(2.0, qij));
+            if (quad <= 0.0) quad = SMO_TAU;
+            const double delta = __ddiv_rn(__dsub_rn(gi, gj), quad);
+            const double sum = __dadd_rn(ai, aj);
+            ai = __dsub_rn(ai, delta);
+            aj = __dadd_rn(aj, delta);
+            if (sum > ci) {
+                if (ai > ci) { ai = ci; aj = __dsub_rn(sum, ci); }
+            } else {
+                if (aj < 0.0) { aj = 0.0; ai = sum; }
+            }
+            if (sum > cj) {
+                if (aj > cj) { aj = cj; ai = __dsub_rn(sum, cj); }
+            } else {
+                if (ai < 0.0) { ai = 0.0; aj = sum; }
+            }
+        }
+        dai = __dsub_rn(ai, ai0);
+        daj = __dsub_rn(aj, aj0);
+        // f += da_i G_i + da_j G_j + (da_i^2 Q_ii + da_j^2 Q_jj) / 2 + da_i da_j Q_ij   (old G)
+        const double lin = __dadd_rn(__dmul_rn(dai, gi), __dmul_rn(daj, gj));
+        const double sq = __dadd_rn(__dmul_rn(__dmul_rn(dai, dai), qii), __dmul_rn(__dmul_rn(daj, daj), qjj));
+        f = __dadd_rn(f, __dadd_rn(__dadd_rn(lin, __dmul_rn(0.5, sq)), __dmul_rn(__dmul_rn(dai, daj), qij)));
+        if (tid == 0) {
+            if (i >= t0 && i < t0 + len) s_alpha[i - t0] = ai;
+            if (j >= t0 && j < t0 + len) s_alpha[j - t0] = aj;
+        }
+        pending = true;
+        pj = j;
+        __syncthreads();   // alpha of i / j in place for the next phase 1
+    }
+    for (int l = tid; l < len; l += SMO_NT) {
+        a.x[t0 + l] = s_alpha[l];
+        a.g[t0 + l] = s_g[l];
+    }
+}

@@ -17,6 +17,7 @@
 #include "k2_symv.cuh"     // K2s: one pass over the upper triangle of a symmetric matrix (opt-in)
 #include "k3_vector.cuh"   // K3 vector phases and kernel entry points (device code)
 #include "k_persistent.cuh"  // the whole loop in one cooperative kernel, matrix in shared memory (small problems)
+#include "k_smo.cuh"         // K11: SMO with the equality constraint, one cooperative kernel for many iterations
 #include <math.h>
 #include <stdlib.h>
 
@@ -477,7 +478,7 @@ struct svmb200_pg {
     const double* dQ = nullptr;
     int64_t n = 0, ld = 0, row0 = 0, nrows = 0, nvars = 0, rows_per_rank = 0;
     int svr = 0;
-    int solver = 0;      // 0: projected gradient, 1: Frank-Wolfe, 2: augmented Lagrangian + stochastic rule
+    int solver = 0;      // 0: projected gradient, 1: Frank-Wolfe, 2: augmented Lagrangian + stochastic rule, 3: SMO
     ALArgs al = {};      // solver 2 only
     double fw_t = 0.0;   // Frank-Wolfe stabilisation parameter
     double eps = 1e-6;
@@ -510,6 +511,10 @@ struct svmb200_pg {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // the context's solver pair (svmb200_timer_* has its own)
     void* slab = nullptr;        // all device buffers below live in this slab
     bool slab_private = false;   // true: allocated for this solver only (the context's slab was busy)
+    // SMO (solver 3): grid and slice of its launches, candidate slots, history grown with the iterations actually run
+    int smo_grid = 0, smo_slice = 0;
+    SmoCand* smo_cand = nullptr;
+    double* smo_hist = nullptr;  // hist_f | hist_ng, hist_cap each
 };
 
 constexpr size_t POLL_SLOT_BYTES = 128;  // {PGDeviceState, ..., int fault} per poll slot of the pinned block
@@ -664,6 +669,7 @@ extern "C" int svmb200_pg_destroy(svmb200_pg* pg) {
     if (pg->ctx) {
         cudaSetDevice(pg->ctx->device);
         cudaStreamSynchronize(pg->ctx->stream);
+        if (pg->smo_hist) cudaFree(pg->smo_hist);
         if (pg->slab_private) {
             if (pg->slab) cudaFree(pg->slab);
             if (pg->pinned) cudaFreeHost(pg->pinned);
@@ -1210,10 +1216,12 @@ static int run_many(svmb200_pg* const* pgs, int count, int64_t max_new) {
     return SVMB200_OK;
 }
 
+static int smo_run(svmb200_pg* pg, int64_t max_new);
+
 extern "C" int svmb200_pg_run(svmb200_pg* pg, int64_t max_new, int64_t* iter, int* status) {
     SVM_CHECK_ARG(pg != nullptr, "null solver");
     SVM_CHECK_ARG(!pg->deferred_start, "a solver of a single-process group runs through svmb200_pg_run_group");
-    SVM_TRY(run_many(&pg, 1, max_new));
+    SVM_TRY(pg->solver == 3 ? smo_run(pg, max_new) : run_many(&pg, 1, max_new));
     if (iter) *iter = pg->st_host->iter;
     if (status) *status = pg->st_host->done ? pg->st_host->status : SVMB200_STATUS_UNKNOWN;
     return SVMB200_OK;
@@ -1225,6 +1233,7 @@ static int check_group(svmb200_pg* const* pgs, int count) {
     for (int r = 0; r < count; ++r) {
         const svmb200_pg* p = pgs[r];
         SVM_CHECK_ARG(p != nullptr && p->ctx != nullptr, "null solver");
+        SVM_CHECK_ARG(p->solver != 3, "an SMO solver runs through svmb200_pg_run");
         SVM_CHECK_ARG(p->ctx->local_group && p->ctx->nranks == count && p->ctx->rank == r,
                       "pass one solver per rank of the single-process group, in rank order");
         SVM_CHECK_ARG(p->n == pgs[0]->n && p->solver == pgs[0]->solver && p->max_iter == pgs[0]->max_iter &&
@@ -1365,6 +1374,7 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
     for (int b = 0; b < count; ++b) {
         const svmb200_pg* p = pgs[b];
         SVM_CHECK_ARG(p != nullptr, "null solver");
+        SVM_CHECK_ARG(p->solver != 3, "SMO solvers have no lockstep batch: run them one by one");
         SVM_CHECK_ARG(p->ctx == p0->ctx && p->dQ == p0->dQ && p->n == p0->n && p->ld == p0->ld && p->row0 == p0->row0 &&
                           p->nrows == p0->nrows && p->svr == p0->svr,
                       "the solvers of a batch must share the resident matrix, its shard and its layout");
@@ -1606,6 +1616,204 @@ extern "C" int svmb200_al_multipliers(svmb200_pg* pg, double* mu, double* lam_lb
     if (lam_ub_host) SVM_CUDA(cudaMemcpyAsync(lam_ub_host, pg->al.lam_ub, nv, cudaMemcpyDeviceToHost, s));
     SVM_CUDA(cudaStreamSynchronize(s));
     if (mu) *mu = pg->st_host->mu;
+    return SVMB200_OK;
+}
+
+// ------------------------------------------------------------------------------------------ K11: SMO (k_smo.cuh)
+// libsvm's problem  min a'Qa/2 + q'a  s.t.  y'a = 0, 0 <= a <= ub  on the resident matrix.  One cooperative launch runs up
+// to SMO_CHUNK iterations with the variables in the shared memory of its CTAs; the host polls the state between launches.
+// The grid is one CTA per SM, but no CTA takes fewer than SMO_MIN_SLICE variables: an iteration costs two grid barriers plus
+// the slice's work, and a barrier over fewer CTAs is cheaper (profiles/smo_grid_sweep.jsonl, B200: C1, 2 000 variables,
+// 8.63 us per iteration on 148 CTAs, 7.77 on 16; C4, 50 000 variables, 12.4 us on 148, 12.2 on 74, 16.2 on 37).
+// SVMB200_SMO_GRID overrides it (sweeps; tests on the host emulation); the grid grows when the slices would not fit the
+// shared memory.
+constexpr int64_t SMO_CHUNK = 65536;
+constexpr int64_t SMO_MIN_SLICE = 128;
+constexpr size_t SMO_SMEM_MAX = 221 * 1024;
+constexpr int64_t SMO_SLICE_MAX = (int64_t)(SMO_SMEM_MAX / (SMO_ARRAYS * sizeof(double)));
+
+static size_t smo_smem_bytes(const svmb200_pg* pg) { return (size_t)pg->smo_slice * SMO_ARRAYS * sizeof(double); }
+
+extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
+                                  int hessian, const double* sign_host, const double* q_host, const double* ub_host,
+                                  double tol, int64_t max_iter, svmb200_pg** out) {
+    SVM_TRY(svm_use(ctx));
+    SVM_CHECK_ARG(out != nullptr, "out is null");
+    *out = nullptr;
+    SVM_CHECK_ARG(dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
+    SVM_CHECK_ARG(n > 1, "Q is too small");
+    SVM_CHECK_ARG(ld >= n && ld % 2 == 0, "ld must be >= n and even");
+    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
+    SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
+    SVM_CHECK_ARG(max_iter > 0, "max_iter must be > 0");
+    SVM_CHECK_ARG(tol >= 0.0, "tol must be >= 0");
+    const int64_t nvars = hessian == SVMB200_HESSIAN_SVR ? 2 * n : n;
+    SVM_CHECK_ARG(nvars < (1ll << 31), "too many variables");
+    for (int64_t t = 0; t < nvars; ++t) {
+        SVM_CHECK_ARG(sign_host[t] == 1.0 || sign_host[t] == -1.0, "signs must be +-1");
+        SVM_CHECK_ARG(ub_host[t] > 0.0 && ub_host[t] < INFINITY, "upper bounds must be finite and > 0");
+    }
+    int grid = ctx->sm_count > 0 ? ctx->sm_count : 1;
+    if ((int64_t)grid * SMO_MIN_SLICE > nvars) grid = (int)((nvars + SMO_MIN_SLICE - 1) / SMO_MIN_SLICE);
+    if (const char* ev = getenv("SVMB200_SMO_GRID")) grid = atoi(ev);
+    SVM_CHECK_ARG(grid >= 1, "SVMB200_SMO_GRID must be >= 1");
+    int64_t slice = (nvars + grid - 1) / grid;
+    if (slice > SMO_SLICE_MAX) slice = SMO_SLICE_MAX;
+    svmb200_pg* pg = new svmb200_pg();
+    pg->ctx = ctx;
+    pg->dQ = dQ;
+    pg->n = n;
+    pg->ld = ld;
+    pg->row0 = row0;
+    pg->nrows = nrows;
+    pg->svr = hessian == SVMB200_HESSIAN_SVR;
+    pg->nvars = nvars;
+    pg->rows_per_rank = n;
+    pg->solver = 3;
+    pg->eps = tol;
+    pg->max_iter = max_iter;
+    pg->smo_slice = (int)slice;
+    pg->smo_grid = (int)((nvars + slice - 1) / slice);
+    pg->slab_private = true;
+    auto fail = [&](int code) {
+        svmb200_pg_destroy(pg);
+        return code;
+    };
+#define SMO_CUDA(call)                                                                                 \
+    do {                                                                                               \
+        cudaError_t e__ = (call);                                                                      \
+        if (e__ != cudaSuccess) {                                                                      \
+            svmb200_set_error("%s:%d %s failed: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e__)); \
+            return fail(SVMB200_ERR_CUDA);                                                             \
+        }                                                                                              \
+    } while (0)
+#ifndef SVMB200_HOST_EMULATION
+    {
+        // a cooperative grid must be co-resident
+        static bool configured[64] = {};
+        const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
+        if (!configured[dev]) {
+            SMO_CUDA(cudaFuncSetAttribute(smo_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMO_SMEM_MAX));
+            configured[dev] = true;
+        }
+        int per_sm = 0;
+        SMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, smo_persistent_kernel, SMO_NT, smo_smem_bytes(pg)));
+        if ((long long)per_sm * ctx->sm_count < pg->smo_grid) {
+            svmb200_set_error("SMO: %d CTAs of %zu bytes of shared memory cannot be co-resident", pg->smo_grid, smo_smem_bytes(pg));
+            return fail(SVMB200_ERR_ARG);
+        }
+    }
+#endif
+    // one private slab: alpha, G, signs, ub (nvars each) | candidate slots | state
+    auto up = [](size_t b) { return (b + 255) & ~size_t(255); };
+    const size_t nv = (size_t)nvars * sizeof(double), sz_nv = up(nv);
+    const size_t sz_cand = up((size_t)4 * pg->smo_grid * sizeof(SmoCand));
+    SMO_CUDA(cudaMalloc(&pg->slab, 4 * sz_nv + sz_cand + up(sizeof(PGDeviceState))));
+    SMO_CUDA(cudaMallocHost(&pg->pinned, 256));
+    SMO_CUDA(cudaEventCreate(&pg->ev0));
+    SMO_CUDA(cudaEventCreate(&pg->ev1));
+    for (cudaEvent_t& e : pg->ev_poll) SMO_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    pg->st_host = reinterpret_cast<PGDeviceState*>(pg->pinned);
+    unsigned char* base = static_cast<unsigned char*>(pg->slab);
+    pg->x = reinterpret_cast<double*>(base);
+    pg->g = reinterpret_cast<double*>(base + sz_nv);
+    pg->sgn = reinterpret_cast<double*>(base + 2 * sz_nv);
+    pg->ub = reinterpret_cast<double*>(base + 3 * sz_nv);
+    pg->smo_cand = reinterpret_cast<SmoCand*>(base + 4 * sz_nv);
+    pg->st = reinterpret_cast<PGDeviceState*>(base + 4 * sz_nv + sz_cand);
+    // start: alpha = 0, G = q
+    cudaStream_t s = ctx->stream;
+    SMO_CUDA(cudaMemsetAsync(pg->x, 0, nv, s));
+    SMO_CUDA(cudaMemcpyAsync(pg->g, q_host, nv, cudaMemcpyHostToDevice, s));
+    SMO_CUDA(cudaMemcpyAsync(pg->sgn, sign_host, nv, cudaMemcpyHostToDevice, s));
+    SMO_CUDA(cudaMemcpyAsync(pg->ub, ub_host, nv, cudaMemcpyHostToDevice, s));
+    SMO_CUDA(cudaMemsetAsync(pg->smo_cand, 0, sz_cand, s));
+    SMO_CUDA(cudaMemsetAsync(pg->st, 0, sizeof(PGDeviceState), s));
+    if (!ctx->gbar) {
+        SMO_CUDA(cudaMalloc(&ctx->gbar, 256));
+        SMO_CUDA(cudaMemsetAsync(ctx->gbar, 0, 256, s));
+    }
+    SMO_CUDA(cudaStreamSynchronize(s));   // the host arrays belong to the caller
+#undef SMO_CUDA
+    pg->k_next = 0;
+    *out = pg;
+    return SVMB200_OK;
+}
+
+// history buffers for states 0 .. need - 1: grown geometrically with the iterations actually run (max_iter may be 10^7)
+static int smo_hist_reserve(svmb200_pg* pg, int64_t need) {
+    if (need <= pg->hist_cap) return SVMB200_OK;
+    int64_t cap = pg->hist_cap * 2 > need ? pg->hist_cap * 2 : need;
+    if (cap < 1024) cap = 1024;
+    if (cap > pg->max_iter + 1) cap = pg->max_iter + 1;
+    cudaStream_t s = pg->ctx->stream;
+    double* h = nullptr;
+    SVM_CUDA(cudaMalloc(&h, 2 * (size_t)cap * sizeof(double)));
+    if (pg->smo_hist) {
+        SVM_CUDA(cudaMemcpyAsync(h, pg->hist_f, (size_t)pg->hist_cap * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        SVM_CUDA(cudaMemcpyAsync(h + cap, pg->hist_ng, (size_t)pg->hist_cap * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        SVM_CUDA(cudaStreamSynchronize(s));
+        SVM_CUDA(cudaFree(pg->smo_hist));
+    }
+    pg->smo_hist = h;
+    pg->hist_f = h;
+    pg->hist_ng = h + cap;
+    pg->hist_cap = cap;
+    return SVMB200_OK;
+}
+
+// evaluate states k_next .. k_next + niter, stepping between them, unless the stopping test fires first
+static int smo_launch(svmb200_pg* pg, int64_t niter) {
+    SmoArgs a;
+    a.Q = pg->dQ;
+    a.ld = pg->ld;
+    a.n = pg->n;
+    a.nvars = pg->nvars;
+    a.svr = pg->svr;
+    a.slice = pg->smo_slice;
+    a.x = pg->x;
+    a.g = pg->g;
+    a.sgn = pg->sgn;
+    a.ub = pg->ub;
+    a.cand = pg->smo_cand;
+    a.gbar = pg->ctx->gbar;
+    a.st = pg->st;
+    a.hist_f = pg->hist_f;
+    a.hist_gap = pg->hist_ng;
+    a.hist_cap = pg->hist_cap;
+    a.tol = pg->eps;
+    a.max_iter = pg->max_iter;
+    a.k0 = pg->k_next;
+    a.niter = niter;
+    SVM_CUDA(svm_launch_cooperative(smo_persistent_kernel, dim3((unsigned)pg->smo_grid), dim3(SMO_NT), smo_smem_bytes(pg),
+                                    pg->ctx->stream, a));
+    pg->ctx->launches++;
+    return SVMB200_OK;
+}
+
+static int smo_run(svmb200_pg* pg, int64_t max_new) {
+    svmb200_ctx* ctx = pg->ctx;
+    SVM_TRY(svm_use(ctx));
+    pg->last_passes = 0;   // no full pass over Q: an iteration reads two rows
+    pg->last_samples = 0;
+    pg->last_ms = pg->last_mv_ms = pg->last_comm_ms = pg->last_vec_ms = 0.f;
+    SVM_CUDA(cudaEventRecord(pg->ev0, ctx->stream));
+    if (!pg->finished) {
+        int64_t budget = pg->max_iter - pg->k_next;
+        if (max_new >= 0 && max_new < budget) budget = max_new;
+        do {   // at least one launch: max_new = 0 evaluates the current state
+            const int64_t nb = budget < SMO_CHUNK ? budget : SMO_CHUNK;
+            SVM_TRY(smo_hist_reserve(pg, pg->k_next + nb + 1));
+            SVM_TRY(smo_launch(pg, nb));
+            SVM_TRY(poll_enqueue(pg, 0));
+            SVM_TRY(poll_wait(pg, 0));
+            pg->k_next = pg->finished ? pg->st_host->iter : pg->k_next + nb;
+            budget -= nb;
+        } while (budget > 0 && !pg->finished);
+    }
+    SVM_CUDA(cudaEventRecord(pg->ev1, ctx->stream));
+    SVM_CUDA(cudaEventSynchronize(pg->ev1));
+    SVM_CUDA(cudaEventElapsedTime(&pg->last_ms, pg->ev0, pg->ev1));
     return SVMB200_OK;
 }
 

@@ -24,6 +24,7 @@ from sklearn.base import clone
 from sklearn.preprocessing import LabelBinarizer
 
 from .svm._base import SVC, SVR
+from .svm.smo import SMO
 from .svm.kernels import _dense_f64
 from ..opti.batch import minimize_batch
 
@@ -41,7 +42,8 @@ def fit_shared_gram(estimator, X, targets):
     clones = [clone(estimator) for _ in targets]
     X, _ = _dense_f64(X, None, finite=False)  # the all-finite test runs on the device copy (_build_hessian)
     head = clones[0]
-    head._bcqp_solver_class()  # raises for the branches outside the dual path before any device work
+    if head._bcqp_solver_class() is SMO:  # (raises for the branches outside the dual path before any device work)
+        raise NotImplementedError("optimizer='smo' has no lockstep batch: fit the clones one after the other")
     # K1 once: M = K + bias without label signs (SVC: the solvers apply them; SVR: the block signs are implicit)
     shared = head._build_hessian(X, None, 'svr' if isinstance(estimator, SVR) else 'plain', None, head._bias())
     gram_s = head.fit_times_['gram_s']
@@ -75,10 +77,10 @@ def _lockstep_capable(estimator, n_samples=None):
         if group is not None and group.wants(int(n_samples)):
             return False
     try:
-        estimator._bcqp_solver_class()
+        solver_cls = estimator._bcqp_solver_class()
     except (NotImplementedError, TypeError):
         return False
-    return True
+    return solver_cls is not SMO   # no lockstep SMO batch: sklearn's own fit, one clone after the other
 
 
 class OneVsRestClassifier(_skmc.OneVsRestClassifier):

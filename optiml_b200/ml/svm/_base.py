@@ -1,10 +1,12 @@
 """sklearn-compatible SVM estimators for the dual, box-constrained formulation, trained on the GPU.
 
 Host mirror of optiml/ml/svm/_base.py restricted to the branch
-``dual=True, reg_intercept=True, loss in {hinge, epsilon_insensitive}, optimizer=<BCQP solver>``:
+``dual=True, reg_intercept=True, loss in {hinge, epsilon_insensitive}, optimizer=<BCQP solver>``,
+its augmented-Lagrangian relaxation (``optimizer=<StochasticOptimizer>``) and SMO for the dual with
+its equality constraint (``optimizer='smo', reg_intercept=False``, ml/svm/smo.py):
 same constructor keywords (sklearn ``clone``/``get_params`` work), same validation errors, same
-fitted attributes.  Every other branch of the reference (primal losses, SMO, string QP solvers,
-Lagrangian duals) raises ``NotImplementedError`` -- they are different algorithms and out of scope.
+fitted attributes.  Every other branch of the reference (primal losses, other string QP solvers,
+plain Lagrangian duals) raises ``NotImplementedError`` -- they are different algorithms and out of scope.
 
 Where the reference builds K, Q = K o yy' + yy' and three more n x n temporaries on the host
 (ml/svm/_base.py:552-554, 628; opti/_base.py:243), here the Hessian is produced directly in HBM by
@@ -19,13 +21,14 @@ from sklearn.exceptions import ConvergenceWarning
 from sklearn.preprocessing import LabelBinarizer
 
 from .kernels import gaussian, Kernel, LinearKernel, _dense_f64, gather_rows
+from .smo import SMO
 from .losses import (squared_hinge, squared_epsilon_insensitive, Hinge, SquaredHinge, EpsilonInsensitive,
                      SquaredEpsilonInsensitive)
 from ... import _native as N
 from ...opti import Optimizer, Quadratic
 from ...opti.constrained import AugmentedLagrangianQuadratic, BoxConstrainedQuadraticOptimizer, ProjectedGradient
 from ...opti.unconstrained.stochastic import StochasticOptimizer, StochasticMomentumOptimizer
-from ...runtime import DeviceHessian, DeviceMatrix, GroupHessian, default_context, make_hessian
+from ...runtime import DeviceHessian, DeviceMatrix, GroupHessian, default_context, make_hessian, would_shard
 
 _SCOPE = ('optiml_b200 implements the dual formulation solved by a BoxConstrainedQuadraticOptimizer '
           '(ProjectedGradient, FrankWolfe; reg_intercept=True) or, as its augmented-Lagrangian relaxation, by a '
@@ -111,12 +114,21 @@ class SVM(BaseEstimator):
     # ------------------------------------------------------------------ shared pieces of fit
     def _bcqp_solver_class(self):
         """The solver class to instantiate; mirrors the dispatch of ml/svm/_base.py:559-725.  A
-        ``StochasticOptimizer`` subclass selects the augmented-Lagrangian relaxation (:638-723)."""
+        ``StochasticOptimizer`` subclass selects the augmented-Lagrangian relaxation (:638-723), ``'smo'`` the SMO
+        solver of the problem with its equality constraint (ml/svm/smo.py)."""
         opt = self.optimizer
         if isinstance(opt, (BoxConstrainedQuadraticOptimizer, StochasticOptimizer)):
             opt = type(opt)  # refit of an estimator whose ``optimizer`` was replaced by the fitted instance
+        if isinstance(opt, SMO):
+            opt = 'smo'
         if not self.dual:
             raise NotImplementedError(_SCOPE.format('dual=False (primal formulation)'))
+        if isinstance(opt, str) and opt == 'smo':
+            if self.reg_intercept:
+                raise NotImplementedError("optimizer='smo' solves the dual with the equality constraint of an "
+                                          "unregularised intercept (reg_intercept=False); with reg_intercept=True there "
+                                          "is no such constraint: use ProjectedGradient or FrankWolfe")
+            return SMO
         if isinstance(opt, str) or opt is None:
             raise NotImplementedError(_SCOPE.format(f'optimizer={opt!r}'))
         if isinstance(opt, type) and issubclass(opt, StochasticOptimizer):
@@ -131,6 +143,11 @@ class SVM(BaseEstimator):
     def _make_solver(self, solver_cls, hessian, q, ub, eq_row):
         """The selected solver, ready to run, on  min x'Qx/2 + q'x : 0 <= x <= ub (, eq_row'x = 0 when the intercept
         is not regularised); sets ``self.obj`` like ml/svm/_base.py:628-725."""
+        if solver_cls is SMO:
+            # no callback: for a string optimizer there is no train_loss_history (SVM.__init__); the histories stay
+            # on the solver
+            self.obj = Quadratic(hessian, q)
+            return SMO(quad=self.obj, y=eq_row, C=ub, tol=self.tol, max_iter=self.max_iter, verbose=self.verbose)
         if issubclass(solver_cls, BoxConstrainedQuadraticOptimizer):
             self.obj = Quadratic(hessian, q)
             solver = solver_cls(quad=self.obj, ub=ub, tol=self.tol, max_iter=self.max_iter,
@@ -153,8 +170,15 @@ class SVM(BaseEstimator):
         return solver
 
     def _after_solver(self, solver):
-        if isinstance(solver, StochasticOptimizer) and solver.status == 'stopped':  # ml/svm/_base.py:715-717
+        if isinstance(solver, (StochasticOptimizer, SMO)) and solver.status == 'stopped':  # ml/svm/_base.py:715-717
             warnings.warn('max_iter reached but the optimization has not converged yet', ConvergenceWarning)
+
+    @staticmethod
+    def _check_solver_scope(solver_cls, n):
+        """SMO holds the whole Hessian on one GPU: refuse, before any device work, a fit whose matrix would be sharded."""
+        if solver_cls is SMO and would_shard(n):
+            raise NotImplementedError("optimizer='smo' runs on one GPU: this fit would shard its Hessian over several "
+                                      "(torchrun world > 1, or a device group)")
 
     def _bias(self):
         """The Hessian carries the rank-one term yy' (SVC) / ee' (SVR) only when the intercept is regularised
@@ -320,6 +344,7 @@ class SVC(ClassifierMixin, SVM):
                              'to train a model over more than two labels')
         y = _binarize(self.lb, y)
         solver_cls = self._bcqp_solver_class()
+        self._check_solver_scope(solver_cls, len(y))
         if self.loss == SquaredHinge:
             raise NotImplementedError  # ml/svm/_base.py:771-774
         if self.loss != Hinge:
@@ -354,6 +379,9 @@ class SVC(ClassifierMixin, SVM):
         self.dual_coef_ = alphas * sv_y
         if isinstance(self.kernel, LinearKernel):
             self.coef_ = np.dot(self.dual_coef_, self.support_vectors_)
+        if isinstance(self.optimizer, SMO):
+            self.intercept_ = -self.optimizer.rho   # libsvm's intercept from the final alpha and G
+            return self
         # K5: sum_m dual_coef_m K[n, m] for every n from ONE masked pass over the resident
         # Q = s_n s_m (K + bias):  s_n (Q beta)_n = sum_m dual_coef_m K[n, m] + bias sum_m dual_coef_m
         v = self.obj.device_hessian().product(np.where(sv, self.alphas_, 0.))
@@ -404,6 +432,7 @@ class SVR(RegressorMixin, SVM):
             raise ValueError('use sklearn.multioutput.MultiOutputRegressor '
                              'to train a model over more than one target')
         solver_cls = self._bcqp_solver_class()
+        self._check_solver_scope(solver_cls, len(y))
         if self.loss == SquaredEpsilonInsensitive:
             raise NotImplementedError  # ml/svm/_base.py:1325-1328
         if self.loss != EpsilonInsensitive:
@@ -441,6 +470,9 @@ class SVR(RegressorMixin, SVM):
         self.dual_coef_ = alphas_p[sv] - alphas_n[sv]
         if isinstance(self.kernel, LinearKernel):
             self.coef_ = np.dot(self.dual_coef_, self.support_vectors_)
+        if isinstance(self.optimizer, SMO):
+            self.intercept_ = -self.optimizer.rho
+            return self
         beta = np.where(sv, alphas_p - alphas_n, 0.)
         v = self.obj.device_hessian().product(np.concatenate((beta, np.zeros(n))))[:n]  # (K + bias) beta
         k_dot = v[sv] - bias * np.sum(self.dual_coef_)

@@ -1,0 +1,90 @@
+"""Sequential minimal optimization for the SVM dual with its equality constraint, run on the GPU.
+
+Where the reference keeps its SMO (optiml/ml/svm/smo.py: SMOClassifier, SMORegression) this module keeps the host mirror
+of K11 (csrc/k_smo.cuh): libsvm's solver without shrinking (Fan, Chen & Lin 2005, working-set selection WSS2) for
+
+    min a'Qa/2 + q'a   s.t.  y'a = 0,  0 <= a <= C
+
+-- the problem ``sklearn.svm.SVC`` / ``SVR`` solve, i.e. an unregularised intercept.  The reference's own selection rules
+(Platt / Keerthi) are not reproduced: the algorithm is the one csrc/k_smo.cuh documents.  The estimators reach it with
+``optimizer='smo'`` (and ``reg_intercept=False``).
+"""
+import ctypes as C
+
+import numpy as np
+
+from ... import _native as N
+from ...opti import Optimizer, Quadratic
+from ...opti.constrained._device_loop import DeviceLoopMixin
+
+
+def calculate_rho(alpha, G, y, C):
+    """libsvm's Solver::calculate_rho: the mean of y_t G_t over the free variables (0 < alpha_t < C_t); without any, the
+    middle of the interval the KKT conditions leave.  The decision function's intercept is -rho."""
+    yG = y * G
+    free = (alpha > 0) & (alpha < C)
+    if np.any(free):
+        return float(np.sum(yG[free]) / np.count_nonzero(free))
+    at_lo, at_hi = alpha <= 0, alpha >= C
+    ub_set = ((y > 0) & at_lo) | ((y < 0) & at_hi)
+    lb_set = ((y > 0) & at_hi) | ((y < 0) & at_lo)
+    ub = np.min(yG[ub_set]) if np.any(ub_set) else np.inf
+    lb = np.max(yG[lb_set]) if np.any(lb_set) else -np.inf
+    return float((ub + lb) / 2)
+
+
+class SMO(DeviceLoopMixin, Optimizer):
+    """``min x'Qx/2 + q'x : y'x = 0, 0 <= x <= C`` by SMO on the resident Hessian of ``quad`` (the whole matrix on one GPU).
+
+    ``y``: the sign row of the equality constraint (+-1: the labels for SVC, ``[1, ..., -1, ...]`` for SVR); ``C``: the
+    upper bounds (a scalar or one per variable); ``tol``: stop when the maximal violating pair's gap m - M drops below it.
+    After ``minimize``: ``x`` (alpha), ``g_x`` (G = Qx + q), ``f_x`` (= sum x_t (G_t + q_t) / 2), ``iter``, ``status``
+    ('optimal' or 'stopped'), ``gap``, ``f_hist`` / ``gap_hist`` (one entry per evaluated state 0 .. iter) and ``rho``
+    (libsvm's; the intercept is -rho)."""
+
+    _verbose_header = 'iter\t cost\t\t gap'
+
+    def __init__(self, quad, y, C, tol=1e-3, max_iter=1000, callback=None, callback_args=(), verbose=False):
+        if not isinstance(quad, Quadratic):
+            raise TypeError(f'{quad} is not an allowed quadratic function')
+        n = quad.ndim
+        y = np.asarray(y, dtype=float).ravel()
+        if y.size != n or not np.all(np.abs(y) == 1):
+            raise ValueError('y must hold one sign (+-1) per variable')
+        C = np.broadcast_to(np.asarray(C, dtype=float), (n,)).copy()
+        if not np.all(C > 0):
+            raise ValueError('C must be > 0')
+        if not tol >= 0:
+            raise ValueError('tol must be >= 0')
+        super(SMO, self).__init__(f=quad, x=np.zeros(n), eps=tol, tol=tol, max_iter=max_iter, callback=callback,
+                                  callback_args=callback_args, verbose=verbose)
+        self.y, self.ub = y, C
+        self.gap, self.rho = np.nan, np.nan
+
+    def _create(self, profile=False):
+        H = self.f.device_hessian()
+        if len(H.shards()) != 1 or H.nrows != H.n:
+            raise NotImplementedError('SMO runs on one GPU: the Hessian must not be sharded')
+        if H.signs is not None:
+            raise NotImplementedError('SMO reads the signed matrix itself: signed views of a shared matrix are not supported')
+        n = H.nvars
+        layout = N.HESSIAN_SVR if H.layout == 'svr' else N.HESSIAN_PLAIN
+        q, y, ub = (np.ascontiguousarray(v, dtype=np.float64) for v in (self.f.q, self.y, self.ub))
+        h = C.c_void_p()
+        N.call('svmb200_smo_create', H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows, layout,
+               N.ptr(y), N.ptr(q), N.ptr(ub), float(self.tol), int(self.max_iter), C.byref(h))
+        self.symmetric_pass = False
+        return h, n
+
+    def _print_iteration(self, scalars):
+        print('\n{:4d}\t{: 1.4e}\t{: 1.4e}'.format(self.iter, self.f_x, scalars[1]), end='')
+
+    def _after_run(self, h, n):
+        self._collect_stats(h)
+        self.gap = self._pull_state(h, n)
+        cnt = C.c_int64(0)
+        f_hist, gap_hist = np.empty(self.iter + 1), np.empty(self.iter + 1)
+        N.call('svmb200_pg_history', h, N.ptr(f_hist), N.ptr(gap_hist), C.byref(cnt))
+        self.f_hist, self.gap_hist = f_hist[:cnt.value], gap_hist[:cnt.value]
+        self.f_x = float(0.5 * np.dot(self.x, self.g_x + self.f.q))
+        self.rho = calculate_rho(self.x, self.g_x, self.y, self.ub)

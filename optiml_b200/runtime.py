@@ -361,9 +361,7 @@ class DeviceGroup:
 
     def wants(self, n):
         """shard an n x n matrix over the group?  (every rank must own rows: the fused exchange has no collective)"""
-        P = len(self.ctxs)
-        rows_per_rank = shard_rows(n, 0, P)[1]
-        return n >= P * self.MIN_ROWS_PER_GPU and (P - 1) * rows_per_rank < n
+        return _group_shards(len(self.ctxs), n)
 
     def replicate(self, src):
         """copies of a DeviceMatrix on every rank's device (rank order); the source's own device reuses it in place"""
@@ -381,6 +379,11 @@ class DeviceGroup:
     def trim(self):
         for c in self.ctxs:
             c.trim()
+
+
+def _group_shards(P, n):
+    rows_per_rank = shard_rows(n, 0, P)[1]
+    return n >= P * DeviceGroup.MIN_ROWS_PER_GPU and (P - 1) * rows_per_rank < n
 
 
 class GroupHessian:
@@ -537,6 +540,20 @@ def default_context():
         _attach_group(ctx)
     _default_ctx = ctx
     return ctx
+
+
+def would_shard(n):
+    """Would the Hessian of an n-variable fit started now be row-sharded (torchrun world > 1, or a device group that
+    shards n)?  Answered without creating a context."""
+    if _default_ctx is not None:
+        return _default_ctx.nranks > 1 or (_default_ctx.group is not None and _default_ctx.group.wants(int(n)))
+    import sys
+    if 'torch' in sys.modules:
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            return True
+    devs = _configured_devices()
+    return devs is not None and len(devs) >= 2 and _group_shards(len(devs), int(n))
 
 
 def broadcast_unique_id(dist, make_id):
