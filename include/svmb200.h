@@ -186,6 +186,25 @@ int svmb200_fw_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
 int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                        int hessian, const double* sign_host, const double* q_host, const double* ub_host, double tol,
                        int64_t max_iter, svmb200_pg** out);
+/* K12: the same SMO solver for problems whose Hessian does not fit in HBM.  No matrix is stored: every row of Q the
+ * solver needs is computed from X on the device, Q_st = sign_s sign_t k(x_{s mod n}, x_{t mod n}) (PLAIN: nvars = n,
+ * SVC with sign = the labels; SVR: nvars = 2n, sign = e), with K1's arithmetic for the kernel value (svmb200_gram with
+ * dA = dB = X, same = 1, bias 0, no signs).  dX: n x d, row stride ldx (even, 16-byte aligned), kept alive by the caller
+ * until svmb200_pg_destroy.  A row cache of cache_bytes (rounded down to whole rows of nvars doubles; 0: no cache) is
+ * owned by the solver.  Hits and misses never change a bit of the trajectory.  At most svmb200_smo_max_vars(SMs)
+ * variables (the shared-memory slice: 4 714 per SM); more is SVMB200_ERR_ARG.  Then svmb200_pg_run / _state / _history
+ * / _scalars / _stats / _destroy as for svmb200_smo_create. */
+int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel,
+                            double gamma, double coef0, double degree, int hessian, const double* sign_host,
+                            const double* q_host, const double* ub_host, double tol, int64_t max_iter, size_t cache_bytes,
+                            svmb200_pg** out);
+int64_t svmb200_smo_max_vars(int sm_count);
+/* row source of an SMO solver (computed = 1: svmb200_smo_create_rows), cache slots, hits and misses so far (every row
+ * computed without a cache counts as a miss); any output pointer may be NULL */
+int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses);
+/* dout[r][t] = k(X_{rows[r]}, X_t) for t < n (0 for t in [n, ldo)), unsigned, no bias: the values SMO's computed rows use */
+int svmb200_kernel_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel, double gamma,
+                        double coef0, double degree, const int64_t* rows_host, int64_t nrows, double* dout, int64_t ldo);
 /* Advance by at most `max_new` iterations (< 0: run to termination; 0: only evaluate the state at
  * the current callback point, i.e. f, |d| and the stopping tests).  The callback point of the
  * reference (projected_gradient.py:95-98) is reached once per iteration; the state visible after

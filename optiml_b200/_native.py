@@ -67,6 +67,10 @@ PROTOTYPES = {
                                  C.c_double, C.c_int, C.c_int, c_vp, c_vp, C.c_double, C.c_double, C.c_double,
                                  C.c_double, C.c_double, i64, C.POINTER(c_vp)],
     'svmb200_smo_create': [c_vp, c_vp, i64, i64, i64, i64, C.c_int, c_vp, c_vp, c_vp, C.c_double, i64, C.POINTER(c_vp)],
+    'svmb200_smo_create_rows': [c_vp, c_vp, i64, i64, i64, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, c_vp,
+                                c_vp, c_vp, C.c_double, i64, C.c_size_t, C.POINTER(c_vp)],
+    'svmb200_smo_cache_stats': [c_vp, C.POINTER(C.c_int), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)],
+    'svmb200_kernel_rows': [c_vp, c_vp, i64, i64, i64, C.c_int, C.c_double, C.c_double, C.c_double, c_vp, i64, c_vp, i64],
     'svmb200_pg_run_batch': [C.POINTER(c_vp), C.c_int, C.POINTER(i64), C.POINTER(C.c_int)],
     'svmb200_matvec_multi': [c_vp, c_vp, i64, i64, C.POINTER(c_vp), C.POINTER(c_vp), C.c_int],
     'svmb200_al_multipliers': [c_vp, C.POINTER(C.c_double), c_vp, c_vp],
@@ -111,6 +115,7 @@ _NON_STATUS = {
     'svmb200_last_error': ([], C.c_char_p),
     'svmb200_version': ([], C.c_char_p),
     'svmb200_padded_ld': ([i64], i64),
+    'svmb200_smo_max_vars': ([C.c_int], i64),
 }
 
 _lib = None

@@ -20,6 +20,7 @@
 // lives at chunk c^(r&7); the four k-slots of an m8n8k4 fragment are mapped to chunks {s, s+4}
 // (s = k-step), so the 16 lanes of a half-warp hit 16 distinct 8-byte bank pairs.
 #include "common.cuh"
+#include "kernel_fn.cuh"   // exp8, ipow_rn, pow / tanh out of line (shared with K12)
 #include <cudaTypedefs.h>
 #include <math.h>
 #include <stdlib.h>
@@ -143,64 +144,6 @@ __device__ __forceinline__ uint64_t l2_evict_first_policy() { return 0; }
 __device__ __forceinline__ void st_evict_first_f64x2(double* ptr, double2 v, uint64_t) { *reinterpret_cast<double2*>(ptr) = v; }
 #define SVM_PTX(...) ((void)0)
 #endif
-
-// pow() stays out of line (the poly epilogue is unrolled 64x per thread and pow is ~300 instructions).
-__device__ __noinline__ double pow_outofline(double x, double y) { return pow(x, y); }
-// x ** n for a small positive integer n (PolyKernel's default degree = 3, kernels.py:79, 95) by binary powering with
-// separately rounded products: n = 2 is NumPy's own fast path (np.square, exact same bits); n = 3 is (x*x)*x, two
-// roundings against libm pow's one (<= ~1.5 ulp apart, SURVEY.md A.12: far inside the 1e-12 Gram bar).  pow() was
-// ~300 instructions per output and made the poly Gram 6x slower than the Gaussian one per element.
-__device__ __forceinline__ double ipow_rn(double x, int n) {
-    double r = 1.0, b = x;
-    bool first = true;
-    for (;;) {
-        if (n & 1) {
-            r = first ? b : __dmul_rn(r, b);
-            first = false;
-        }
-        n >>= 1;
-        if (n == 0) break;
-        b = __dmul_rn(b, b);
-    }
-    return r;
-}
-__device__ __noinline__ double tanh_outofline(double x) { return tanh(x); }
-
-// exp(x), x <= 0, for the Gaussian epilogue, evaluated for EIGHT independent arguments in lock-step so
-// that the FP64 unit sees 8 independent dependency chains (a scalar exp() is one chain of dependent DFMAs,
-// 9.4 cycles each).  Classic scheme: k = rint(x log2 e) through the 1.5*2^52 trick, r = x - k ln2 (hi/lo
-// split), degree-13 Taylor polynomial on |r| <= ln2/2 (truncation 6e-18), then 2^k in two exact steps
-// (2^(k+1000) on the exponent field, times 2^-1000) so that results in the denormal range are rounded once
-// and everything below underflows to 0 -- no branch, no call.  <= 1.5 ulp; exp8(0) == 1 exactly.
-__device__ __forceinline__ void exp8(const double (&x)[8], double (&out)[8]) {
-    constexpr double L2E = 1.4426950408889634074, MAGIC = 6755399441055744.0;
-    constexpr double LN2_HI = 6.93147180369123816490e-01, LN2_LO = 1.90821492927058770002e-10;
-    constexpr double TWO_M1000 = 9.33263618503218878990e-302;  // 2^-1000
-    double r[8], p[8];
-    int k[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-        // exp(-800) == 0 in FP64; keeps k in range.  A compare + select, not fmax(): fmax's NaN rule costs DSETP + 2 SEL +
-        // LOP3 + moves (7 instructions), the select 3, and the results agree for every non-NaN argument
-        const double xe = x[e] < -800.0 ? -800.0 : x[e];
-        double t = fma(xe, L2E, MAGIC);
-        k[e] = __double2loint(t);
-        t -= MAGIC;
-        r[e] = fma(t, -LN2_HI, xe);
-        r[e] = fma(t, -LN2_LO, r[e]);
-        p[e] = 1.0 / 6227020800.0;  // 1/13!
-    }
-    constexpr double C[13] = {1.0, 1.0, 1.0 / 2, 1.0 / 6, 1.0 / 24, 1.0 / 120, 1.0 / 720, 1.0 / 5040, 1.0 / 40320,
-                              1.0 / 362880, 1.0 / 3628800, 1.0 / 39916800, 1.0 / 479001600};
-#pragma unroll
-    for (int j = 12; j >= 0; --j) {
-#pragma unroll
-        for (int e = 0; e < 8; ++e) p[e] = fma(p[e], r[e], C[j]);
-    }
-#pragma unroll
-    for (int e = 0; e < 8; ++e)
-        out[e] = __hiloint2double(__double2hiint(p[e]) + ((k[e] + 1000) << 20), __double2loint(p[e])) * TWO_M1000;
-}
 
 #ifndef SVMB200_HOST_EMULATION
 __device__ __forceinline__ void cp_async_8(double* smem_dst, const double* gmem_src) {
@@ -659,6 +602,14 @@ int launch_gram(svmb200_ctx* ctx, const CUtensorMap& ma, const CUtensorMap& mb, 
     return SVMB200_OK;
 }
 
+// K12: the listed rows of the unsigned kernel matrix, one thread per element, through kfn_value (kernel_fn.cuh)
+__global__ void kernel_rows_kernel(const KernelFn p, long long n, const long long* __restrict__ rows, long long nrows,
+                                   double* __restrict__ out, long long ldo) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= ldo) return;
+    for (long long r = blockIdx.y; r < nrows; r += gridDim.y) out[r * ldo + t] = t < n ? kfn_value(p, rows[r], t) : 0.0;
+}
+
 }  // namespace
 
 extern "C" int64_t svmb200_padded_ld(int64_t ncols) { return round_up64(ncols < 1 ? 1 : ncols, 16); }
@@ -752,12 +703,68 @@ extern "C" int svmb200_gram(svmb200_ctx* ctx, const double* dA, int64_t na, int6
         a.coef0 = coef0;
         a.degree = degree;
         a.bias = bias;
-        a.int_degree = (degree >= 1.0 && degree <= 64.0 && degree == (double)(int)degree) ? (int)degree : 0;
-        if (getenv("SVMB200_POLY_LIBM_POW") != nullptr && atoi(getenv("SVMB200_POLY_LIBM_POW")) != 0) a.int_degree = 0;  // A/B
+        a.int_degree = svm_gram_int_degree(degree);
         if (kernel == SVMB200_KERNEL_LINEAR) rc = launch_gram<SVMB200_KERNEL_LINEAR>(ctx, ma, mb, a);
         else if (kernel == SVMB200_KERNEL_POLY) rc = launch_gram<SVMB200_KERNEL_POLY>(ctx, ma, mb, a);
         else if (kernel == SVMB200_KERNEL_SIGMOID) rc = launch_gram<SVMB200_KERNEL_SIGMOID>(ctx, ma, mb, a);
         else rc = launch_gram<SVMB200_KERNEL_GAUSSIAN>(ctx, ma, mb, a);
     }
     return rc;
+}
+
+int svm_gram_int_degree(double degree) {
+    if (getenv("SVMB200_POLY_LIBM_POW") != nullptr && atoi(getenv("SVMB200_POLY_LIBM_POW")) != 0) return 0;  // A/B
+    return (degree >= 1.0 && degree <= 64.0 && degree == (double)(int)degree) ? (int)degree : 0;
+}
+
+int svm_row_sqnorms(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ld, int64_t d, double* out) {
+    const int wpb = 8;
+    row_sqnorm_kernel<<<(unsigned)((n + wpb - 1) / wpb), wpb * 32, 0, ctx->stream>>>(dX, n, ld, d, out);
+    ctx->launches++;
+    SVM_CUDA(cudaGetLastError());
+    return SVMB200_OK;
+}
+
+extern "C" int svmb200_kernel_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel,
+                                   double gamma, double coef0, double degree, const int64_t* rows_host, int64_t nrows,
+                                   double* dout, int64_t ldo) {
+    SVM_TRY(svm_use(ctx));
+    SVM_CHECK_ARG(dX != nullptr && dout != nullptr, "null matrix");
+    SVM_CHECK_ARG(n > 0 && d > 0 && nrows >= 0, "empty operand");
+    SVM_CHECK_ARG(ldx >= d && ldx % 2 == 0 && (reinterpret_cast<uintptr_t>(dX) & 15) == 0,
+                  "ldx must be even and >= d, X 16-byte aligned");
+    SVM_CHECK_ARG(ldo >= n, "ldo must be >= n");
+    SVM_CHECK_ARG(kernel >= SVMB200_KERNEL_LINEAR && kernel <= SVMB200_KERNEL_LAPLACIAN, "unknown kernel id");
+    SVM_CHECK_ARG((kernel != SVMB200_KERNEL_GAUSSIAN && kernel != SVMB200_KERNEL_LAPLACIAN) || gamma >= 0.0,
+                  "gamma must be >= 0 for the gaussian / laplacian kernels");
+    SVM_CHECK_ARG(n < (1ll << 31) && d < (1ll << 31), "dimension too large");
+    if (nrows == 0) return SVMB200_OK;
+    SVM_CHECK_ARG(rows_host != nullptr, "null row list");
+    for (int64_t r = 0; r < nrows; ++r) SVM_CHECK_ARG(rows_host[r] >= 0 && rows_host[r] < n, "row index out of range");
+    const size_t idx_bytes = (size_t)nrows * sizeof(long long), sq_bytes = kernel == SVMB200_KERNEL_GAUSSIAN ? (size_t)n * sizeof(double) : 0;
+    SVM_TRY(svm_scratch_reserve(ctx, &ctx->idx_buf, &ctx->idx_bytes, idx_bytes));
+    cudaStream_t s = ctx->stream;
+    SVM_CUDA(cudaMemcpyAsync(ctx->idx_buf, rows_host, idx_bytes, cudaMemcpyHostToDevice, s));
+    KernelFn p;
+    p.X = dX;
+    p.ldx = ldx;
+    p.d = d;
+    p.sqn = nullptr;
+    p.kernel = kernel;
+    p.gamma = gamma;
+    p.coef0 = coef0;
+    p.degree = degree;
+    p.int_degree = svm_gram_int_degree(degree);
+    if (sq_bytes) {
+        SVM_TRY(svm_scratch_reserve(ctx, &ctx->norm_buf, &ctx->norm_bytes, sq_bytes));
+        p.sqn = static_cast<double*>(ctx->norm_buf);
+        SVM_TRY(svm_row_sqnorms(ctx, dX, n, ldx, d, static_cast<double*>(ctx->norm_buf)));
+    }
+    const unsigned nt = 256;
+    dim3 grid((unsigned)((ldo + nt - 1) / nt), (unsigned)(nrows < 65535 ? nrows : 65535));
+    kernel_rows_kernel<<<grid, nt, 0, s>>>(p, n, static_cast<const long long*>(ctx->idx_buf), nrows, dout, ldo);
+    ctx->launches++;
+    SVM_CUDA(cudaGetLastError());
+    SVM_CUDA(cudaStreamSynchronize(s));  // pageable row list: the caller may reuse it right away
+    return SVMB200_OK;
 }

@@ -28,12 +28,28 @@
 // operation of the step, of G's update and of the objective is an explicit _rn intrinsic (the library is built with
 // --fmad=true): no contraction, so a NumPy restatement of the algorithm replays the whole trajectory bit for bit.
 // Layouts: PLAIN, Q itself resident (SVC: y_s y_t K_st);  SVR, M = K resident (n x n) and Q_st = e_s e_t M[s mod n][t mod n].
+//
+// K12, the row source (template parameter ROWS).  SMO_ROWS_RESIDENT reads Q from HBM as above.  SMO_ROWS_COMPUTED reads
+// no matrix: Q_st = sign_s sign_t k(x_{s mod n}, x_{t mod n}) (both layouts), the kernel value from X by kfn_value
+// (kernel_fn.cuh), so a problem far larger than HBM runs.  A CTA only ever needs its own slice of row j (phase 1) and of
+// row i (phase 2): it computes that slice, or reads it from a row cache in HBM --
+//   `slots` rows of nvars doubles, keyed by the sample index (SVR rows s and s + n share a slot), unsigned values;
+//   set-associative (sets x ways; every sample has its own slot when the cache holds all n rows), LRU within a set by
+//   the stamp of the last use (2k for row j in phase 1 of iteration k, 2k + 1 for row i in phase 2);
+//   every CTA keeps a private copy of the tags and stamps and updates it identically from the (i, j) sequence, and
+//   reads and writes only its own slice of a slot: no inter-CTA traffic, no race.
+// A value is the same whether it was cached or computed, so hits and misses never change a bit of the trajectory.
+// Q_ij (phase 3) travels from j's owner, which holds Q_it for t = j in its part of row i, through a per-CTA slot
+// published beside the j candidate.
 #pragma once
 #include "k_persistent.cuh"   // pk_grid_barrier
+#include "kernel_fn.cuh"      // kfn_value
 
 constexpr int SMO_NT = 256;
 constexpr int SMO_ARRAYS = 6;        // doubles of shared memory per owned variable: alpha, G, sign, Q_tt, C, Q_it
 constexpr double SMO_TAU = 1e-12;
+constexpr int SMO_ROWS_RESIDENT = 0, SMO_ROWS_COMPUTED = 1;
+constexpr int SMO_CACHE_WAYS = 8;
 
 struct SmoCand {      // the winner of one CTA's slice (64 bytes)
     double key;       // i pass: -y_t G_t;  j pass: b_t^2 / a_t  (the larger wins, ties to the larger index)
@@ -58,6 +74,14 @@ struct SmoArgs {
     long long max_iter;
     long long k0;           // first state this launch evaluates
     long long niter;        // steps to take unless the stopping test fires first (states k0 .. k0 + niter are evaluated)
+    // computed rows only
+    KernelFn kf;
+    double* qij;            // [2 parities][grid]: Q_it at t = the CTA's j candidate
+    double* cache;          // slots x nvars, or null (no cache)
+    int* tags;              // [grid][slots] sample index per slot (-1: empty)
+    long long* stamps;      // [grid][slots] stamp of the last use
+    long long sets, ways;
+    unsigned long long* stats;  // hits, misses (CTA 0)
 };
 
 // Q[s][t] as read from row s
@@ -66,6 +90,50 @@ __device__ __forceinline__ double smo_q(const SmoArgs& a, long long s, long long
     const bool s_lo = s < a.n, t_lo = t < a.n;
     const double v = __ldg(a.Q + (s_lo ? s : s - a.n) * a.ld + (t_lo ? t : t - a.n));
     return s_lo == t_lo ? v : -v;
+}
+
+// thread 0 of a CTA: the slot of sample r in this CTA's copy of the cache tags (LRU victim on a miss), -1 without cache
+__device__ __forceinline__ long long smo_cache_lookup(const SmoArgs& a, long long r, long long stamp, int& hit) {
+    hit = 0;
+    long long slot = -1;
+    if (a.sets > 0) {
+        const long long slots = a.sets * a.ways, base = (r % a.sets) * a.ways;
+        int* tags = a.tags + (size_t)blockIdx.x * slots;
+        long long* st = a.stamps + (size_t)blockIdx.x * slots;
+        // all ways are loaded before any is compared: independent loads, one round trip to L2 instead of `ways`
+        int tg[SMO_CACHE_WAYS];
+        long long sp[SMO_CACHE_WAYS];
+#pragma unroll
+        for (int w = 0; w < SMO_CACHE_WAYS; ++w) {
+            tg[w] = w < a.ways ? tags[base + w] : -1;
+            sp[w] = w < a.ways ? st[base + w] : 0;
+        }
+        long long oldest = 0;
+#pragma unroll
+        for (int w = 0; w < SMO_CACHE_WAYS; ++w) {
+            if (w >= a.ways || hit) continue;
+            if (tg[w] == (int)r) {
+                slot = base + w;
+                hit = 1;
+            } else if (slot < 0 || sp[w] < oldest) {
+                slot = base + w;
+                oldest = sp[w];
+            }
+        }
+        tags[slot] = (int)r;
+        st[slot] = stamp;
+    }
+    if (blockIdx.x == 0) a.stats[hit ? 0 : 1] += 1;
+    return slot;
+}
+
+// unsigned K[r][t mod n] for the own variable t: from the cache slot on a hit, else from X (and into the slot)
+__device__ __forceinline__ double smo_row_value(const SmoArgs& a, long long r, long long t, long long slot, int hit) {
+    double* c = slot >= 0 ? a.cache + slot * a.nvars + t : nullptr;
+    if (hit) return *c;
+    const double v = kfn_value(a.kf, r, t < a.n ? t : t - a.n);
+    if (c) *c = v;
+    return v;
 }
 
 __device__ __forceinline__ bool smo_wins(double k, double i, double bk, double bi) { return k > bk || (k == bk && i > bi); }
@@ -132,6 +200,7 @@ __device__ __forceinline__ void smo_grid_reduce(const SmoCand* slots, unsigned g
     __syncthreads();
 }
 
+template <int ROWS>
 __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs a) {
 #ifndef SVMB200_HOST_EMULATION
     extern __shared__ __align__(16) unsigned char smo_smem_raw[];
@@ -141,6 +210,8 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
 #endif
     __shared__ double red[3][SMO_NT / 32];
     __shared__ SmoCand win_i, win_j;
+    __shared__ long long s_slot[2];   // computed rows: cache slot of row j (phase 1) and of row i (phase 2)
+    __shared__ int s_hit[2];
     const int tid = threadIdx.x;
     const unsigned grid = gridDim.x;
     const int S = a.slice;
@@ -154,7 +225,12 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         s_g[l] = a.g[t];
         s_y[l] = a.sgn[t];
         s_c[l] = a.ub[t];
-        s_qd[l] = smo_q(a, t, t);
+        if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+            const long long tm = t < a.n ? t : t - a.n;
+            s_qd[l] = kfn_value(a.kf, tm, tm);
+        } else {
+            s_qd[l] = smo_q(a, t, t);
+        }
         s_qi[l] = 0.0;
     }
     double f = a.st->f;   // objective at state k0 (CTA 0 rewrites it only after the first grid barrier)
@@ -173,7 +249,14 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
             const long long t = t0 + l;
             double gt = s_g[l];
             if (pending) {
-                gt = __dadd_rn(gt, __dadd_rn(__dmul_rn(s_qi[l], dai), __dmul_rn(smo_q(a, pj, t), daj)));
+                double qjt;
+                if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+                    const double v = smo_row_value(a, pj < a.n ? pj : pj - a.n, t, s_slot[0], s_hit[0]);
+                    qjt = win_j.y == s_y[l] ? v : -v;
+                } else {
+                    qjt = smo_q(a, pj, t);
+                }
+                gt = __dadd_rn(gt, __dadd_rn(__dmul_rn(s_qi[l], dai), __dmul_rn(qjt, daj)));
                 s_g[l] = gt;
             }
             const double y = s_y[l], al = s_alpha[l];
@@ -203,12 +286,24 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         smo_grid_reduce(slots_i, grid, S, red, &win_i);
         const double m = win_i.key, yi = win_i.y, qii = win_i.qd;
         const long long i = (long long)win_i.idx;
+        if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+            if (tid == 0 && i >= 0) s_slot[1] = smo_cache_lookup(a, i < a.n ? i : i - a.n, 2 * k + 1, s_hit[1]);
+            __syncthreads();
+        }
         key = -INFINITY;
         idx = -1.0;
         low = INFINITY;
         for (int l = tid; l < len; l += SMO_NT) {
             const long long t = t0 + l;
-            const double qit = i >= 0 ? smo_q(a, i, t) : 0.0;
+            double qit = 0.0;
+            if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+                if (i >= 0) {
+                    const double v = smo_row_value(a, i < a.n ? i : i - a.n, t, s_slot[1], s_hit[1]);
+                    qit = yi == s_y[l] ? v : -v;
+                }
+            } else {
+                qit = i >= 0 ? smo_q(a, i, t) : 0.0;
+            }
             s_qi[l] = qit;
             const double y = s_y[l], al = s_alpha[l];
             const bool lowset = y > 0.0 ? al > 0.0 : al < s_c[l];
@@ -237,6 +332,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
                 c.y = s_y[l];
                 c.qd = s_qd[l];
                 c.c = s_c[l];
+                if constexpr (ROWS == SMO_ROWS_COMPUTED) a.qij[(size_t)(k & 1) * grid + blockIdx.x] = s_qi[l];
             }
             slots_j[blockIdx.x] = c;
         }
@@ -271,7 +367,9 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         // a_i - a_j, quad = Q_ii + Q_jj + 2 Q_ij;  y_i == y_j: it keeps a_i + a_j, quad = Q_ii + Q_jj - 2 Q_ij.  With
         // Q_ij = y_i y_j K_ij both are K_ii + K_jj - 2 K_ij, the curvature along the feasible direction.
         const double qjj = win_j.qd, gi = win_i.g, gj = win_j.g, ci = win_i.c, cj = win_j.c;
-        const double qij = smo_q(a, i, j);
+        double qij;
+        if constexpr (ROWS == SMO_ROWS_COMPUTED) qij = __ldcg(a.qij + (size_t)(k & 1) * grid + j / S);
+        else qij = smo_q(a, i, j);
         const double ai0 = win_i.alpha, aj0 = win_j.alpha;
         double ai = ai0, aj = aj0;
         if (yi != win_j.y) {
@@ -321,6 +419,9 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         }
         pending = true;
         pj = j;
+        if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+            if (tid == 0) s_slot[0] = smo_cache_lookup(a, j < a.n ? j : j - a.n, 2 * (k + 1), s_hit[0]);
+        }
         __syncthreads();   // alpha of i / j in place for the next phase 1
     }
     for (int l = tid; l < len; l += SMO_NT) {

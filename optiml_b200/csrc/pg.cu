@@ -515,6 +515,16 @@ struct svmb200_pg {
     int smo_grid = 0, smo_slice = 0;
     SmoCand* smo_cand = nullptr;
     double* smo_hist = nullptr;  // hist_f | hist_ng, hist_cap each
+    // computed rows (K12): kernel of X, row cache (sets x ways slots), private tags per CTA, Q_ij slots, hit / miss count
+    int smo_rows = SMO_ROWS_RESIDENT;
+    KernelFn smo_kf = {};
+    void* smo_rows_buf = nullptr;  // |x|^2 | Q_ij slots | tags | stamps | stats | cache
+    double* smo_qij = nullptr;
+    double* smo_cache = nullptr;
+    int* smo_tags = nullptr;
+    long long* smo_stamps = nullptr;
+    unsigned long long* smo_stats = nullptr;
+    long long smo_sets = 0, smo_ways = 0;
 };
 
 constexpr size_t POLL_SLOT_BYTES = 128;  // {PGDeviceState, ..., int fault} per poll slot of the pinned block
@@ -670,6 +680,7 @@ extern "C" int svmb200_pg_destroy(svmb200_pg* pg) {
         cudaSetDevice(pg->ctx->device);
         cudaStreamSynchronize(pg->ctx->stream);
         if (pg->smo_hist) cudaFree(pg->smo_hist);
+        if (pg->smo_rows_buf) cudaFree(pg->smo_rows_buf);
         if (pg->slab_private) {
             if (pg->slab) cudaFree(pg->slab);
             if (pg->pinned) cudaFreeHost(pg->pinned);
@@ -1634,21 +1645,30 @@ constexpr int64_t SMO_SLICE_MAX = (int64_t)(SMO_SMEM_MAX / (SMO_ARRAYS * sizeof(
 
 static size_t smo_smem_bytes(const svmb200_pg* pg) { return (size_t)pg->smo_slice * SMO_ARRAYS * sizeof(double); }
 
-extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
-                                  int hessian, const double* sign_host, const double* q_host, const double* ub_host,
-                                  double tol, int64_t max_iter, svmb200_pg** out) {
-    SVM_TRY(svm_use(ctx));
-    SVM_CHECK_ARG(out != nullptr, "out is null");
-    *out = nullptr;
-    SVM_CHECK_ARG(dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
-    SVM_CHECK_ARG(n > 1, "Q is too small");
-    SVM_CHECK_ARG(ld >= n && ld % 2 == 0, "ld must be >= n and even");
-    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
-    SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
+// computed rows (K12): what svmb200_smo_create_rows adds to the resident solver
+struct SmoRowsSpec {
+    KernelFn kf;
+    size_t cache_bytes;
+};
+
+extern "C" int64_t svmb200_smo_max_vars(int sm_count) { return SMO_SLICE_MAX * (int64_t)sm_count; }
+
+static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int hessian, const double* sign_host,
+                      const double* q_host, const double* ub_host, double tol, int64_t max_iter, const SmoRowsSpec* rows,
+                      svmb200_pg** out) {
     SVM_CHECK_ARG(max_iter > 0, "max_iter must be > 0");
     SVM_CHECK_ARG(tol >= 0.0, "tol must be >= 0");
     const int64_t nvars = hessian == SVMB200_HESSIAN_SVR ? 2 * n : n;
     SVM_CHECK_ARG(nvars < (1ll << 31), "too many variables");
+    if (rows) {
+        const int64_t cap = svmb200_smo_max_vars(ctx->sm_count > 0 ? ctx->sm_count : 1);
+        if (nvars > cap) {
+            svmb200_set_error("SMO with computed rows holds at most %lld variables on this GPU (%lld per CTA x %d SMs, the "
+                              "shared-memory slice): %lld requested", (long long)cap, (long long)SMO_SLICE_MAX, ctx->sm_count,
+                              (long long)nvars);
+            return SVMB200_ERR_ARG;
+        }
+    }
     for (int64_t t = 0; t < nvars; ++t) {
         SVM_CHECK_ARG(sign_host[t] == 1.0 || sign_host[t] == -1.0, "signs must be +-1");
         SVM_CHECK_ARG(ub_host[t] > 0.0 && ub_host[t] < INFINITY, "upper bounds must be finite and > 0");
@@ -1664,8 +1684,8 @@ extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n,
     pg->dQ = dQ;
     pg->n = n;
     pg->ld = ld;
-    pg->row0 = row0;
-    pg->nrows = nrows;
+    pg->row0 = 0;
+    pg->nrows = n;
     pg->svr = hessian == SVMB200_HESSIAN_SVR;
     pg->nvars = nvars;
     pg->rows_per_rank = n;
@@ -1675,6 +1695,10 @@ extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n,
     pg->smo_slice = (int)slice;
     pg->smo_grid = (int)((nvars + slice - 1) / slice);
     pg->slab_private = true;
+    if (rows) {
+        pg->smo_rows = SMO_ROWS_COMPUTED;
+        pg->smo_kf = rows->kf;
+    }
     auto fail = [&](int code) {
         svmb200_pg_destroy(pg);
         return code;
@@ -1693,11 +1717,16 @@ extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n,
         static bool configured[64] = {};
         const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
         if (!configured[dev]) {
-            SMO_CUDA(cudaFuncSetAttribute(smo_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMO_SMEM_MAX));
+            SMO_CUDA(cudaFuncSetAttribute(smo_persistent_kernel<SMO_ROWS_RESIDENT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)SMO_SMEM_MAX));
+            SMO_CUDA(cudaFuncSetAttribute(smo_persistent_kernel<SMO_ROWS_COMPUTED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)SMO_SMEM_MAX));
             configured[dev] = true;
         }
         int per_sm = 0;
-        SMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, smo_persistent_kernel, SMO_NT, smo_smem_bytes(pg)));
+        SMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
+            &per_sm, rows ? smo_persistent_kernel<SMO_ROWS_COMPUTED> : smo_persistent_kernel<SMO_ROWS_RESIDENT>, SMO_NT,
+            smo_smem_bytes(pg)));
         if ((long long)per_sm * ctx->sm_count < pg->smo_grid) {
             svmb200_set_error("SMO: %d CTAs of %zu bytes of shared memory cannot be co-resident", pg->smo_grid, smo_smem_bytes(pg));
             return fail(SVMB200_ERR_ARG);
@@ -1733,10 +1762,102 @@ extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n,
         SMO_CUDA(cudaMalloc(&ctx->gbar, 256));
         SMO_CUDA(cudaMemsetAsync(ctx->gbar, 0, 256, s));
     }
+    if (rows) {
+        // cache geometry: every sample its own slot when all n rows fit, else sets of SMO_CACHE_WAYS (fewer if the
+        // cache has fewer slots); cache_bytes = 0: no cache, every row is computed
+        int64_t slots = (int64_t)(rows->cache_bytes / (nv > 0 ? nv : 1));
+        if (slots >= n) {
+            pg->smo_sets = n;
+            pg->smo_ways = 1;
+        } else if (slots > 0) {
+            pg->smo_ways = slots < SMO_CACHE_WAYS ? slots : SMO_CACHE_WAYS;
+            pg->smo_sets = slots / pg->smo_ways;
+        }
+        slots = pg->smo_sets * pg->smo_ways;
+        const size_t sz_sq = up((size_t)n * sizeof(double)), sz_qij = up((size_t)2 * pg->smo_grid * sizeof(double));
+        const size_t sz_tags = up((size_t)pg->smo_grid * slots * sizeof(int));
+        const size_t sz_st = up((size_t)pg->smo_grid * slots * sizeof(long long)), sz_stats = 256;
+        const size_t sz_cache = (size_t)slots * nv;
+        SMO_CUDA(cudaMalloc(&pg->smo_rows_buf, sz_sq + sz_qij + sz_tags + sz_st + sz_stats + sz_cache));
+        unsigned char* rb = static_cast<unsigned char*>(pg->smo_rows_buf);
+        double* sqn = reinterpret_cast<double*>(rb);
+        pg->smo_qij = reinterpret_cast<double*>(rb + sz_sq);
+        pg->smo_tags = reinterpret_cast<int*>(rb + sz_sq + sz_qij);
+        pg->smo_stamps = reinterpret_cast<long long*>(rb + sz_sq + sz_qij + sz_tags);
+        pg->smo_stats = reinterpret_cast<unsigned long long*>(rb + sz_sq + sz_qij + sz_tags + sz_st);
+        pg->smo_cache = slots > 0 ? reinterpret_cast<double*>(rb + sz_sq + sz_qij + sz_tags + sz_st + sz_stats) : nullptr;
+        SMO_CUDA(cudaMemsetAsync(pg->smo_qij, 0, sz_qij, s));
+        SMO_CUDA(cudaMemsetAsync(pg->smo_tags, 0xff, sz_tags + sz_st, s));   // tag -1 (empty), stamp -1
+        SMO_CUDA(cudaMemsetAsync(pg->smo_stats, 0, sz_stats, s));
+        if (pg->smo_kf.kernel == SVMB200_KERNEL_GAUSSIAN) {
+            int rc = svm_row_sqnorms(ctx, pg->smo_kf.X, n, pg->smo_kf.ldx, pg->smo_kf.d, sqn);
+            if (rc != SVMB200_OK) return fail(rc);
+            pg->smo_kf.sqn = sqn;
+        }
+    }
     SMO_CUDA(cudaStreamSynchronize(s));   // the host arrays belong to the caller
 #undef SMO_CUDA
     pg->k_next = 0;
     *out = pg;
+    return SVMB200_OK;
+}
+
+extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
+                                  int hessian, const double* sign_host, const double* q_host, const double* ub_host,
+                                  double tol, int64_t max_iter, svmb200_pg** out) {
+    SVM_TRY(svm_use(ctx));
+    SVM_CHECK_ARG(out != nullptr, "out is null");
+    *out = nullptr;
+    SVM_CHECK_ARG(dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
+    SVM_CHECK_ARG(n > 1, "Q is too small");
+    SVM_CHECK_ARG(ld >= n && ld % 2 == 0, "ld must be >= n and even");
+    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
+    SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
+    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, out);
+}
+
+extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel,
+                                       double gamma, double coef0, double degree, int hessian, const double* sign_host,
+                                       const double* q_host, const double* ub_host, double tol, int64_t max_iter,
+                                       size_t cache_bytes, svmb200_pg** out) {
+    SVM_TRY(svm_use(ctx));
+    SVM_CHECK_ARG(out != nullptr, "out is null");
+    *out = nullptr;
+    SVM_CHECK_ARG(dX != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
+    SVM_CHECK_ARG(n > 1, "X is too small");
+    SVM_CHECK_ARG(d > 0 && ldx >= d && ldx % 2 == 0 && (reinterpret_cast<uintptr_t>(dX) & 15) == 0,
+                  "ldx must be even and >= d, X 16-byte aligned");
+    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
+    SVM_CHECK_ARG(kernel >= SVMB200_KERNEL_LINEAR && kernel <= SVMB200_KERNEL_LAPLACIAN, "unknown kernel id");
+    SVM_CHECK_ARG((kernel != SVMB200_KERNEL_GAUSSIAN && kernel != SVMB200_KERNEL_LAPLACIAN) || gamma >= 0.0,
+                  "gamma must be >= 0 for the gaussian / laplacian kernels");
+    SVM_CHECK_ARG(d < (1ll << 31), "dimension too large");
+    SmoRowsSpec rows;
+    rows.kf.X = dX;
+    rows.kf.ldx = ldx;
+    rows.kf.d = d;
+    rows.kf.sqn = nullptr;
+    rows.kf.kernel = kernel;
+    rows.kf.gamma = gamma;
+    rows.kf.coef0 = coef0;
+    rows.kf.degree = degree;
+    rows.kf.int_degree = svm_gram_int_degree(degree);
+    rows.cache_bytes = cache_bytes;
+    return smo_create(ctx, nullptr, n, 0, hessian, sign_host, q_host, ub_host, tol, max_iter, &rows, out);
+}
+
+extern "C" int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses) {
+    SVM_CHECK_ARG(pg != nullptr && pg->solver == 3, "not an SMO solver");
+    SVM_TRY(svm_use(pg->ctx));
+    unsigned long long hm[2] = {0, 0};
+    if (pg->smo_rows == SMO_ROWS_COMPUTED) {
+        SVM_CUDA(cudaMemcpyAsync(hm, pg->smo_stats, sizeof(hm), cudaMemcpyDeviceToHost, pg->ctx->stream));
+        SVM_CUDA(cudaStreamSynchronize(pg->ctx->stream));
+    }
+    if (computed) *computed = pg->smo_rows == SMO_ROWS_COMPUTED;
+    if (slots) *slots = pg->smo_sets * pg->smo_ways;
+    if (hits) *hits = (int64_t)hm[0];
+    if (misses) *misses = (int64_t)hm[1];
     return SVMB200_OK;
 }
 
@@ -1785,8 +1906,17 @@ static int smo_launch(svmb200_pg* pg, int64_t niter) {
     a.max_iter = pg->max_iter;
     a.k0 = pg->k_next;
     a.niter = niter;
-    SVM_CUDA(svm_launch_cooperative(smo_persistent_kernel, dim3((unsigned)pg->smo_grid), dim3(SMO_NT), smo_smem_bytes(pg),
-                                    pg->ctx->stream, a));
+    a.kf = pg->smo_kf;
+    a.qij = pg->smo_qij;
+    a.cache = pg->smo_cache;
+    a.tags = pg->smo_tags;
+    a.stamps = pg->smo_stamps;
+    a.sets = pg->smo_sets;
+    a.ways = pg->smo_ways;
+    a.stats = pg->smo_stats;
+    SVM_CUDA(svm_launch_cooperative(pg->smo_rows == SMO_ROWS_COMPUTED ? smo_persistent_kernel<SMO_ROWS_COMPUTED>
+                                                                        : smo_persistent_kernel<SMO_ROWS_RESIDENT>,
+                                    dim3((unsigned)pg->smo_grid), dim3(SMO_NT), smo_smem_bytes(pg), pg->ctx->stream, a));
     pg->ctx->launches++;
     return SVMB200_OK;
 }

@@ -21,14 +21,15 @@ from sklearn.exceptions import ConvergenceWarning
 from sklearn.preprocessing import LabelBinarizer
 
 from .kernels import gaussian, Kernel, LinearKernel, _dense_f64, gather_rows
-from .smo import SMO
+from .smo import SMO, select_row_source
 from .losses import (squared_hinge, squared_epsilon_insensitive, Hinge, SquaredHinge, EpsilonInsensitive,
                      SquaredEpsilonInsensitive)
 from ... import _native as N
 from ...opti import Optimizer, Quadratic
 from ...opti.constrained import AugmentedLagrangianQuadratic, BoxConstrainedQuadraticOptimizer, ProjectedGradient
 from ...opti.unconstrained.stochastic import StochasticOptimizer, StochasticMomentumOptimizer
-from ...runtime import DeviceHessian, DeviceMatrix, GroupHessian, default_context, make_hessian, would_shard
+from ...runtime import (DeviceHessian, DeviceMatrix, GroupHessian, KernelRowsHessian, default_context, make_hessian,
+                       would_shard)
 
 _SCOPE = ('optiml_b200 implements the dual formulation solved by a BoxConstrainedQuadraticOptimizer '
           '(ProjectedGradient, FrankWolfe; reg_intercept=True) or, as its augmented-Lagrangian relaxation, by a '
@@ -221,6 +222,33 @@ class SVM(BaseEstimator):
         self.fit_times_ = {'gram_s': time.perf_counter() - t0}  # gamma + upload + Gram kernel (wall clock)
         return H
 
+    def _smo_hessian(self, X, signs, layout, X_device=None):
+        """SMO's Hessian: resident (K1, as for the other solvers) when it fits in the free device memory, else computed
+        rows (K12: no matrix, rows from X on the device, with a row cache) -- chosen by smo.select_row_source before
+        any device work."""
+        import time
+        ctx = default_context()
+        n, d = X.shape
+        nvars = 2 * n if layout == 'svr' else n
+        info = ctx.info()
+        info['free_bytes'] += ctx.pooled_bytes()   # parked buffers are given back when an allocation needs them
+        source, cache_bytes = select_row_source(n, nvars, N.padded_ld(n), d, info)
+        if source == 'resident':
+            return self._build_hessian(X, signs, layout, X_device, 0.0)
+        ctx.trim()   # the row cache is allocated by the solver, outside the pool
+        t0 = time.perf_counter()
+        dX = X_device if X_device is not None else ctx.upload_matrix(X)
+        spec = self.kernel.gram_spec(X, device=dX)
+        if X_device is not None:   # the Hessian owns its reference to X: a private copy of the caller's matrix
+            own = DeviceMatrix(ctx, dX.rows, dX.cols, dX.ld)
+            N.call('svmb200_d2d', ctx.handle, C.c_void_p(own.dptr), C.c_void_p(dX.dptr), dX.nbytes)
+            dX = own
+        H = KernelRowsHessian(ctx, dX, X, spec, layout, signs, cache_bytes)
+        # the support vectors are gathered from the Hessian's X, which it frees on release (_set_support_vectors)
+        self._train_X_device = (dX, False)
+        self.fit_times_ = {'gram_s': time.perf_counter() - t0}  # gamma + upload (no Gram matrix is built)
+        return H
+
     # ------------------------------------------------------------------ support vectors: device-resident, host copy on demand
     @property
     def support_vectors_(self):
@@ -358,6 +386,8 @@ class SVC(ClassifierMixin, SVM):
         if shared is not None:
             hessian = shared.with_signs(ys)
             self.fit_times_ = {}
+        elif solver_cls is SMO:
+            hessian = self._smo_hessian(X, ys, 'plain', X_device)
         else:
             hessian = self._build_hessian(X, ys, 'plain', X_device, bias)
         ub = np.ones(n) * self.C
@@ -447,6 +477,8 @@ class SVR(RegressorMixin, SVM):
         if shared is not None:
             hessian = shared
             self.fit_times_ = {}
+        elif solver_cls is SMO:
+            hessian = self._smo_hessian(X, None, 'svr', X_device)
         else:
             hessian = self._build_hessian(X, None, 'svr', X_device, bias)
         ub = np.ones(2 * n) * self.C

@@ -10,12 +10,46 @@ of K11 (csrc/k_smo.cuh): libsvm's solver without shrinking (Fan, Chen & Lin 2005
 ``optimizer='smo'`` (and ``reg_intercept=False``).
 """
 import ctypes as C
+import os
 
 import numpy as np
 
 from ... import _native as N
 from ...opti import Optimizer, Quadratic
 from ...opti.constrained._device_loop import DeviceLoopMixin
+from ...runtime import KernelRowsHessian
+
+RESIDENT_SHARE = 0.9   # the resident matrix may take this share of the free device memory
+CACHE_SHARE = 0.8      # the row cache of the computed form may take this share of what is free once X is in place
+
+
+def select_row_source(n, nvars, ld, d, info):
+    """Where an SMO fit of ``n`` samples (``nvars`` variables, ``d`` features) gets the rows of Q: ``('resident', 0)``
+    when the n x ld matrix fits ``RESIDENT_SHARE`` of ``info['free_bytes']`` (``Context.info()`` after ``trim()``), else
+    ``('computed', cache_bytes)`` with a row cache of ``CACHE_SHARE`` of what X leaves free, at most all n rows.  Raises
+    ``ValueError`` before any device work when the computed form cannot hold ``nvars`` (the shared-memory slice:
+    ``svmb200_smo_max_vars``).  ``SVMB200_SMO_ROWS=resident|computed`` and ``SVMB200_SMO_CACHE_MB`` override the
+    choice and the cache size (tests, sweeps)."""
+    free = int(info['free_bytes'])
+    source = 'resident' if n * ld * 8 <= RESIDENT_SHARE * free else 'computed'
+    forced = os.environ.get('SVMB200_SMO_ROWS', '').strip().lower()
+    if forced:
+        if forced not in ('resident', 'computed'):
+            raise ValueError(f'SVMB200_SMO_ROWS must be resident or computed, not {forced!r}')
+        source = forced
+    if source == 'resident':
+        return source, 0
+    cap = int(N.load_library().svmb200_smo_max_vars(int(info['sm_count'])))
+    if nvars > cap:
+        raise ValueError(f"optimizer='smo' holds at most {cap} variables on this GPU ({cap // max(int(info['sm_count']), 1)} "
+                         f"per SM, the shared-memory slice); this fit has {nvars}")
+    row = nvars * 8
+    mb = os.environ.get('SVMB200_SMO_CACHE_MB', '').strip()
+    if mb:
+        cache = int(float(mb) * (1 << 20))
+    else:
+        cache = int(CACHE_SHARE * max(free - n * (d + (d & 1)) * 8, 0))   # the fit's copy of X, ld = d rounded to even
+    return source, min(cache // row, n) * row
 
 
 def calculate_rho(alpha, G, y, C):
@@ -60,20 +94,32 @@ class SMO(DeviceLoopMixin, Optimizer):
                                   callback_args=callback_args, verbose=verbose)
         self.y, self.ub = y, C
         self.gap, self.rho = np.nan, np.nan
+        self.row_source, self.cache_slots, self.cache_hits, self.cache_misses = None, 0, 0, 0
 
     def _create(self, profile=False):
         H = self.f.device_hessian()
+        q, y, ub = (np.ascontiguousarray(v, dtype=np.float64) for v in (self.f.q, self.y, self.ub))
+        self.symmetric_pass = False
+        if isinstance(H, KernelRowsHessian):
+            layout = N.HESSIAN_SVR if H.layout == 'svr' else N.HESSIAN_PLAIN
+            if not np.array_equal(y, H.row_signs):
+                raise ValueError('with computed rows the sign row y must be the signs of the Hessian')
+            h = C.c_void_p()
+            N.call('svmb200_smo_create_rows', H.ctx.handle, C.c_void_p(H.X.dptr), H.n, H.X.ld, H.X.cols, int(H.kernel),
+                   float(H.gamma), float(H.coef0), float(H.degree), layout, N.ptr(y), N.ptr(q), N.ptr(ub),
+                   float(self.tol), int(self.max_iter), H.cache_bytes, C.byref(h))
+            self.row_source = 'computed'
+            return h, H.nvars
         if len(H.shards()) != 1 or H.nrows != H.n:
             raise NotImplementedError('SMO runs on one GPU: the Hessian must not be sharded')
         if H.signs is not None:
             raise NotImplementedError('SMO reads the signed matrix itself: signed views of a shared matrix are not supported')
         n = H.nvars
         layout = N.HESSIAN_SVR if H.layout == 'svr' else N.HESSIAN_PLAIN
-        q, y, ub = (np.ascontiguousarray(v, dtype=np.float64) for v in (self.f.q, self.y, self.ub))
         h = C.c_void_p()
         N.call('svmb200_smo_create', H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows, layout,
                N.ptr(y), N.ptr(q), N.ptr(ub), float(self.tol), int(self.max_iter), C.byref(h))
-        self.symmetric_pass = False
+        self.row_source = 'resident'
         return h, n
 
     def _print_iteration(self, scalars):
@@ -81,6 +127,9 @@ class SMO(DeviceLoopMixin, Optimizer):
 
     def _after_run(self, h, n):
         self._collect_stats(h)
+        slots, hits, misses = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        N.call('svmb200_smo_cache_stats', h, None, C.byref(slots), C.byref(hits), C.byref(misses))
+        self.cache_slots, self.cache_hits, self.cache_misses = slots.value, hits.value, misses.value
         self.gap = self._pull_state(h, n)
         cnt = C.c_int64(0)
         f_hist, gap_hist = np.empty(self.iter + 1), np.empty(self.iter + 1)

@@ -2,7 +2,7 @@
 uses (reference: optiml/opti/_base.py).  Matrix work is done by the svmb200 CUDA library."""
 import numpy as np
 
-from ..runtime import DeviceHessian, GroupHessian, default_context, hessian_from_host
+from ..runtime import DeviceHessian, GroupHessian, KernelRowsHessian, default_context, hessian_from_host
 
 
 class OptimizationFunction:
@@ -48,7 +48,7 @@ class Quadratic(OptimizationFunction):
 
     def __init__(self, Q, q):
         q = np.array(q, dtype=float)
-        if isinstance(Q, (DeviceHessian, GroupHessian)):
+        if isinstance(Q, (DeviceHessian, GroupHessian, KernelRowsHessian)):
             self._device, self._host_Q = Q, None
             n = Q.nvars
         else:

@@ -337,6 +337,74 @@ class DeviceHessian:
             self.matrix.release()
 
 
+class KernelRowsHessian:
+    """The Hessian of an SVM dual that is never stored: SMO computes the rows it needs from X on the device (K12,
+    ``svmb200_smo_create_rows``).  ``Q_st = s_s s_t k(x_{s mod n}, x_{t mod n})``: ``layout='plain'`` with ``signs`` = the
+    labels (SVC), ``layout='svr'`` with the block signs ``e = [1, -1]`` (SVR).  ``spec`` = ``(kernel id, gamma, coef0,
+    degree)`` as ``gram_spec`` resolved it.  Holds ``X`` (a :class:`DeviceMatrix`) until :meth:`release`, and the host copy
+    of X that :meth:`product` evaluates against; ``cache_bytes`` sizes the solver's row cache."""
+
+    def __init__(self, ctx, X_device, X_host, spec, layout='plain', signs=None, cache_bytes=0):
+        self.ctx, self.X, self.layout = ctx, X_device, layout
+        self.X_host = np.ascontiguousarray(X_host, dtype=np.float64)
+        self.n = X_device.rows
+        self.kernel, self.gamma, self.coef0, self.degree = spec
+        self.signs = None if signs is None else np.ascontiguousarray(signs, dtype=np.float64).ravel()
+        self.cache_bytes = int(cache_bytes)
+        self.row0, self.nrows = 0, self.n
+
+    @property
+    def nvars(self):
+        return 2 * self.n if self.layout == 'svr' else self.n
+
+    @property
+    def row_signs(self):
+        """the sign row of Q = (s s') o [k(x_s mod n, x_t mod n)]"""
+        if self.layout == 'svr':
+            return np.hstack((np.ones(self.n), -np.ones(self.n)))
+        return np.ones(self.n) if self.signs is None else self.signs
+
+    def shards(self):
+        return [self]
+
+    def kernel_rows(self, rows):
+        """k(x_r, x_t) for the listed rows r and every t (unsigned), by the device function the solver uses"""
+        rows = np.ascontiguousarray(rows, dtype=np.int64)
+        ld = N.padded_ld(self.n)
+        out = DeviceMatrix(self.ctx, len(rows), self.n, ld)
+        try:
+            N.call('svmb200_kernel_rows', self.ctx.handle, C.c_void_p(self.X.dptr), self.n, self.X.ld, self.X.cols,
+                   int(self.kernel), float(self.gamma), float(self.coef0), float(self.degree),
+                   rows.ctypes.data_as(C.c_void_p), len(rows), C.c_void_p(out.dptr), ld)
+            return out.to_host()
+        finally:
+            out.release()
+
+    def to_host(self):
+        """The whole Hessian on the host, from svmb200_kernel_rows (small problems: tests)."""
+        K = self.kernel_rows(np.arange(self.n))
+        if self.layout == 'svr':
+            return np.vstack((np.hstack((K, -K)), np.hstack((-K, K))))
+        return self.signs[:, None] * K * self.signs[None, :] if self.signs is not None else K
+
+    def product(self, v):
+        """Q @ v through K6 (svmb200_decision_device: K1 blocks contracted on the fly), at any n."""
+        v = np.asarray(v, dtype=np.float64).ravel()
+        s = self.row_signs
+        beta = s * v
+        beta = beta[:self.n] + beta[self.n:] if self.layout == 'svr' else beta
+        out = np.empty(self.n)
+        N.call('svmb200_decision_device', self.ctx.handle, C.c_void_p(self.X.dptr), self.n, self.X.ld,
+               N.ptr(np.ascontiguousarray(beta)), N.ptr(self.X_host), self.n, self.X.cols, int(self.kernel),
+               float(self.gamma), float(self.coef0), float(self.degree), 0.0, N.ptr(out))
+        return s * (np.concatenate((out, out)) if self.layout == 'svr' else out)
+
+    def release(self):
+        if self.X is not None:
+            self.X.release()
+            self.X = None
+
+
 class DeviceGroup:
     """One process, N GPUs: ranks 0..N-1 are contexts of the calling thread (one per device) whose exchange arenas are
     mapped by plain peer access (``svmb200_comm_local_group``).  Problems with at least ``MIN_ROWS_PER_GPU`` rows per GPU

@@ -3,7 +3,11 @@ per config: iterations, status, final gap, fit time (device events and wall cloc
 matrix bytes per iteration, the GPU's name and power limit -- and a host arm, sklearn.svm.SVC / SVR (libsvm) on the
 same kernel, gamma, C and tol, with both dual objectives evaluated in FP64 on the same resident Q.
     python scripts/bench_smo.py [--configs C1,C4,C2] [--tol 1e-3] [--no-sklearn] [--grid G] [--n N]
---grid sets SVMB200_SMO_GRID (CTAs of the cooperative launch; default one per SM) for grid-size sweeps."""
+                                [--rows auto|resident|computed] [--cache-mb MB] [--large]
+--grid sets SVMB200_SMO_GRID (CTAs of the cooperative launch; default one per SM) for grid-size sweeps.  --rows and
+--cache-mb set SVMB200_SMO_ROWS / SVMB200_SMO_CACHE_MB (the row source, K12, and its row cache; default: the automatic
+choice); every line reports the row source, the cache's slots and hit rate and the X bytes one computed row reads.
+--large is for sizes only the computed form runs: one fit, no warm-up fit, no sklearn arm."""
 import argparse
 import json
 import os
@@ -32,7 +36,7 @@ def dual_objective(H, q, alpha):
     return float(0.5 * alpha @ H.product(alpha) + q @ alpha)
 
 
-def run(name, tol, max_iter, sklearn_arm, n=None):
+def run(name, tol, max_iter, sklearn_arm, n=None, large=False):
     from optiml_b200.configs import make_config
     from optiml_b200.ml.svm import SVC, SVR
     from optiml_b200.ml.svm.kernels import GaussianKernel, PolyKernel
@@ -42,7 +46,7 @@ def run(name, tol, max_iter, sklearn_arm, n=None):
     spec, X, y = make_config(name, n=n)
     n = len(y)
     ctx = default_context()
-    for rep in range(2):   # the first fit warms the module, the buffer pools and the kernel's shared-memory setting
+    for rep in range(1 if large else 2):   # the first fit warms the module, the buffer pools and the kernel's shared-memory setting
         if spec['task'] == 'svc':
             m = SVC(loss=hinge, kernel=GaussianKernel(), C=1, dual=True, optimizer='smo', tol=tol, max_iter=max_iter)
         else:
@@ -62,7 +66,10 @@ def run(name, tol, max_iter, sklearn_arm, n=None):
                grid=os.environ.get('SVMB200_SMO_GRID', 'one CTA per SM'), iters=o.iter, status=o.status, gap=o.gap,
                fit_s_wall=round(fit_wall, 4), fit_ms_device=round(fit_dev_ms, 2), solve_ms_device=round(o.device_ms, 2),
                us_per_iter=round(1e3 * o.device_ms / max(o.iter, 1), 3), matrix_bytes_per_iter=16 * n,
-               n_sv=int(len(m.support_)), f=o.f_x, gpu=gpu, power_limit=power)
+               n_sv=int(len(m.support_)), f=o.f_x, gpu=gpu, power_limit=power, row_source=o.row_source,
+               cache_slots=o.cache_slots, cache_hits=o.cache_hits, cache_misses=o.cache_misses,
+               hit_rate=round(o.cache_hits / max(o.cache_hits + o.cache_misses, 1), 5),
+               x_bytes_per_miss=n * X.shape[1] * 8)
     if sklearn_arm:
         from sklearn.svm import SVC as SkSVC, SVR as SkSVR
         gamma = resolve_gamma('scale', X)
@@ -95,11 +102,19 @@ def main():
     ap.add_argument('--no-sklearn', action='store_true', help='skip the host arm (long configs)')
     ap.add_argument('--n', type=int, default=None, help='sample count (default: the config\'s full size)')
     ap.add_argument('--grid', type=int, default=None, help='CTAs of the cooperative launch (SVMB200_SMO_GRID)')
+    ap.add_argument('--rows', choices=['auto', 'resident', 'computed'], default='auto', help='row source (K12)')
+    ap.add_argument('--cache-mb', type=float, default=None, help='row cache of the computed form (SVMB200_SMO_CACHE_MB)')
+    ap.add_argument('--large', action='store_true', help='one fit, no sklearn arm (sizes beyond HBM)')
     args = ap.parse_args()
+    if args.rows != 'auto':
+        os.environ['SVMB200_SMO_ROWS'] = args.rows
+    if args.cache_mb is not None:
+        os.environ['SVMB200_SMO_CACHE_MB'] = repr(args.cache_mb)
     if args.grid is not None:
         os.environ['SVMB200_SMO_GRID'] = str(args.grid)
     for name in args.configs.split(','):
-        print(json.dumps(run(name.strip(), args.tol, args.max_iter, not args.no_sklearn, args.n)), flush=True)
+        print(json.dumps(run(name.strip(), args.tol, args.max_iter, not (args.no_sklearn or args.large), args.n,
+                             args.large)), flush=True)
 
 
 if __name__ == '__main__':
