@@ -20,6 +20,7 @@
 #include "k_smo.cuh"         // K11: SMO with the equality constraint, one cooperative kernel for many iterations
 #include <math.h>
 #include <stdlib.h>
+#include <memory>
 
 // ------------------------------------------------------------------------------------------ K2 launchers
 struct MatvecScratch {
@@ -473,13 +474,30 @@ extern "C" int svmb200_shard_rows(int64_t n, int rank, int nranks, int64_t* row0
 }
 
 // ------------------------------------------------------------------------------------------ driver
+enum SolverKind : int {
+    SOLVER_PG = 0,   // projected gradient
+    SOLVER_FW = 1,   // Frank-Wolfe
+    SOLVER_AL = 2,   // augmented Lagrangian + stochastic rule
+    SOLVER_SMO = 3,  // SMO (K11 / K12)
+};
+
+// SMO: the kernel's arguments, filled at creation (smo_launch sets the iteration range and the history), its grid, the
+// row source and the buffer of the computed rows
+struct SmoSolver {
+    SmoArgs a = {};
+    int grid = 0;
+    int rows = SMO_ROWS_RESIDENT;
+    void* rows_buf = nullptr;  // |x|^2 | Q_ij slots | tags | stamps | stats | cache
+};
+
 struct svmb200_pg {
     svmb200_ctx* ctx = nullptr;
     const double* dQ = nullptr;
     int64_t n = 0, ld = 0, row0 = 0, nrows = 0, nvars = 0, rows_per_rank = 0;
     int svr = 0;
-    int solver = 0;      // 0: projected gradient, 1: Frank-Wolfe, 2: augmented Lagrangian + stochastic rule, 3: SMO
-    ALArgs al = {};      // solver 2 only
+    SolverKind solver = SOLVER_PG;
+    ALArgs al = {};      // SOLVER_AL only
+    SmoSolver smo;       // SOLVER_SMO only
     double fw_t = 0.0;   // Frank-Wolfe stabilisation parameter
     double eps = 1e-6;
     int64_t max_iter = 1000;
@@ -493,10 +511,10 @@ struct svmb200_pg {
     int nctas = 1;
     double *q = nullptr, *lb = nullptr, *ub = nullptr;
     double* sgn = nullptr;  // label signs (Q = (s s') o resident matrix), or null
-    double *part = nullptr, *hist_f = nullptr, *hist_ng = nullptr;
+    double *part = nullptr, *hist_f = nullptr, *hist_ng = nullptr;  // SMO: one allocation (smo_hist_reserve) at hist_f
     PGDeviceState* st = nullptr;
     PGDeviceState* st_host = nullptr;  // pinned; points at the slot of the most recent completed poll
-    unsigned char* pinned = nullptr;   // 256 bytes: two poll slots of {PGDeviceState, fault flag}
+    void* pinned = nullptr;            // 256 bytes: two poll slots of {PGDeviceState, fault flag}
     cudaEvent_t ev_poll[2] = {nullptr, nullptr};
     int64_t last_samples = 0;          // iterations of the last run that carried profiling events
     bool deferred_start = false;       // single-process group: first product + INIT are issued by svmb200_pg_start_group
@@ -510,21 +528,7 @@ struct svmb200_pg {
     std::vector<cudaEvent_t> mv_ev;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // the context's solver pair (svmb200_timer_* has its own)
     void* slab = nullptr;        // all device buffers below live in this slab
-    bool slab_private = false;   // true: allocated for this solver only (the context's slab was busy)
-    // SMO (solver 3): grid and slice of its launches, candidate slots, history grown with the iterations actually run
-    int smo_grid = 0, smo_slice = 0;
-    SmoCand* smo_cand = nullptr;
-    double* smo_hist = nullptr;  // hist_f | hist_ng, hist_cap each
-    // computed rows (K12): kernel of X, row cache (sets x ways slots), private tags per CTA, Q_ij slots, hit / miss count
-    int smo_rows = SMO_ROWS_RESIDENT;
-    KernelFn smo_kf = {};
-    void* smo_rows_buf = nullptr;  // |x|^2 | Q_ij slots | tags | stamps | stats | cache
-    double* smo_qij = nullptr;
-    double* smo_cache = nullptr;
-    int* smo_tags = nullptr;
-    long long* smo_stamps = nullptr;
-    unsigned long long* smo_stats = nullptr;
-    long long smo_sets = 0, smo_ways = 0;
+    bool slab_private = false;   // true: allocated for this solver only (the context's slab was busy, or SMO)
 };
 
 constexpr size_t POLL_SLOT_BYTES = 128;  // {PGDeviceState, ..., int fault} per poll slot of the pinned block
@@ -575,8 +579,8 @@ static int launch_vec(svmb200_pg* pg, long long k) {
     VecArgs a = make_vec_args(pg);
     const dim3 grid((unsigned)pg->nctas), block(VP_NT);
     cudaStream_t s = pg->ctx->stream;
-    if (pg->solver == 2) SVM_CUDA(svm_launch_chained(al_vector_kernel<MODE>, grid, block, s, a, pg->al, (long long)(MODE == VP_INIT ? -1 : k)));
-    else if (pg->solver == 1) SVM_CUDA(svm_launch_chained(fw_vector_kernel<MODE>, grid, block, s, a, k));
+    if (pg->solver == SOLVER_AL) SVM_CUDA(svm_launch_chained(al_vector_kernel<MODE>, grid, block, s, a, pg->al, (long long)(MODE == VP_INIT ? -1 : k)));
+    else if (pg->solver == SOLVER_FW) SVM_CUDA(svm_launch_chained(fw_vector_kernel<MODE>, grid, block, s, a, k));
     else SVM_CUDA(svm_launch_chained(pg_vector_kernel<MODE>, grid, block, s, a, k));
     pg->ctx->launches++;
     return SVMB200_OK;
@@ -679,8 +683,8 @@ extern "C" int svmb200_pg_destroy(svmb200_pg* pg) {
     if (pg->ctx) {
         cudaSetDevice(pg->ctx->device);
         cudaStreamSynchronize(pg->ctx->stream);
-        if (pg->smo_hist) cudaFree(pg->smo_hist);
-        if (pg->smo_rows_buf) cudaFree(pg->smo_rows_buf);
+        if (pg->solver == SOLVER_SMO && pg->hist_f) cudaFree(pg->hist_f);
+        if (pg->smo.rows_buf) cudaFree(pg->smo.rows_buf);
         if (pg->slab_private) {
             if (pg->slab) cudaFree(pg->slab);
             if (pg->pinned) cudaFreeHost(pg->pinned);
@@ -697,7 +701,89 @@ extern "C" int svmb200_pg_destroy(svmb200_pg* pg) {
     return SVMB200_OK;
 }
 
-// host-side description of an augmented-Lagrangian solve (solver 2)
+// a solver under construction: destroyed (whatever it holds so far) unless creation succeeds and releases it
+struct PgDestroy {
+    void operator()(svmb200_pg* pg) const { svmb200_pg_destroy(pg); }
+};
+using PgGuard = std::unique_ptr<svmb200_pg, PgDestroy>;
+
+// Consecutive regions of one allocation, each rounded up to 256 bytes.  A layout is written once as a sequence of
+// take() calls: run on a Carve without a base it sizes the allocation, run on one with the allocation as base it places
+// the pointers.
+struct Carve {
+    unsigned char* base = nullptr;
+    size_t bytes = 0;
+    template <typename T>
+    void take(T*& p, size_t size) {
+        p = base ? reinterpret_cast<T*>(base + bytes) : nullptr;
+        bytes += (size + 255) & ~size_t(255);
+    }
+};
+
+// The solver's device slab of `bytes`, pinned poll block and event pair: the context's set, grown as needed, when
+// `may_share` and no other solver holds it; else a private set.  svmb200_pg_destroy releases either, also after a
+// failure part-way.
+static int acquire_workspace(svmb200_pg* pg, size_t bytes, bool may_share) {
+    svmb200_ctx* ctx = pg->ctx;
+    const bool shared = may_share && !ctx->pg_slab_busy;
+    pg->slab_private = !shared;
+    if (shared && ctx->pg_slab_bytes < bytes) {
+        SVM_CUDA(cudaStreamSynchronize(ctx->stream));
+        if (ctx->pg_slab) cudaFree(ctx->pg_slab);
+        ctx->pg_slab = nullptr;
+        ctx->pg_slab_bytes = 0;
+    }
+    void*& slab = shared ? ctx->pg_slab : pg->slab;
+    void*& pinned = shared ? ctx->pg_pinned : pg->pinned;
+    cudaEvent_t& ev0 = shared ? ctx->pg_ev0 : pg->ev0;
+    cudaEvent_t& ev1 = shared ? ctx->pg_ev1 : pg->ev1;
+    cudaEvent_t* ev_poll = shared ? ctx->pg_ev_poll : pg->ev_poll;
+    if (!slab) {
+        SVM_CUDA(cudaMalloc(&slab, bytes));
+        if (shared) ctx->pg_slab_bytes = bytes;
+    }
+    if (!pinned) SVM_CUDA(cudaMallocHost(&pinned, 256));
+    if (!ev0) SVM_CUDA(cudaEventCreate(&ev0));
+    if (!ev1) SVM_CUDA(cudaEventCreate(&ev1));
+    for (int i = 0; i < 2; ++i)
+        if (!ev_poll[i]) SVM_CUDA(cudaEventCreateWithFlags(&ev_poll[i], cudaEventDisableTiming));
+    if (shared) {
+        ctx->pg_slab_busy = true;
+        ctx->event_pool_used = 0;
+        pg->slab = ctx->pg_slab;
+        pg->pinned = ctx->pg_pinned;
+        pg->ev0 = ctx->pg_ev0;
+        pg->ev1 = ctx->pg_ev1;
+        pg->ev_poll[0] = ctx->pg_ev_poll[0];
+        pg->ev_poll[1] = ctx->pg_ev_poll[1];
+    }
+    static_assert(sizeof(PGDeviceState) <= POLL_SLOT_BYTES - sizeof(int), "poll slot too small");
+    pg->st_host = static_cast<PGDeviceState*>(pg->pinned);
+    return SVMB200_OK;
+}
+
+// the checks every creator makes first, in this order; `fn` (the creator) prefixes the messages
+static int check_create_args(const char* fn, svmb200_ctx* ctx, svmb200_pg** out, bool inputs, int64_t n,
+                             const char* too_small, bool ld_ok, const char* ld_msg, int hessian) {
+    SVM_TRY(svm_use(ctx));
+    const char* msg = nullptr;
+    if (out == nullptr) {
+        msg = "out is null";
+    } else {
+        *out = nullptr;
+        if (!inputs) msg = "null input";
+        else if (n <= 1) msg = too_small;
+        else if (!ld_ok) msg = ld_msg;
+        else if (hessian != SVMB200_HESSIAN_PLAIN && hessian != SVMB200_HESSIAN_SVR) msg = "bad hessian layout";
+    }
+    if (msg) {
+        svmb200_set_error("%s: %s", fn, msg);
+        return SVMB200_ERR_ARG;
+    }
+    return SVMB200_OK;
+}
+
+// host-side description of an augmented-Lagrangian solve (SOLVER_AL)
 struct ALSpec {
     ALParams p;
     const double* a_host;      // equality row or null
@@ -707,27 +793,27 @@ struct ALSpec {
 
 static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows, int hessian,
                        const double* q_host, const double* lb_host, const double* ub_host, const double* x0_host,
-                       double eps, int64_t max_iter, int solver, double fw_t, svmb200_pg** out,
+                       double eps, int64_t max_iter, SolverKind solver, double fw_t, svmb200_pg** out,
                        const ALSpec* al = nullptr, const double* sign_host = nullptr);
 
 extern "C" int svmb200_pg_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                                  int hessian, const double* q_host, const double* lb_host, const double* ub_host,
                                  const double* x0_host, double eps, int64_t max_iter, svmb200_pg** out) {
-    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, 0, 0.0, out);
+    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, SOLVER_PG, 0.0, out);
 }
 
 extern "C" int svmb200_fw_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                                  int hessian, const double* q_host, const double* lb_host, const double* ub_host,
                                  const double* x0_host, double eps, int64_t max_iter, double t, svmb200_pg** out) {
     SVM_CHECK_ARG(t >= 0.0 && t < 1.0, "t has to lie in [0, 1)");  // frank_wolfe.py:84-85
-    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, 1, t, out);
+    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, SOLVER_FW, t, out);
 }
 
 extern "C" int svmb200_pg_create_signed(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0,
                                         int64_t nrows, int hessian, const double* sign_host, const double* q_host,
                                         const double* lb_host, const double* ub_host, const double* x0_host, double eps,
                                         int64_t max_iter, svmb200_pg** out) {
-    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, 0, 0.0, out,
+    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, SOLVER_PG, 0.0, out,
                        nullptr, sign_host);
 }
 
@@ -736,21 +822,17 @@ extern "C" int svmb200_fw_create_signed(svmb200_ctx* ctx, const double* dQ, int6
                                         const double* lb_host, const double* ub_host, const double* x0_host, double eps,
                                         int64_t max_iter, double t, svmb200_pg** out) {
     SVM_CHECK_ARG(t >= 0.0 && t < 1.0, "t has to lie in [0, 1)");  // frank_wolfe.py:84-85
-    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, 1, t, out,
+    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, eps, max_iter, SOLVER_FW, t, out,
                        nullptr, sign_host);
 }
 
 static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows, int hessian,
                        const double* q_host, const double* lb_host, const double* ub_host, const double* x0_host,
-                       double eps, int64_t max_iter, int solver, double fw_t, svmb200_pg** out, const ALSpec* al,
+                       double eps, int64_t max_iter, SolverKind solver, double fw_t, svmb200_pg** out, const ALSpec* al,
                        const double* sign_host) {
-    SVM_TRY(svm_use(ctx));
-    SVM_CHECK_ARG(out != nullptr, "out is null");
-    *out = nullptr;
-    SVM_CHECK_ARG(dQ != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
-    SVM_CHECK_ARG(n > 1, "Q is too small");  // opti/_base.py:249-250
-    SVM_CHECK_ARG(ld >= n && ld % 2 == 0, "ld must be >= n and even");
-    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
+    // n > 1: opti/_base.py:249-250
+    SVM_TRY(check_create_args(__func__, ctx, out, dQ != nullptr && q_host != nullptr && ub_host != nullptr, n, "Q is too small",
+                              ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
     SVM_CHECK_ARG(max_iter > 0, "max_iter must be > 0");  // opti/_base.py:73-74
     SVM_CHECK_ARG(sign_host == nullptr || hessian == SVMB200_HESSIAN_PLAIN, "label signs need the plain layout");
     if (sign_host != nullptr) {
@@ -763,7 +845,8 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
         SVM_TRY(svmb200_shard_rows(n, ctx->rank, P, &exp_row0, &exp_rows));
         SVM_CHECK_ARG(row0 == exp_row0 && nrows == exp_rows, "row shard does not match svmb200_shard_rows");
     }
-    svmb200_pg* pg = new svmb200_pg();
+    PgGuard guard(new svmb200_pg());
+    svmb200_pg* pg = guard.get();
     pg->ctx = ctx;
     pg->dQ = dQ;
     pg->n = n;
@@ -797,129 +880,60 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
     pg->max_iter = max_iter;
     pg->hist_cap = max_iter + 1 < (1ll << 24) ? max_iter + 1 : (1ll << 24);
     const size_t nv = (size_t)pg->nvars * sizeof(double);
-    int rc = SVMB200_OK;
-    auto fail = [&](int code) {
-        svmb200_pg_destroy(pg);
-        return code;
-    };
-#define PG_CUDA(call)                                                                                  \
-    do {                                                                                               \
-        cudaError_t e__ = (call);                                                                      \
-        if (e__ != cudaSuccess) {                                                                      \
-            svmb200_set_error("%s:%d %s failed: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e__)); \
-            return fail(SVMB200_ERR_CUDA);                                                             \
-        }                                                                                              \
-    } while (0)
-    {
-        // one slab: x g d q lb ub (nvars each) | u (ld) | gathered (stride*P) | partials | two histories | state
-        auto up = [](size_t b) { return (b + 255) & ~size_t(255); };
-        const size_t sz_nv = up(nv), sz_u = up((size_t)ld * sizeof(double)), sz_w = up((size_t)(pg->stride * P) * sizeof(double));
-        const size_t sz_part = up(2 * 3 * VP_MAXC * sizeof(double)), sz_hist = up((size_t)pg->hist_cap * sizeof(double));
-        // augmented Lagrangian: + multipliers, rule state, previous step, pre-jump point, equality row (nvars each),
-        // four per-iteration scalar arrays (epochs + 1), double-buffered per-CTA sums, two slots of mu
-        const size_t sz_sched = up((size_t)(max_iter + 1) * sizeof(double));
-        const size_t sz_alpart = up(2 * AL_NSUMS * VP_MAXC * sizeof(double));
-        const size_t al_extra = solver == 2 ? 8 * sz_nv + 4 * sz_sched + sz_alpart + up(2 * sizeof(double)) : 0;
-        const size_t total = 7 * sz_nv + sz_u + sz_w + sz_part + 2 * sz_hist + up(sizeof(PGDeviceState)) + al_extra;
-        unsigned char* base = nullptr;
-        if (!ctx->pg_slab_busy) {
-            if (ctx->pg_slab_bytes < total) {
-                PG_CUDA(cudaStreamSynchronize(ctx->stream));
-                if (ctx->pg_slab) cudaFree(ctx->pg_slab);
-                ctx->pg_slab = nullptr;
-                ctx->pg_slab_bytes = 0;
-                PG_CUDA(cudaMalloc(&ctx->pg_slab, total));
-                ctx->pg_slab_bytes = total;
-            }
-            if (!ctx->pg_pinned) PG_CUDA(cudaMallocHost(&ctx->pg_pinned, 256));
-            if (!ctx->pg_ev0) PG_CUDA(cudaEventCreate(&ctx->pg_ev0));
-            if (!ctx->pg_ev1) PG_CUDA(cudaEventCreate(&ctx->pg_ev1));
-            for (cudaEvent_t& e : ctx->pg_ev_poll)
-                if (!e) PG_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            ctx->pg_slab_busy = true;
-            ctx->event_pool_used = 0;
-            pg->slab = ctx->pg_slab;
-            pg->slab_private = false;
-            pg->pinned = static_cast<unsigned char*>(ctx->pg_pinned);
-            pg->ev0 = ctx->pg_ev0;
-            pg->ev1 = ctx->pg_ev1;
-            pg->ev_poll[0] = ctx->pg_ev_poll[0];
-            pg->ev_poll[1] = ctx->pg_ev_poll[1];
-        } else {
-            pg->slab_private = true;  // a second live solver on the same context: private workspace
-            PG_CUDA(cudaMalloc(&pg->slab, total));
-            PG_CUDA(cudaMallocHost(&pg->pinned, 256));
-            PG_CUDA(cudaEventCreate(&pg->ev0));
-            PG_CUDA(cudaEventCreate(&pg->ev1));
-            for (cudaEvent_t& e : pg->ev_poll) PG_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        }
-        static_assert(sizeof(PGDeviceState) <= POLL_SLOT_BYTES - sizeof(int), "poll slot too small");
-        pg->st_host = reinterpret_cast<PGDeviceState*>(pg->pinned);
-        base = static_cast<unsigned char*>(pg->slab);
-        size_t off = 0;
-        auto take = [&](size_t b) { unsigned char* q = base + off; off += b; return reinterpret_cast<double*>(q); };
-        pg->x = take(sz_nv);
-        pg->g = take(sz_nv);
-        pg->d = take(sz_nv);
-        pg->q = take(sz_nv);
-        pg->lb = take(sz_nv);
-        pg->ub = take(sz_nv);
-        {
-            double* sg = take(sz_nv);
-            pg->sgn = sign_host ? sg : nullptr;
-        }
-        pg->u = take(sz_u);
-        pg->w = take(sz_w);
-        pg->part = take(sz_part);
-        pg->hist_f = take(sz_hist);
-        pg->hist_ng = take(sz_hist);
-        pg->st = reinterpret_cast<PGDeviceState*>(take(up(sizeof(PGDeviceState))));
-        if (solver == 2) {
+    const size_t sz_sched = (size_t)(max_iter + 1) * sizeof(double);
+    double *sgn = nullptr, *arow = nullptr;
+    auto layout = [&](Carve c) {
+        // x g d q lb ub signs (nvars each) | u (ld) | gathered (stride*P) | partials | two histories | state
+        for (double** v : {&pg->x, &pg->g, &pg->d, &pg->q, &pg->lb, &pg->ub, &sgn}) c.take(*v, nv);
+        c.take(pg->u, (size_t)ld * sizeof(double));
+        c.take(pg->w, (size_t)(pg->stride * P) * sizeof(double));
+        c.take(pg->part, 2 * 3 * VP_MAXC * sizeof(double));
+        c.take(pg->hist_f, (size_t)pg->hist_cap * sizeof(double));
+        c.take(pg->hist_ng, (size_t)pg->hist_cap * sizeof(double));
+        c.take(pg->st, sizeof(PGDeviceState));
+        if (solver == SOLVER_AL) {
+            // + multipliers, rule state, previous step, pre-jump point, equality row (nvars each), four per-iteration
+            // scalar arrays (epochs + 1), double-buffered per-CTA sums, two slots of mu
             ALArgs& A = pg->al;
-            A.p = al->p;
-            A.lam_lb = take(sz_nv);
-            A.lam_ub = take(sz_nv);
-            A.s1 = take(sz_nv);
-            A.s2 = take(sz_nv);
-            A.s3 = take(sz_nv);
-            A.step = take(sz_nv);
-            A.xpre = take(sz_nv);
-            double* arow = take(sz_nv);
-            A.A = al->a_host ? arow : nullptr;
-            double* sched = take(4 * sz_sched);
-            A.lr = sched;
-            A.mom = sched + sz_sched / sizeof(double);
-            A.bc1 = sched + 2 * (sz_sched / sizeof(double));
-            A.bc2 = sched + 3 * (sz_sched / sizeof(double));
-            A.part = take(sz_alpart);
-            A.mu = take(up(2 * sizeof(double)));
+            for (double** v : {&A.lam_lb, &A.lam_ub, &A.s1, &A.s2, &A.s3, &A.step, &A.xpre, &arow}) c.take(*v, nv);
+            for (const double** v : {&A.lr, &A.mom, &A.bc1, &A.bc2}) c.take(*v, sz_sched);
+            c.take(A.part, 2 * AL_NSUMS * VP_MAXC * sizeof(double));
+            c.take(A.mu, 2 * sizeof(double));
         }
+        return c.bytes;
+    };
+    SVM_TRY(acquire_workspace(pg, layout(Carve{}), true));
+    layout(Carve{static_cast<unsigned char*>(pg->slab)});
+    pg->sgn = sign_host ? sgn : nullptr;
+    if (solver == SOLVER_AL) {
+        pg->al.p = al->p;
+        pg->al.A = al->a_host ? arow : nullptr;
     }
     cudaStream_t s = ctx->stream;
-    PG_CUDA(cudaMemsetAsync(pg->st, 0, sizeof(PGDeviceState), s));
-    PG_CUDA(cudaMemsetAsync(pg->u, 0, (size_t)ld * sizeof(double), s));
-    PG_CUDA(cudaMemsetAsync(pg->w, 0, (size_t)(pg->stride * P) * sizeof(double), s));
-    PG_CUDA(cudaMemsetAsync(pg->part, 0, 2 * 3 * VP_MAXC * sizeof(double), s));
-    PG_CUDA(cudaMemsetAsync(pg->d, 0, nv, s));
-    PG_CUDA(cudaMemsetAsync(pg->g, 0, nv, s));
+    SVM_CUDA(cudaMemsetAsync(pg->st, 0, sizeof(PGDeviceState), s));
+    SVM_CUDA(cudaMemsetAsync(pg->u, 0, (size_t)ld * sizeof(double), s));
+    SVM_CUDA(cudaMemsetAsync(pg->w, 0, (size_t)(pg->stride * P) * sizeof(double), s));
+    SVM_CUDA(cudaMemsetAsync(pg->part, 0, 2 * 3 * VP_MAXC * sizeof(double), s));
+    SVM_CUDA(cudaMemsetAsync(pg->d, 0, nv, s));
+    SVM_CUDA(cudaMemsetAsync(pg->g, 0, nv, s));
     // bounds / start point: opti/constrained/_base.py:61-65 (lb = 0, x0 = (lb+ub)/2)
     std::vector<double> lbv((size_t)pg->nvars, 0.0), x0v((size_t)pg->nvars), u0((size_t)n);
     if (lb_host) memcpy(lbv.data(), lb_host, nv);
     for (int64_t i = 0; i < pg->nvars; ++i) x0v[i] = x0_host ? x0_host[i] : (lbv[i] + ub_host[i]) / 2;
     for (int64_t j = 0; j < n; ++j) u0[j] = pg->svr ? x0v[j] - x0v[j + n] : (sign_host ? sign_host[j] * x0v[j] : x0v[j]);
-    PG_CUDA(cudaMemcpyAsync(pg->q, q_host, nv, cudaMemcpyHostToDevice, s));
-    PG_CUDA(cudaMemcpyAsync(pg->ub, ub_host, nv, cudaMemcpyHostToDevice, s));
-    PG_CUDA(cudaMemcpyAsync(pg->lb, lbv.data(), nv, cudaMemcpyHostToDevice, s));
-    PG_CUDA(cudaMemcpyAsync(pg->x, x0v.data(), nv, cudaMemcpyHostToDevice, s));
-    PG_CUDA(cudaMemcpyAsync(pg->u, u0.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, s));
-    if (sign_host) PG_CUDA(cudaMemcpyAsync(pg->sgn, sign_host, nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->q, q_host, nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->ub, ub_host, nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->lb, lbv.data(), nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->x, x0v.data(), nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->u, u0.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (sign_host) SVM_CUDA(cudaMemcpyAsync(pg->sgn, sign_host, nv, cudaMemcpyHostToDevice, s));
     std::vector<double> sched;  // staging of the per-iteration scalars (augmented Lagrangian)
-    if (solver == 2) {
+    if (solver == SOLVER_AL) {
         ALArgs& A = pg->al;
         // multipliers, rule state, previous step: zero (rmsprop.py:93 starts its moving mean of g^2 at one)
-        PG_CUDA(cudaMemsetAsync(A.lam_lb, 0, 7 * (((nv + 255) & ~size_t(255))), s));
-        PG_CUDA(cudaMemsetAsync(A.part, 0, 2 * AL_NSUMS * VP_MAXC * sizeof(double), s));
-        PG_CUDA(cudaMemsetAsync(A.mu, 0, 2 * sizeof(double), s));
+        SVM_CUDA(cudaMemsetAsync(A.lam_lb, 0, reinterpret_cast<unsigned char*>(arow) - reinterpret_cast<unsigned char*>(A.lam_lb), s));
+        SVM_CUDA(cudaMemsetAsync(A.part, 0, 2 * AL_NSUMS * VP_MAXC * sizeof(double), s));
+        SVM_CUDA(cudaMemsetAsync(A.mu, 0, 2 * sizeof(double), s));
         const size_t ne = (size_t)max_iter + 1;
         sched.assign(4 * ne, 0.0);
         for (size_t k = 0; k < ne; ++k) {
@@ -929,19 +943,18 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
             sched[2 * ne + k] = 1.0 - pow(A.p.beta1, (double)(k + 1));
             sched[3 * ne + k] = 1.0 - pow(A.p.beta2, (double)(k + 1));
         }
-        PG_CUDA(cudaMemcpyAsync(const_cast<double*>(A.lr), sched.data(), ne * sizeof(double), cudaMemcpyHostToDevice, s));
-        PG_CUDA(cudaMemcpyAsync(const_cast<double*>(A.mom), sched.data() + ne, ne * sizeof(double), cudaMemcpyHostToDevice, s));
-        PG_CUDA(cudaMemcpyAsync(const_cast<double*>(A.bc1), sched.data() + 2 * ne, ne * sizeof(double), cudaMemcpyHostToDevice, s));
-        PG_CUDA(cudaMemcpyAsync(const_cast<double*>(A.bc2), sched.data() + 3 * ne, ne * sizeof(double), cudaMemcpyHostToDevice, s));
-        if (al->a_host) PG_CUDA(cudaMemcpyAsync(const_cast<double*>(A.A), al->a_host, nv, cudaMemcpyHostToDevice, s));
+        SVM_CUDA(cudaMemcpyAsync(const_cast<double*>(A.lr), sched.data(), ne * sizeof(double), cudaMemcpyHostToDevice, s));
+        SVM_CUDA(cudaMemcpyAsync(const_cast<double*>(A.mom), sched.data() + ne, ne * sizeof(double), cudaMemcpyHostToDevice, s));
+        SVM_CUDA(cudaMemcpyAsync(const_cast<double*>(A.bc1), sched.data() + 2 * ne, ne * sizeof(double), cudaMemcpyHostToDevice, s));
+        SVM_CUDA(cudaMemcpyAsync(const_cast<double*>(A.bc2), sched.data() + 3 * ne, ne * sizeof(double), cudaMemcpyHostToDevice, s));
+        if (al->a_host) SVM_CUDA(cudaMemcpyAsync(const_cast<double*>(A.A), al->a_host, nv, cudaMemcpyHostToDevice, s));
     }
-    PG_CUDA(cudaStreamSynchronize(s));  // staging vectors go out of scope
-    if (solver == 2 && pg->al.p.rule == AL_RMSPROP) {
+    SVM_CUDA(cudaStreamSynchronize(s));  // staging vectors go out of scope
+    if (solver == SOLVER_AL && pg->al.p.rule == AL_RMSPROP) {
         std::vector<double> ones((size_t)pg->nvars, 1.0);
-        PG_CUDA(cudaMemcpyAsync(pg->al.s1, ones.data(), nv, cudaMemcpyHostToDevice, s));
-        PG_CUDA(cudaStreamSynchronize(s));
+        SVM_CUDA(cudaMemcpyAsync(pg->al.s1, ones.data(), nv, cudaMemcpyHostToDevice, s));
+        SVM_CUDA(cudaStreamSynchronize(s));
     }
-#undef PG_CUDA
     pg->last_passes = 0;
     if (ctx->local_group && P > 1) {
         // one host thread drives every rank: it cannot issue a collective, and a vector launch that waits for a peer's
@@ -951,11 +964,11 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
         if (!pg->p2p) {
             svmb200_set_error("a single-process group needs the fused exchange: every rank must own rows of the matrix "
                               "(n > %lld) and the gathered buffers must fit the arena", (long long)((P - 1) * rpr));
-            return fail(SVMB200_ERR_ARG);
+            return SVMB200_ERR_ARG;
         }
         pg->deferred_start = true;
         pg->k_next = 0;
-        *out = pg;
+        *out = guard.release();
         return SVMB200_OK;
     }
     if (pg->p2p) {
@@ -965,22 +978,14 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
         // fused exchange would be correct between two solves only by timing.  (SVMB200_P2P_CREATE_BARRIER=0 removes it
         // for A/B timing; ~30 us per solve.)
         const char* ev = getenv("SVMB200_P2P_CREATE_BARRIER");
-        if (ev == nullptr || atoi(ev) != 0) {
-            rc = svm_comm_allgather(ctx, pg->w, 1);
-            if (rc != SVMB200_OK) return fail(rc);
-        }
+        if (ev == nullptr || atoi(ev) != 0) SVM_TRY(svm_comm_allgather(ctx, pg->w, 1));
     }
-    if (solver == 2) {
-        // sums of state 0 (no product needed: every launch of the loop is preceded by its own pass w = Q xe)
-        rc = launch_vec<VP_INIT>(pg, 0);
-    } else {
-        // g0 = Q x0 + q, first direction and its partial reductions
-        rc = pg_product(pg, false);
-        if (rc == SVMB200_OK) rc = launch_vec<VP_INIT>(pg, 0);
-    }
-    if (rc != SVMB200_OK) return fail(rc);
+    // augmented Lagrangian: sums of state 0 (no product needed: every launch of the loop is preceded by its own pass
+    // w = Q xe); the others: g0 = Q x0 + q, first direction and its partial reductions
+    if (solver != SOLVER_AL) SVM_TRY(pg_product(pg, false));
+    SVM_TRY(launch_vec<VP_INIT>(pg, 0));
     pg->k_next = 0;
-    *out = pg;
+    *out = guard.release();
     return SVMB200_OK;
 }
 
@@ -990,7 +995,7 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
 // a C1-sized solve).
 static int poll_enqueue(svmb200_pg* pg, int slot) {
     cudaStream_t s = pg->ctx->stream;
-    unsigned char* dst = pg->pinned + (size_t)slot * POLL_SLOT_BYTES;
+    unsigned char* dst = static_cast<unsigned char*>(pg->pinned) + (size_t)slot * POLL_SLOT_BYTES;
     SVM_CUDA(cudaMemcpyAsync(dst, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, s));
     int* fault = reinterpret_cast<int*>(dst + POLL_SLOT_BYTES - sizeof(int));
     *fault = 0;
@@ -1002,7 +1007,7 @@ static int poll_enqueue(svmb200_pg* pg, int slot) {
 
 static int poll_wait(svmb200_pg* pg, int slot) {
     SVM_CUDA(cudaEventSynchronize(pg->ev_poll[slot]));
-    unsigned char* src = pg->pinned + (size_t)slot * POLL_SLOT_BYTES;
+    unsigned char* src = static_cast<unsigned char*>(pg->pinned) + (size_t)slot * POLL_SLOT_BYTES;
     pg->st_host = reinterpret_cast<PGDeviceState*>(src);
     if (pg->st_host->done) pg->finished = true;
     if (*reinterpret_cast<const int*>(src + POLL_SLOT_BYTES - sizeof(int))) {
@@ -1018,7 +1023,32 @@ static int poll_wait(svmb200_pg* pg, int slot) {
 // A projected-gradient solve on one GPU whose matrix fits the shared memory of the SMs (n <= 2 016 on a B200) runs as
 // ONE cooperative launch (k_persistent.cuh) instead of two launches per iteration.  Same bits; SVMB200_PERSISTENT=0
 // keeps the two-kernel loop (A/B), SVMB200_PERSISTENT_GRID overrides the grid size (tests on the host emulation).
-constexpr size_t PK_SMEM_MAX = 221 * 1024;  // dynamic part; the kernel's static arrays take ~4 KB of the 227 KB
+// dynamic shared memory the cooperative kernels (this loop and SMO) may use: their static arrays take the rest of the 227 KB
+constexpr size_t COOP_SMEM_MAX = 221 * 1024;
+
+// Ready a cooperative launch of `kernel` on `grid` CTAs of `block` threads and `smem` bytes of dynamic shared memory: the
+// opt-in to COOP_SMEM_MAX (once per device and kernel), the check that such a grid can be co-resident (it cannot on a
+// partitioned GPU), and the context's grid barrier.  *fits tells whether the grid can run.
+template <auto kernel>
+static int cooperative_setup(svmb200_ctx* ctx, int grid, int block, size_t smem, bool* fits) {
+    *fits = true;
+#ifndef SVMB200_HOST_EMULATION
+    static bool configured[64] = {};
+    const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
+    if (!configured[dev]) {
+        SVM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM_MAX));
+        configured[dev] = true;
+    }
+    int per_sm = 0;
+    SVM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, block, smem));
+    *fits = (long long)per_sm * ctx->sm_count >= grid;
+#endif
+    if (*fits && !ctx->gbar) {
+        SVM_CUDA(cudaMalloc(&ctx->gbar, 256));
+        SVM_CUDA(cudaMemsetAsync(ctx->gbar, 0, 256, ctx->stream));
+    }
+    return SVMB200_OK;
+}
 
 struct PersistPlan {
     int grid = 0, rows_per_cta = 0;
@@ -1031,7 +1061,7 @@ static bool persistent_plan(const svmb200_pg* pg, int64_t budget, PersistPlan* p
         return ev == nullptr ? 1 : atoi(ev);
     }();
     const svmb200_ctx* ctx = pg->ctx;
-    if (!enabled || pg->solver != 0 || ctx->nranks != 1 || pg->profile || budget < 8) return false;
+    if (!enabled || pg->solver != SOLVER_PG || ctx->nranks != 1 || pg->profile || budget < 8) return false;
     if (pg->svr || pg->sgn != nullptr) return false;  // plain layout, no label-sign view (k_persistent.cuh)
     if (pg->ld > 2 * PK_NT * PK_UMAX || pg->nrows != pg->n) return false;
     int grid = ctx->sm_count;
@@ -1039,7 +1069,7 @@ static bool persistent_plan(const svmb200_pg* pg, int64_t budget, PersistPlan* p
     if (grid < 1 || grid < pg->nctas) return false;
     const int64_t rows = (pg->n + grid - 1) / grid;
     const size_t smem = (size_t)rows * pg->ld * sizeof(double);
-    if (rows > PK_RMAX || smem > PK_SMEM_MAX || pg->nctas > PK_VMAX) return false;
+    if (rows > PK_RMAX || smem > COOP_SMEM_MAX || pg->nctas > PK_VMAX) return false;
     plan->grid = grid;
     plan->rows_per_cta = (int)rows;
     plan->smem = smem;
@@ -1051,29 +1081,12 @@ static int launch_persistent(svmb200_pg* pg, const PersistPlan& plan, int64_t ni
     // scratch: two w buffers, two product buffers, grid - 1 private copies of u (ld each)
     const size_t doubles = 4 * (size_t)pg->ld + (size_t)(plan.grid - 1) * (size_t)pg->ld;
     SVM_TRY(svm_scratch_reserve(ctx, &ctx->persist_buf, &ctx->persist_bytes, doubles * sizeof(double)));
-    if (!ctx->gbar) {
-        SVM_CUDA(cudaMalloc(&ctx->gbar, 256));
-        SVM_CUDA(cudaMemsetAsync(ctx->gbar, 0, 256, ctx->stream));
+    bool fits = false;
+    SVM_TRY(cooperative_setup<pg_persistent_kernel>(ctx, plan.grid, PK_NT, plan.smem, &fits));
+    if (!fits) {
+        svmb200_set_error("persistent loop: %d CTAs cannot be co-resident", plan.grid);
+        return SVMB200_ERR_STATE;
     }
-#ifndef SVMB200_HOST_EMULATION
-    static bool configured[64] = {};  // per-device opt-in to the dynamic shared memory size
-    const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
-    if (!configured[dev]) {
-        SVM_CUDA(cudaFuncSetAttribute(pg_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PK_SMEM_MAX));
-        configured[dev] = true;
-    }
-#endif
-#ifndef SVMB200_HOST_EMULATION
-    {
-        // a cooperative grid must be co-resident: one CTA of this size per SM, `grid` SMs (fails on a partitioned GPU)
-        int per_sm = 0;
-        SVM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pg_persistent_kernel, PK_NT, plan.smem));
-        if ((long long)per_sm * ctx->sm_count < plan.grid) {
-            svmb200_set_error("persistent loop: %d CTAs cannot be co-resident", plan.grid);
-            return SVMB200_ERR_STATE;
-        }
-    }
-#endif
     PersistArgs a;
     a.Q = pg->dQ;
     a.ld = pg->ld;
@@ -1091,6 +1104,14 @@ static int launch_persistent(svmb200_pg* pg, const PersistPlan& plan, int64_t ni
     return SVMB200_OK;
 }
 
+// statistics of the run about to start (pooled profiling events: reused, never destroyed per run)
+static void reset_run_stats(svmb200_pg* pg) {
+    pg->mv_ev.clear();
+    pg->last_passes = 0;
+    pg->last_samples = 0;
+    pg->last_ms = pg->last_mv_ms = pg->last_comm_ms = pg->last_vec_ms = 0.f;
+}
+
 // The ranks of a single-process group (count > 1), or one solver (count == 1): `max_new` more iterations (< 0: to the
 // end).  Launches are enqueued ITERATION-MAJOR over the ranks -- every rank's product k, then every rank's vector launch
 // k -- so that in each stream a launch that waits for a peer's entries comes after that peer's product has been
@@ -1100,13 +1121,8 @@ static int run_many(svmb200_pg* const* pgs, int count, int64_t max_new) {
     for (int r = 0; r < count; ++r) {
         svmb200_pg* pg = pgs[r];
         SVM_TRY(svm_use(pg->ctx));
-        if (r == 0) {
-            pg->mv_ev.clear();  // pooled events: reused, never destroyed per run
-            pg->ctx->event_pool_used = 0;
-        }
-        pg->last_passes = 0;
-        pg->last_samples = 0;
-        pg->last_ms = pg->last_mv_ms = pg->last_comm_ms = pg->last_vec_ms = 0.f;
+        if (r == 0) pg->ctx->event_pool_used = 0;
+        reset_run_stats(pg);
         SVM_CUDA(cudaEventRecord(pg->ev0, pg->ctx->stream));
     }
     if (!p0->finished) {
@@ -1191,7 +1207,7 @@ static int run_many(svmb200_pg* const* pgs, int count, int64_t max_new) {
         if (!p0->finished) {
             // make the state at callback point k_next visible (f, |d|, stopping tests); the augmented Lagrangian
             // needs w = Q xe for that (value and gradient at xe), the box-constrained solvers carry g along
-            if (p0->solver == 2)
+            if (p0->solver == SOLVER_AL)
                 for (int ph = count > 1 ? 1 : 0; ph <= (count > 1 ? 2 : 0); ++ph)
                     for (int r = 0; r < count; ++r) {
                         SVM_TRY(svm_use(pgs[r]->ctx));
@@ -1232,7 +1248,7 @@ static int smo_run(svmb200_pg* pg, int64_t max_new);
 extern "C" int svmb200_pg_run(svmb200_pg* pg, int64_t max_new, int64_t* iter, int* status) {
     SVM_CHECK_ARG(pg != nullptr, "null solver");
     SVM_CHECK_ARG(!pg->deferred_start, "a solver of a single-process group runs through svmb200_pg_run_group");
-    SVM_TRY(pg->solver == 3 ? smo_run(pg, max_new) : run_many(&pg, 1, max_new));
+    SVM_TRY(pg->solver == SOLVER_SMO ? smo_run(pg, max_new) : run_many(&pg, 1, max_new));
     if (iter) *iter = pg->st_host->iter;
     if (status) *status = pg->st_host->done ? pg->st_host->status : SVMB200_STATUS_UNKNOWN;
     return SVMB200_OK;
@@ -1244,7 +1260,7 @@ static int check_group(svmb200_pg* const* pgs, int count) {
     for (int r = 0; r < count; ++r) {
         const svmb200_pg* p = pgs[r];
         SVM_CHECK_ARG(p != nullptr && p->ctx != nullptr, "null solver");
-        SVM_CHECK_ARG(p->solver != 3, "an SMO solver runs through svmb200_pg_run");
+        SVM_CHECK_ARG(p->solver != SOLVER_SMO, "an SMO solver runs through svmb200_pg_run");
         SVM_CHECK_ARG(p->ctx->local_group && p->ctx->nranks == count && p->ctx->rank == r,
                       "pass one solver per rank of the single-process group, in rank order");
         SVM_CHECK_ARG(p->n == pgs[0]->n && p->solver == pgs[0]->solver && p->max_iter == pgs[0]->max_iter &&
@@ -1258,7 +1274,7 @@ static int check_group(svmb200_pg* const* pgs, int count) {
 extern "C" int svmb200_pg_start_group(svmb200_pg* const* pgs, int count) {
     SVM_TRY(check_group(pgs, count));
     for (int r = 0; r < count; ++r) SVM_CHECK_ARG(pgs[r]->deferred_start, "solver already started");
-    if (pgs[0]->solver != 2)
+    if (pgs[0]->solver != SOLVER_AL)
         for (int ph = 1; ph <= 2; ++ph)
             for (int r = 0; r < count; ++r) {
                 SVM_TRY(svm_use(pgs[r]->ctx));
@@ -1344,14 +1360,14 @@ static int batch_product(svmb200_ctx* ctx, svmb200_pg* const* pgs, int count, Ba
 }
 
 template <int MODE>
-static int launch_vec_batch(svmb200_ctx* ctx, int solver, int nctas, int count, const VecArgs* dva, const ALArgs* dal,
+static int launch_vec_batch(svmb200_ctx* ctx, SolverKind solver, int nctas, int count, const VecArgs* dva, const ALArgs* dal,
                             long long k, const BatchExchange& bx) {
     const dim3 grid((unsigned)nctas, (unsigned)count);
     const unsigned tag = bx.p2p ? exchange_tag(bx.seq) : 0u;
     const int parity = bx.p2p ? (int)(bx.seq & 1) : 0;
     const dim3 block(VP_NT);
-    if (solver == 2) SVM_CUDA(svm_launch_chained(al_vector_batch_kernel<MODE>, grid, block, ctx->stream, dva, dal, k, tag, parity));
-    else if (solver == 1) SVM_CUDA(svm_launch_chained(fw_vector_batch_kernel<MODE>, grid, block, ctx->stream, dva, k, tag, parity));
+    if (solver == SOLVER_AL) SVM_CUDA(svm_launch_chained(al_vector_batch_kernel<MODE>, grid, block, ctx->stream, dva, dal, k, tag, parity));
+    else if (solver == SOLVER_FW) SVM_CUDA(svm_launch_chained(fw_vector_batch_kernel<MODE>, grid, block, ctx->stream, dva, k, tag, parity));
     else SVM_CUDA(svm_launch_chained(pg_vector_batch_kernel<MODE>, grid, block, ctx->stream, dva, k, tag, parity));
     ctx->launches++;
     return SVMB200_OK;
@@ -1385,7 +1401,7 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
     for (int b = 0; b < count; ++b) {
         const svmb200_pg* p = pgs[b];
         SVM_CHECK_ARG(p != nullptr, "null solver");
-        SVM_CHECK_ARG(p->solver != 3, "SMO solvers have no lockstep batch: run them one by one");
+        SVM_CHECK_ARG(p->solver != SOLVER_SMO, "SMO solvers have no lockstep batch: run them one by one");
         SVM_CHECK_ARG(p->ctx == p0->ctx && p->dQ == p0->dQ && p->n == p0->n && p->ld == p0->ld && p->row0 == p0->row0 &&
                           p->nrows == p0->nrows && p->svr == p0->svr,
                       "the solvers of a batch must share the resident matrix, its shard and its layout");
@@ -1408,17 +1424,15 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
     for (int b = 0; b < count; ++b) {
         pgs[b]->p2p = false;  // the members' own (single-solver) exchange path is not used from here on
         for (int c = 0; c < b; ++c) SVM_CHECK_ARG(pgs[c]->st_host != pgs[b]->st_host, "solvers share a state block");
-        pgs[b]->mv_ev.clear();
-        pgs[b]->last_passes = 0;
-        pgs[b]->last_ms = pgs[b]->last_mv_ms = pgs[b]->last_comm_ms = pgs[b]->last_vec_ms = 0.f;
+        reset_run_stats(pgs[b]);
     }
     // argument blocks of the vector kernels (constant over the run: only k changes from launch to launch)
-    const int solver = p0->solver;
+    const SolverKind solver = p0->solver;
     const size_t va_bytes = ((size_t)count * sizeof(VecArgs) + 255) & ~size_t(255);
-    const size_t al_bytes = solver == 2 ? (((size_t)count * sizeof(ALArgs) + 255) & ~size_t(255)) : 0;
+    const size_t al_bytes = solver == SOLVER_AL ? (((size_t)count * sizeof(ALArgs) + 255) & ~size_t(255)) : 0;
     SVM_TRY(svm_scratch_reserve(ctx, &ctx->batch_buf, &ctx->batch_bytes, va_bytes + al_bytes));
     VecArgs* dva = static_cast<VecArgs*>(ctx->batch_buf);
-    ALArgs* dal = solver == 2 ? reinterpret_cast<ALArgs*>(static_cast<unsigned char*>(ctx->batch_buf) + va_bytes) : nullptr;
+    ALArgs* dal = solver == SOLVER_AL ? reinterpret_cast<ALArgs*>(static_cast<unsigned char*>(ctx->batch_buf) + va_bytes) : nullptr;
     {
         std::vector<VecArgs> hv((size_t)count);
         for (int b = 0; b < count; ++b) {
@@ -1430,7 +1444,7 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
             }
         }
         SVM_CUDA(cudaMemcpyAsync(dva, hv.data(), (size_t)count * sizeof(VecArgs), cudaMemcpyHostToDevice, ctx->stream));
-        if (solver == 2) {
+        if (solver == SOLVER_AL) {
             std::vector<ALArgs> ha((size_t)count);
             for (int b = 0; b < count; ++b) ha[b] = pgs[b]->al;
             SVM_CUDA(cudaMemcpyAsync(dal, ha.data(), (size_t)count * sizeof(ALArgs), cudaMemcpyHostToDevice, ctx->stream));
@@ -1452,7 +1466,7 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
     }
     if (running > 0) {
         // state at callback point max_iter (see svmb200_pg_run): the epoch / iteration limit ends every problem left
-        if (solver == 2) SVM_TRY(batch_product(ctx, pgs, count, bx));
+        if (solver == SOLVER_AL) SVM_TRY(batch_product(ctx, pgs, count, bx));
         SVM_TRY(launch_vec_batch<VP_FINALISE>(ctx, solver, p0->nctas, count, dva, dal, k, bx));
         SVM_TRY(batch_poll(ctx, pgs, count, &running, bx));
     }
@@ -1474,16 +1488,22 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
     return SVMB200_OK;
 }
 
+// the device state block into st_host, once the work enqueued so far is done
+static int pull_state(svmb200_pg* pg) {
+    SVM_TRY(svm_use(pg->ctx));
+    SVM_CUDA(cudaMemcpyAsync(pg->st_host, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, pg->ctx->stream));
+    SVM_CUDA(cudaStreamSynchronize(pg->ctx->stream));
+    return SVMB200_OK;
+}
+
 extern "C" int svmb200_pg_state(svmb200_pg* pg, double* x_host, double* g_host, double* f, double* ng) {
     SVM_CHECK_ARG(pg != nullptr, "null solver");
-    SVM_TRY(svm_use(pg->ctx));
+    SVM_TRY(pull_state(pg));
     cudaStream_t s = pg->ctx->stream;
     const size_t nv = (size_t)pg->nvars * sizeof(double);
-    SVM_CUDA(cudaMemcpyAsync(pg->st_host, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, s));
-    SVM_CUDA(cudaStreamSynchronize(s));
     // augmented Lagrangian with Nesterov momentum: the device iterate is the next evaluation point (jump included);
     // when the optimality test ends the run the reference has not taken that jump yet
-    const bool pre_jump = pg->solver == 2 && pg->al.p.momentum_type == AL_MOM_NESTEROV && pg->st_host->done &&
+    const bool pre_jump = pg->solver == SOLVER_AL && pg->al.p.momentum_type == AL_MOM_NESTEROV && pg->st_host->done &&
                           pg->st_host->status == SVMB200_STATUS_OPTIMAL;
     if (x_host) SVM_CUDA(cudaMemcpyAsync(x_host, pre_jump ? pg->al.xpre : pg->x, nv, cudaMemcpyDeviceToHost, s));
     if (g_host) SVM_CUDA(cudaMemcpyAsync(g_host, pg->g, nv, cudaMemcpyDeviceToHost, s));
@@ -1495,10 +1515,7 @@ extern "C" int svmb200_pg_state(svmb200_pg* pg, double* x_host, double* g_host, 
 
 extern "C" int svmb200_pg_scalars(svmb200_pg* pg, double* vals6) {
     SVM_CHECK_ARG(pg != nullptr && vals6 != nullptr, "null argument");
-    SVM_TRY(svm_use(pg->ctx));
-    cudaStream_t s = pg->ctx->stream;
-    SVM_CUDA(cudaMemcpyAsync(pg->st_host, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, s));
-    SVM_CUDA(cudaStreamSynchronize(s));
+    SVM_TRY(pull_state(pg));
     vals6[0] = pg->st_host->f;
     vals6[1] = pg->st_host->ng;
     vals6[2] = pg->st_host->s;
@@ -1510,10 +1527,8 @@ extern "C" int svmb200_pg_scalars(svmb200_pg* pg, double* vals6) {
 
 extern "C" int svmb200_pg_history(svmb200_pg* pg, double* f_hist_host, double* ng_hist_host, int64_t* count) {
     SVM_CHECK_ARG(pg != nullptr, "null solver");
-    SVM_TRY(svm_use(pg->ctx));
+    SVM_TRY(pull_state(pg));
     cudaStream_t s = pg->ctx->stream;
-    SVM_CUDA(cudaMemcpyAsync(pg->st_host, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, s));
-    SVM_CUDA(cudaStreamSynchronize(s));
     int64_t cnt = pg->st_host->iter + 1;
     if (cnt > pg->hist_cap) cnt = pg->hist_cap;
     if (f_hist_host) SVM_CUDA(cudaMemcpyAsync(f_hist_host, pg->hist_f, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -1613,16 +1628,15 @@ extern "C" int svmb200_al_create_signed(svmb200_ctx* ctx, const double* dQ, int6
     spec.a_host = a_host;
     spec.lr_host = step_sizes;
     spec.mom_host = momentum_type == AL_MOM_NONE ? nullptr : momenta;
-    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, 0.0, epochs, 2, 0.0, out,
+    return bcqp_create(ctx, dQ, n, ld, row0, nrows, hessian, q_host, lb_host, ub_host, x0_host, 0.0, epochs, SOLVER_AL, 0.0, out,
                        &spec, sign_host);
 }
 
 extern "C" int svmb200_al_multipliers(svmb200_pg* pg, double* mu, double* lam_lb_host, double* lam_ub_host) {
-    SVM_CHECK_ARG(pg != nullptr && pg->solver == 2, "not an augmented-Lagrangian solver");
-    SVM_TRY(svm_use(pg->ctx));
+    SVM_CHECK_ARG(pg != nullptr && pg->solver == SOLVER_AL, "not an augmented-Lagrangian solver");
+    SVM_TRY(pull_state(pg));
     cudaStream_t s = pg->ctx->stream;
     const size_t nv = (size_t)pg->nvars * sizeof(double);
-    SVM_CUDA(cudaMemcpyAsync(pg->st_host, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, s));
     if (lam_lb_host) SVM_CUDA(cudaMemcpyAsync(lam_lb_host, pg->al.lam_lb, nv, cudaMemcpyDeviceToHost, s));
     if (lam_ub_host) SVM_CUDA(cudaMemcpyAsync(lam_ub_host, pg->al.lam_ub, nv, cudaMemcpyDeviceToHost, s));
     SVM_CUDA(cudaStreamSynchronize(s));
@@ -1640,10 +1654,9 @@ extern "C" int svmb200_al_multipliers(svmb200_pg* pg, double* mu, double* lam_lb
 // shared memory.
 constexpr int64_t SMO_CHUNK = 65536;
 constexpr int64_t SMO_MIN_SLICE = 128;
-constexpr size_t SMO_SMEM_MAX = 221 * 1024;
-constexpr int64_t SMO_SLICE_MAX = (int64_t)(SMO_SMEM_MAX / (SMO_ARRAYS * sizeof(double)));
+constexpr int64_t SMO_SLICE_MAX = (int64_t)(COOP_SMEM_MAX / (SMO_ARRAYS * sizeof(double)));
 
-static size_t smo_smem_bytes(const svmb200_pg* pg) { return (size_t)pg->smo_slice * SMO_ARRAYS * sizeof(double); }
+static size_t smo_smem_bytes(const svmb200_pg* pg) { return (size_t)pg->smo.a.slice * SMO_ARRAYS * sizeof(double); }
 
 // computed rows (K12): what svmb200_smo_create_rows adds to the resident solver
 struct SmoRowsSpec {
@@ -1679,7 +1692,8 @@ static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
     SVM_CHECK_ARG(grid >= 1, "SVMB200_SMO_GRID must be >= 1");
     int64_t slice = (nvars + grid - 1) / grid;
     if (slice > SMO_SLICE_MAX) slice = SMO_SLICE_MAX;
-    svmb200_pg* pg = new svmb200_pg();
+    PgGuard guard(new svmb200_pg());
+    svmb200_pg* pg = guard.get();
     pg->ctx = ctx;
     pg->dQ = dQ;
     pg->n = n;
@@ -1689,129 +1703,99 @@ static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
     pg->svr = hessian == SVMB200_HESSIAN_SVR;
     pg->nvars = nvars;
     pg->rows_per_rank = n;
-    pg->solver = 3;
+    pg->solver = SOLVER_SMO;
     pg->eps = tol;
     pg->max_iter = max_iter;
-    pg->smo_slice = (int)slice;
-    pg->smo_grid = (int)((nvars + slice - 1) / slice);
-    pg->slab_private = true;
-    if (rows) {
-        pg->smo_rows = SMO_ROWS_COMPUTED;
-        pg->smo_kf = rows->kf;
+    SmoSolver& smo = pg->smo;
+    SmoArgs& a = smo.a;
+    a.slice = (int)slice;
+    smo.grid = (int)((nvars + slice - 1) / slice);
+    smo.rows = rows ? SMO_ROWS_COMPUTED : SMO_ROWS_RESIDENT;
+    bool fits = false;
+    SVM_TRY((rows ? cooperative_setup<smo_persistent_kernel<SMO_ROWS_COMPUTED>>
+                  : cooperative_setup<smo_persistent_kernel<SMO_ROWS_RESIDENT>>)(ctx, smo.grid, SMO_NT, smo_smem_bytes(pg), &fits));
+    if (!fits) {
+        svmb200_set_error("SMO: %d CTAs of %zu bytes of shared memory cannot be co-resident", smo.grid, smo_smem_bytes(pg));
+        return SVMB200_ERR_ARG;
     }
-    auto fail = [&](int code) {
-        svmb200_pg_destroy(pg);
-        return code;
-    };
-#define SMO_CUDA(call)                                                                                 \
-    do {                                                                                               \
-        cudaError_t e__ = (call);                                                                      \
-        if (e__ != cudaSuccess) {                                                                      \
-            svmb200_set_error("%s:%d %s failed: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e__)); \
-            return fail(SVMB200_ERR_CUDA);                                                             \
-        }                                                                                              \
-    } while (0)
-#ifndef SVMB200_HOST_EMULATION
-    {
-        // a cooperative grid must be co-resident
-        static bool configured[64] = {};
-        const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
-        if (!configured[dev]) {
-            SMO_CUDA(cudaFuncSetAttribute(smo_persistent_kernel<SMO_ROWS_RESIDENT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)SMO_SMEM_MAX));
-            SMO_CUDA(cudaFuncSetAttribute(smo_persistent_kernel<SMO_ROWS_COMPUTED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)SMO_SMEM_MAX));
-            configured[dev] = true;
-        }
-        int per_sm = 0;
-        SMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-            &per_sm, rows ? smo_persistent_kernel<SMO_ROWS_COMPUTED> : smo_persistent_kernel<SMO_ROWS_RESIDENT>, SMO_NT,
-            smo_smem_bytes(pg)));
-        if ((long long)per_sm * ctx->sm_count < pg->smo_grid) {
-            svmb200_set_error("SMO: %d CTAs of %zu bytes of shared memory cannot be co-resident", pg->smo_grid, smo_smem_bytes(pg));
-            return fail(SVMB200_ERR_ARG);
-        }
-    }
-#endif
     // one private slab: alpha, G, signs, ub (nvars each) | candidate slots | state
-    auto up = [](size_t b) { return (b + 255) & ~size_t(255); };
-    const size_t nv = (size_t)nvars * sizeof(double), sz_nv = up(nv);
-    const size_t sz_cand = up((size_t)4 * pg->smo_grid * sizeof(SmoCand));
-    SMO_CUDA(cudaMalloc(&pg->slab, 4 * sz_nv + sz_cand + up(sizeof(PGDeviceState))));
-    SMO_CUDA(cudaMallocHost(&pg->pinned, 256));
-    SMO_CUDA(cudaEventCreate(&pg->ev0));
-    SMO_CUDA(cudaEventCreate(&pg->ev1));
-    for (cudaEvent_t& e : pg->ev_poll) SMO_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    pg->st_host = reinterpret_cast<PGDeviceState*>(pg->pinned);
-    unsigned char* base = static_cast<unsigned char*>(pg->slab);
-    pg->x = reinterpret_cast<double*>(base);
-    pg->g = reinterpret_cast<double*>(base + sz_nv);
-    pg->sgn = reinterpret_cast<double*>(base + 2 * sz_nv);
-    pg->ub = reinterpret_cast<double*>(base + 3 * sz_nv);
-    pg->smo_cand = reinterpret_cast<SmoCand*>(base + 4 * sz_nv);
-    pg->st = reinterpret_cast<PGDeviceState*>(base + 4 * sz_nv + sz_cand);
+    const size_t nv = (size_t)nvars * sizeof(double), cand_bytes = (size_t)4 * smo.grid * sizeof(SmoCand);
+    auto layout = [&](Carve c) {
+        for (double** v : {&pg->x, &pg->g, &pg->sgn, &pg->ub}) c.take(*v, nv);
+        c.take(a.cand, cand_bytes);
+        c.take(pg->st, sizeof(PGDeviceState));
+        return c.bytes;
+    };
+    SVM_TRY(acquire_workspace(pg, layout(Carve{}), false));
+    layout(Carve{static_cast<unsigned char*>(pg->slab)});
     // start: alpha = 0, G = q
     cudaStream_t s = ctx->stream;
-    SMO_CUDA(cudaMemsetAsync(pg->x, 0, nv, s));
-    SMO_CUDA(cudaMemcpyAsync(pg->g, q_host, nv, cudaMemcpyHostToDevice, s));
-    SMO_CUDA(cudaMemcpyAsync(pg->sgn, sign_host, nv, cudaMemcpyHostToDevice, s));
-    SMO_CUDA(cudaMemcpyAsync(pg->ub, ub_host, nv, cudaMemcpyHostToDevice, s));
-    SMO_CUDA(cudaMemsetAsync(pg->smo_cand, 0, sz_cand, s));
-    SMO_CUDA(cudaMemsetAsync(pg->st, 0, sizeof(PGDeviceState), s));
-    if (!ctx->gbar) {
-        SMO_CUDA(cudaMalloc(&ctx->gbar, 256));
-        SMO_CUDA(cudaMemsetAsync(ctx->gbar, 0, 256, s));
-    }
+    SVM_CUDA(cudaMemsetAsync(pg->x, 0, nv, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->g, q_host, nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->sgn, sign_host, nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(pg->ub, ub_host, nv, cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemsetAsync(a.cand, 0, cand_bytes, s));
+    SVM_CUDA(cudaMemsetAsync(pg->st, 0, sizeof(PGDeviceState), s));
     if (rows) {
         // cache geometry: every sample its own slot when all n rows fit, else sets of SMO_CACHE_WAYS (fewer if the
         // cache has fewer slots); cache_bytes = 0: no cache, every row is computed
         int64_t slots = (int64_t)(rows->cache_bytes / (nv > 0 ? nv : 1));
         if (slots >= n) {
-            pg->smo_sets = n;
-            pg->smo_ways = 1;
+            a.sets = n;
+            a.ways = 1;
         } else if (slots > 0) {
-            pg->smo_ways = slots < SMO_CACHE_WAYS ? slots : SMO_CACHE_WAYS;
-            pg->smo_sets = slots / pg->smo_ways;
+            a.ways = slots < SMO_CACHE_WAYS ? slots : SMO_CACHE_WAYS;
+            a.sets = slots / a.ways;
         }
-        slots = pg->smo_sets * pg->smo_ways;
-        const size_t sz_sq = up((size_t)n * sizeof(double)), sz_qij = up((size_t)2 * pg->smo_grid * sizeof(double));
-        const size_t sz_tags = up((size_t)pg->smo_grid * slots * sizeof(int));
-        const size_t sz_st = up((size_t)pg->smo_grid * slots * sizeof(long long)), sz_stats = 256;
-        const size_t sz_cache = (size_t)slots * nv;
-        SMO_CUDA(cudaMalloc(&pg->smo_rows_buf, sz_sq + sz_qij + sz_tags + sz_st + sz_stats + sz_cache));
-        unsigned char* rb = static_cast<unsigned char*>(pg->smo_rows_buf);
-        double* sqn = reinterpret_cast<double*>(rb);
-        pg->smo_qij = reinterpret_cast<double*>(rb + sz_sq);
-        pg->smo_tags = reinterpret_cast<int*>(rb + sz_sq + sz_qij);
-        pg->smo_stamps = reinterpret_cast<long long*>(rb + sz_sq + sz_qij + sz_tags);
-        pg->smo_stats = reinterpret_cast<unsigned long long*>(rb + sz_sq + sz_qij + sz_tags + sz_st);
-        pg->smo_cache = slots > 0 ? reinterpret_cast<double*>(rb + sz_sq + sz_qij + sz_tags + sz_st + sz_stats) : nullptr;
-        SMO_CUDA(cudaMemsetAsync(pg->smo_qij, 0, sz_qij, s));
-        SMO_CUDA(cudaMemsetAsync(pg->smo_tags, 0xff, sz_tags + sz_st, s));   // tag -1 (empty), stamp -1
-        SMO_CUDA(cudaMemsetAsync(pg->smo_stats, 0, sz_stats, s));
-        if (pg->smo_kf.kernel == SVMB200_KERNEL_GAUSSIAN) {
-            int rc = svm_row_sqnorms(ctx, pg->smo_kf.X, n, pg->smo_kf.ldx, pg->smo_kf.d, sqn);
-            if (rc != SVMB200_OK) return fail(rc);
-            pg->smo_kf.sqn = sqn;
+        slots = a.sets * a.ways;
+        // kernel of X, |x|^2, Q_ij slots, private tags and stamps per CTA, hit / miss count, row cache (sets x ways slots)
+        a.kf = rows->kf;
+        double* sqn = nullptr;
+        auto rows_layout = [&](Carve c) {
+            c.take(sqn, (size_t)n * sizeof(double));
+            c.take(a.qij, (size_t)2 * smo.grid * sizeof(double));
+            c.take(a.tags, (size_t)smo.grid * slots * sizeof(int));
+            c.take(a.stamps, (size_t)smo.grid * slots * sizeof(long long));
+            c.take(a.stats, 2 * sizeof(unsigned long long));
+            c.take(a.cache, (size_t)slots * nv);
+            return c.bytes;
+        };
+        SVM_CUDA(cudaMalloc(&smo.rows_buf, rows_layout(Carve{})));
+        rows_layout(Carve{static_cast<unsigned char*>(smo.rows_buf)});
+        if (slots == 0) a.cache = nullptr;
+        SVM_CUDA(cudaMemsetAsync(a.qij, 0, (size_t)2 * smo.grid * sizeof(double), s));
+        SVM_CUDA(cudaMemsetAsync(a.tags, 0xff, reinterpret_cast<unsigned char*>(a.stats) - reinterpret_cast<unsigned char*>(a.tags),
+                                 s));   // tag -1 (empty), stamp -1
+        SVM_CUDA(cudaMemsetAsync(a.stats, 0, 2 * sizeof(unsigned long long), s));
+        if (a.kf.kernel == SVMB200_KERNEL_GAUSSIAN) {
+            SVM_TRY(svm_row_sqnorms(ctx, a.kf.X, n, a.kf.ldx, a.kf.d, sqn));
+            a.kf.sqn = sqn;
         }
     }
-    SMO_CUDA(cudaStreamSynchronize(s));   // the host arrays belong to the caller
-#undef SMO_CUDA
+    SVM_CUDA(cudaStreamSynchronize(s));   // the host arrays belong to the caller
+    a.Q = dQ;
+    a.ld = ld;
+    a.n = n;
+    a.nvars = nvars;
+    a.svr = pg->svr;
+    a.x = pg->x;
+    a.g = pg->g;
+    a.sgn = pg->sgn;
+    a.ub = pg->ub;
+    a.gbar = ctx->gbar;
+    a.st = pg->st;
+    a.tol = tol;
+    a.max_iter = max_iter;
     pg->k_next = 0;
-    *out = pg;
+    *out = guard.release();
     return SVMB200_OK;
 }
 
 extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                                   int hessian, const double* sign_host, const double* q_host, const double* ub_host,
                                   double tol, int64_t max_iter, svmb200_pg** out) {
-    SVM_TRY(svm_use(ctx));
-    SVM_CHECK_ARG(out != nullptr, "out is null");
-    *out = nullptr;
-    SVM_CHECK_ARG(dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
-    SVM_CHECK_ARG(n > 1, "Q is too small");
-    SVM_CHECK_ARG(ld >= n && ld % 2 == 0, "ld must be >= n and even");
-    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
+    SVM_TRY(check_create_args(__func__, ctx, out, dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr,
+                              n, "Q is too small", ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
     SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
     return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, out);
 }
@@ -1820,14 +1804,10 @@ extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64
                                        double gamma, double coef0, double degree, int hessian, const double* sign_host,
                                        const double* q_host, const double* ub_host, double tol, int64_t max_iter,
                                        size_t cache_bytes, svmb200_pg** out) {
-    SVM_TRY(svm_use(ctx));
-    SVM_CHECK_ARG(out != nullptr, "out is null");
-    *out = nullptr;
-    SVM_CHECK_ARG(dX != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr, "null input");
-    SVM_CHECK_ARG(n > 1, "X is too small");
-    SVM_CHECK_ARG(d > 0 && ldx >= d && ldx % 2 == 0 && (reinterpret_cast<uintptr_t>(dX) & 15) == 0,
-                  "ldx must be even and >= d, X 16-byte aligned");
-    SVM_CHECK_ARG(hessian == SVMB200_HESSIAN_PLAIN || hessian == SVMB200_HESSIAN_SVR, "bad hessian layout");
+    SVM_TRY(check_create_args(__func__, ctx, out, dX != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr,
+                              n, "X is too small",
+                              d > 0 && ldx >= d && ldx % 2 == 0 && (reinterpret_cast<uintptr_t>(dX) & 15) == 0,
+                              "ldx must be even and >= d, X 16-byte aligned", hessian));
     SVM_CHECK_ARG(kernel >= SVMB200_KERNEL_LINEAR && kernel <= SVMB200_KERNEL_LAPLACIAN, "unknown kernel id");
     SVM_CHECK_ARG((kernel != SVMB200_KERNEL_GAUSSIAN && kernel != SVMB200_KERNEL_LAPLACIAN) || gamma >= 0.0,
                   "gamma must be >= 0 for the gaussian / laplacian kernels");
@@ -1847,21 +1827,23 @@ extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64
 }
 
 extern "C" int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses) {
-    SVM_CHECK_ARG(pg != nullptr && pg->solver == 3, "not an SMO solver");
+    SVM_CHECK_ARG(pg != nullptr && pg->solver == SOLVER_SMO, "not an SMO solver");
     SVM_TRY(svm_use(pg->ctx));
+    const SmoArgs& a = pg->smo.a;
     unsigned long long hm[2] = {0, 0};
-    if (pg->smo_rows == SMO_ROWS_COMPUTED) {
-        SVM_CUDA(cudaMemcpyAsync(hm, pg->smo_stats, sizeof(hm), cudaMemcpyDeviceToHost, pg->ctx->stream));
+    if (pg->smo.rows == SMO_ROWS_COMPUTED) {
+        SVM_CUDA(cudaMemcpyAsync(hm, a.stats, sizeof(hm), cudaMemcpyDeviceToHost, pg->ctx->stream));
         SVM_CUDA(cudaStreamSynchronize(pg->ctx->stream));
     }
-    if (computed) *computed = pg->smo_rows == SMO_ROWS_COMPUTED;
-    if (slots) *slots = pg->smo_sets * pg->smo_ways;
+    if (computed) *computed = pg->smo.rows == SMO_ROWS_COMPUTED;
+    if (slots) *slots = a.sets * a.ways;
     if (hits) *hits = (int64_t)hm[0];
     if (misses) *misses = (int64_t)hm[1];
     return SVMB200_OK;
 }
 
-// history buffers for states 0 .. need - 1: grown geometrically with the iterations actually run (max_iter may be 10^7)
+// history buffers for states 0 .. need - 1, one allocation (hist_f | hist_ng, hist_cap each): grown geometrically with the
+// iterations actually run (max_iter may be 10^7)
 static int smo_hist_reserve(svmb200_pg* pg, int64_t need) {
     if (need <= pg->hist_cap) return SVMB200_OK;
     int64_t cap = pg->hist_cap * 2 > need ? pg->hist_cap * 2 : need;
@@ -1870,13 +1852,12 @@ static int smo_hist_reserve(svmb200_pg* pg, int64_t need) {
     cudaStream_t s = pg->ctx->stream;
     double* h = nullptr;
     SVM_CUDA(cudaMalloc(&h, 2 * (size_t)cap * sizeof(double)));
-    if (pg->smo_hist) {
+    if (pg->hist_f) {
         SVM_CUDA(cudaMemcpyAsync(h, pg->hist_f, (size_t)pg->hist_cap * sizeof(double), cudaMemcpyDeviceToDevice, s));
         SVM_CUDA(cudaMemcpyAsync(h + cap, pg->hist_ng, (size_t)pg->hist_cap * sizeof(double), cudaMemcpyDeviceToDevice, s));
         SVM_CUDA(cudaStreamSynchronize(s));
-        SVM_CUDA(cudaFree(pg->smo_hist));
+        SVM_CUDA(cudaFree(pg->hist_f));
     }
-    pg->smo_hist = h;
     pg->hist_f = h;
     pg->hist_ng = h + cap;
     pg->hist_cap = cap;
@@ -1885,38 +1866,15 @@ static int smo_hist_reserve(svmb200_pg* pg, int64_t need) {
 
 // evaluate states k_next .. k_next + niter, stepping between them, unless the stopping test fires first
 static int smo_launch(svmb200_pg* pg, int64_t niter) {
-    SmoArgs a;
-    a.Q = pg->dQ;
-    a.ld = pg->ld;
-    a.n = pg->n;
-    a.nvars = pg->nvars;
-    a.svr = pg->svr;
-    a.slice = pg->smo_slice;
-    a.x = pg->x;
-    a.g = pg->g;
-    a.sgn = pg->sgn;
-    a.ub = pg->ub;
-    a.cand = pg->smo_cand;
-    a.gbar = pg->ctx->gbar;
-    a.st = pg->st;
+    SmoArgs& a = pg->smo.a;
     a.hist_f = pg->hist_f;
     a.hist_gap = pg->hist_ng;
     a.hist_cap = pg->hist_cap;
-    a.tol = pg->eps;
-    a.max_iter = pg->max_iter;
     a.k0 = pg->k_next;
     a.niter = niter;
-    a.kf = pg->smo_kf;
-    a.qij = pg->smo_qij;
-    a.cache = pg->smo_cache;
-    a.tags = pg->smo_tags;
-    a.stamps = pg->smo_stamps;
-    a.sets = pg->smo_sets;
-    a.ways = pg->smo_ways;
-    a.stats = pg->smo_stats;
-    SVM_CUDA(svm_launch_cooperative(pg->smo_rows == SMO_ROWS_COMPUTED ? smo_persistent_kernel<SMO_ROWS_COMPUTED>
+    SVM_CUDA(svm_launch_cooperative(pg->smo.rows == SMO_ROWS_COMPUTED ? smo_persistent_kernel<SMO_ROWS_COMPUTED>
                                                                         : smo_persistent_kernel<SMO_ROWS_RESIDENT>,
-                                    dim3((unsigned)pg->smo_grid), dim3(SMO_NT), smo_smem_bytes(pg), pg->ctx->stream, a));
+                                    dim3((unsigned)pg->smo.grid), dim3(SMO_NT), smo_smem_bytes(pg), pg->ctx->stream, a));
     pg->ctx->launches++;
     return SVMB200_OK;
 }
@@ -1924,9 +1882,7 @@ static int smo_launch(svmb200_pg* pg, int64_t niter) {
 static int smo_run(svmb200_pg* pg, int64_t max_new) {
     svmb200_ctx* ctx = pg->ctx;
     SVM_TRY(svm_use(ctx));
-    pg->last_passes = 0;   // no full pass over Q: an iteration reads two rows
-    pg->last_samples = 0;
-    pg->last_ms = pg->last_mv_ms = pg->last_comm_ms = pg->last_vec_ms = 0.f;
+    reset_run_stats(pg);   // last_passes stays 0: an iteration reads two rows, never a full pass over Q
     SVM_CUDA(cudaEventRecord(pg->ev0, ctx->stream));
     if (!pg->finished) {
         int64_t budget = pg->max_iter - pg->k_next;
