@@ -153,6 +153,18 @@ int svmb200_symv_plan_info(int64_t n, int64_t ld, int rank, int nranks, int sm_c
 int svmb200_symv_plan_items(int64_t n, int64_t ld, int rank, int nranks, int sm_count, int32_t* items7, int64_t capacity,
                             int64_t* count, int64_t* row0);
 
+/* ---- K2e: svmb200_matvec's product, BIT FOR BIT, from the upper triangle of an EXACTLY symmetric matrix ----------
+ * dw[i] = sum_j dQ[i][j] * du[j] for an n x n matrix with dQ[i][j] == dQ[j][i] bitwise (every self-Gram svmb200_gram
+ * builds, same = 1), in svmb200_matvec's summation order.  Needs at least two column segments of 8192 and the last one
+ * holding real rows (ld < n + 8192).  The lower triangle off the 8192 x 8192 diagonal blocks is never read.
+ *   svmb200_pg_set_self_gram(pg, 1) tells a solver that its matrix is such a self-Gram: on one rank, without the
+ *   opt-in symmetric pass, its products then take this pass (SVMB200_EXACT_SYMV=0 keeps svmb200_matvec's).
+ *   svmb200_pg_is_exact_symv reports what a solver does.                                                          */
+int svmb200_matvec_exact(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw);
+/* bytes one such pass moves: matrix elements read (diagonal blocks in full + the blocks to their right) and the column
+ * chains written and read back; *items = work items of the tile pass.  Any output pointer may be NULL. */
+int svmb200_exact_symv_geometry(int64_t n, int64_t ld, int64_t* matrix_bytes, int64_t* scratch_bytes, int64_t* items);
+
 /* ---- K2+K3(+K4): projected-gradient solve of the box-constrained QP -------------------------
  * Replaces  BoxConstrainedQuadraticOptimizer.__init__ (opti/constrained/_base.py:59-73) +
  * ProjectedGradient.minimize (opti/constrained/projected_gradient.py:76-143).
@@ -225,6 +237,8 @@ int svmb200_pg_set_profile(svmb200_pg* pg, int on);
 int svmb200_pg_stats_ex(svmb200_pg* pg, float* matvec_ms, float* comm_ms, float* vector_ms);
 int svmb200_pg_profile_samples(svmb200_pg* pg, int64_t* samples);
 int svmb200_pg_is_symmetric(svmb200_pg* pg, int* on);   /* 1: products from the upper triangle (K2s above) */
+int svmb200_pg_set_self_gram(svmb200_pg* pg, int on);    /* the matrix is a self-Gram of svmb200_gram (K2e above) */
+int svmb200_pg_is_exact_symv(svmb200_pg* pg, int* on);   /* 1: products from the upper triangle with K2's bits (K2e) */
 int svmb200_pg_device_x(svmb200_pg* pg, double** dx); /* device pointer of the iterate (nvars)     */
 int svmb200_pg_destroy(svmb200_pg* pg);
 

@@ -84,6 +84,10 @@ PROTOTYPES = {
     'svmb200_pg_profile_samples': [c_vp, C.POINTER(i64)],
     'svmb200_pg_device_x': [c_vp, C.POINTER(c_vp)],
     'svmb200_pg_is_symmetric': [c_vp, C.POINTER(C.c_int)],
+    'svmb200_pg_set_self_gram': [c_vp, C.c_int],
+    'svmb200_pg_is_exact_symv': [c_vp, C.POINTER(C.c_int)],
+    'svmb200_matvec_exact': [c_vp, c_vp, i64, i64, c_vp, c_vp],
+    'svmb200_exact_symv_geometry': [i64, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)],
     'svmb200_symv': [c_vp, c_vp, i64, i64, c_vp, c_vp],
     'svmb200_ctx_set_symmetric': [c_vp, C.c_int],
     'svmb200_ctx_get_symmetric': [c_vp, C.POINTER(C.c_int)],

@@ -356,6 +356,7 @@ gram_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
         const long long tile_r0 = p.row0 + (long long)tm * BM, tile_c0 = (long long)tn * BN;
         const bool edge = tile_r0 + BM > p.row0 + p.nrows || tile_c0 + BN > p.nb ||
                           (p.same && tile_r0 < tile_c0 + BN && tile_c0 < tile_r0 + BM);
+        const bool tile_lower = tile_r0 >= tile_c0 + BN;   // an interior tile of a self-Gram lies wholly below the diagonal
         const uint64_t out_policy = l2_evict_first_policy();
         auto epilogue = [&](auto edge_tag) {
             constexpr bool EDGE = decltype(edge_tag)::value;
@@ -368,14 +369,18 @@ gram_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
                 double* orow = p.out + (i - p.row0) * p.ldo;
                 double val[8];
                 if (KERNEL == SVMB200_KERNEL_GAUSSIAN) {
-                    // D = (-2<a,b> + |a|^2) + |b|^2 ; clamp ; exact zero on the diagonal of a self-Gram
+                    // D = (-2<a,b> + |a|^2) + |b|^2 ; clamp ; exact zero on the diagonal of a self-Gram.  In a self-Gram
+                    // the norm of the smaller global index goes inside the fma, so out[t][s] == out[s][t] bit for bit
+                    // (the upper triangle is sklearn's order; the lower one is its mirror)
                     const double na = sm_na[rl];
                     double x[8];
 #pragma unroll
                     for (int ni = 0; ni < 4; ++ni)
 #pragma unroll
                         for (int e = 0; e < 2; ++e) {
-                            double dist = __dadd_rn(fma(-2.0, acc[mi][ni][e], na), nbv[ni][e]);  // -2<a,b> is exact
+                            const bool lower = p.same && (EDGE ? i > col_base + ni * 8 + e : tile_lower);
+                            const double nlo = lower ? nbv[ni][e] : na, nhi = lower ? na : nbv[ni][e];
+                            double dist = __dadd_rn(fma(-2.0, acc[mi][ni][e], nlo), nhi);  // -2<a,b> is exact
                             dist = dist < 0.0 ? 0.0 : dist;  // np.maximum(D, 0); select instead of fmax(), see exp8
                             if (EDGE && p.same && (i == col_base + ni * 8 + e)) dist = 0.0;
                             x[ni * 2 + e] = __dmul_rn(-p.gamma, dist);

@@ -16,7 +16,12 @@
 constexpr int MV_R = 4;
 constexpr int MV_NT = 256;
 constexpr int MV_U = 4;
-constexpr int MV_SEG = 8192;
+// the segment width is a build-time knob for the host emulation only (small problems with several segments); the sm_100a
+// build uses 8192
+#ifndef SVMB200_MV_SEG
+#define SVMB200_MV_SEG 8192
+#endif
+constexpr int MV_SEG = SVMB200_MV_SEG;
 constexpr int MV_MINB = 3;
 constexpr int MV_GROUP = 64;            // rows per group (one u'w share per group)
 constexpr int ROW_ALIGN = MV_GROUP;     // row shards start on multiples of this, see svmb200_shard_rows

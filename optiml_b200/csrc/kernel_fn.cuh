@@ -6,7 +6,8 @@
 //            features 2s, 2s+1, 2s+8, 2s+9 (the k-slots 0..3 of K1's fragments, see gram.cu) -- one fma chain in that
 //            order, which is how the host emulation evaluates K1's DMMA.  Whether the B200's DMMA rounds as that chain
 //            does is measured, not assumed (tests/test_gpu_smo_rows.py).
-//   gaussian exp(-gamma max(0, fma(-2, dot, |x_s|^2) + |x_t|^2)), distance 0 when s == t; |x|^2 from K1's row_sqnorm_kernel
+//   gaussian exp(-gamma max(0, fma(-2, dot, |x_lo|^2) + |x_hi|^2)), lo = min(s, t), hi = max(s, t), distance 0 when
+//            s == t; |x|^2 from K1's row_sqnorm_kernel
 //   poly     (gamma dot + coef0)^degree: ipow_rn for integer degrees in [1, 64], pow otherwise
 //   sigmoid  tanh(gamma dot + coef0)
 //   laplacian exp(-gamma sum_k |x_sk - x_tk|), summed in feature order (laplacian_kernel)
@@ -155,7 +156,8 @@ __device__ __forceinline__ double kfn_value(const KernelFn& p, long long s, long
     }
     const double dot = kfn_dot(xs, xt, p.d);
     if (p.kernel == SVMB200_KERNEL_GAUSSIAN) {
-        double dist = __dadd_rn(fma(-2.0, dot, __ldg(p.sqn + s)), __ldg(p.sqn + t));
+        const long long lo = s < t ? s : t, hi = s < t ? t : s;   // K1's self-Gram order: exactly symmetric
+        double dist = __dadd_rn(fma(-2.0, dot, __ldg(p.sqn + lo)), __ldg(p.sqn + hi));
         dist = dist < 0.0 ? 0.0 : dist;
         if (s == t) dist = 0.0;
         return exp1(__dmul_rn(-p.gamma, dist));

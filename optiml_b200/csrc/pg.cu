@@ -15,6 +15,7 @@
 #include "al_math.cuh"
 #include "k2_matvec.cuh"   // K2, K2 x NB (device code)
 #include "k2_symv.cuh"     // K2s: one pass over the upper triangle of a symmetric matrix (opt-in)
+#include "k2_exact.cuh"    // K2e: K2's bits from the upper triangle of an exactly symmetric matrix
 #include "k3_vector.cuh"   // K3 vector phases and kernel entry points (device code)
 #include "k_persistent.cuh"  // the whole loop in one cooperative kernel, matrix in shared memory (small problems)
 #include "k_smo.cuh"         // K11: SMO with the equality constraint, one cooperative kernel for many iterations
@@ -36,6 +37,11 @@ struct MatvecScratch {
     int64_t sy_n = -1, sy_ld = -1;
     int sy_rank = -1, sy_P = -1;
     SymvPlan sy_plan;
+    // K2e: column chains and the (A, B) segment pairs of the grid, for ex_nseg segments
+    double* ex_colchain = nullptr;
+    int2* ex_pairs = nullptr;
+    size_t ex_cc_elems = 0, ex_pair_cap = 0;
+    int ex_nseg = -1;
 };
 
 static int matvec_scratch_reserve(svmb200_ctx* ctx, MatvecScratch& s, int64_t nrows, int64_t ld, int nvec = 1) {
@@ -355,9 +361,134 @@ void svm_release_matvec_scratch(svmb200_ctx* ctx) {
         if (s->sy_colpart) cudaFree(s->sy_colpart);
         if (s->sy_items) cudaFree(s->sy_items);
         if (s->sy_nseg) cudaFree(s->sy_nseg);
+        if (s->ex_colchain) cudaFree(s->ex_colchain);
+        if (s->ex_pairs) cudaFree(s->ex_pairs);
         delete s;
         ctx->matvec_scratch = nullptr;
     }
+}
+
+// ------------------------------------------------------------------------------------------ K2e launcher
+// w = Q u with K2's bits from the upper triangle of an exactly symmetric n x n matrix (see k2_exact.cuh); same outputs as
+// launch_matvec on one rank (w, and the shares of u'w per 64-row group when du_rows / ddenpart are given).
+static int exact_nseg(int64_t ld) { return (int)((ld + MV_SEG - 1) / MV_SEG); }
+
+// at least two segments, and every segment but the last one made of real rows (the column chains of a segment cover all
+// of its rows)
+static bool exact_shape_ok(int64_t n, int64_t ld) {
+    const int nseg = exact_nseg(ld);
+    return n > 0 && ld >= n && ld % 2 == 0 && nseg >= 2 && n > (int64_t)(nseg - 1) * MV_SEG;
+}
+
+// (A, B) segment pairs, B >= A, in launch order: the full off-diagonal blocks first, the diagonal blocks last
+static std::vector<int2> exact_pairs(int nseg) {
+    std::vector<int2> v;
+    for (int A = 0; A < nseg; ++A)
+        for (int B = A + 1; B < nseg - 1; ++B) v.push_back(make_int2(A, B));
+    for (int A = 0; A < nseg - 1; ++A) v.push_back(make_int2(A, nseg - 1));
+    for (int A = 0; A < nseg; ++A) v.push_back(make_int2(A, A));
+    return v;
+}
+
+static int exact_scratch_reserve(svmb200_ctx* ctx, MatvecScratch& s, int64_t n, int64_t ld) {
+    SVM_TRY(matvec_scratch_reserve(ctx, s, n, ld));
+    const int nseg = exact_nseg(ld);
+    const size_t need_c = (size_t)exact_colchain_off(nseg - 1, ld), need_p = (size_t)nseg * (nseg + 1) / 2;
+    if (need_c > s.ex_cc_elems || need_p > s.ex_pair_cap) {
+        SVM_CUDA(cudaStreamSynchronize(ctx->stream));
+        if (s.ex_colchain) cudaFree(s.ex_colchain);
+        if (s.ex_pairs) cudaFree(s.ex_pairs);
+        s.ex_colchain = nullptr;
+        s.ex_pairs = nullptr;
+        s.ex_cc_elems = s.ex_pair_cap = 0;
+        s.ex_nseg = -1;
+        SVM_CUDA(cudaMalloc(&s.ex_colchain, need_c * sizeof(double)));
+        s.ex_cc_elems = need_c;
+        SVM_CUDA(cudaMalloc(&s.ex_pairs, need_p * sizeof(int2)));
+        s.ex_pair_cap = need_p;
+    }
+    if (s.ex_nseg != nseg) {
+        const std::vector<int2> pairs = exact_pairs(nseg);
+        SVM_CUDA(cudaMemcpyAsync(s.ex_pairs, pairs.data(), pairs.size() * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream));
+        SVM_CUDA(cudaStreamSynchronize(ctx->stream));  // once per segment count; the table stays valid for every later pass
+        s.ex_nseg = nseg;
+    }
+    return SVMB200_OK;
+}
+
+static int launch_matvec_exact(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw,
+                               const double* du_rows, double* ddenpart, const int* d_done) {
+    using S = ExactDefault;
+    if (!exact_shape_ok(n, ld)) {
+        svmb200_set_error("matvec_exact: needs an even ld >= n, two segments of %d columns or more and n > ld - %d",
+                          MV_SEG, MV_SEG);
+        return SVMB200_ERR_ARG;
+    }
+    if ((reinterpret_cast<uintptr_t>(dQ) & 15) || (reinterpret_cast<uintptr_t>(du) & 15)) {
+        svmb200_set_error("matvec_exact: operands must be 16-byte aligned");
+        return SVMB200_ERR_ARG;
+    }
+    if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
+    MatvecScratch& s = *static_cast<MatvecScratch*>(ctx->matvec_scratch);
+    SVM_TRY(exact_scratch_reserve(ctx, s, n, ld));
+    const int nseg = exact_nseg(ld);
+    const long long nrows_pad = round_up64(n, 16);
+    ExactArgs a;
+    a.Q = dQ;
+    a.ld = ld;
+    a.n = n;
+    a.nrows_pad = nrows_pad;
+    a.u = du;
+    a.wpart = s.wpart;
+    a.colchain = s.ex_colchain;
+    a.pairs = s.ex_pairs;
+    a.done = d_done;
+    static bool attr_set[64] = {};   // per device: the ring needs more than the default 48 KB of dynamic shared memory
+    const bool tracked = ctx->device >= 0 && ctx->device < 64;
+    if (!tracked || !attr_set[ctx->device]) {
+        SVM_CUDA(cudaFuncSetAttribute(matvec_exact_tile_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::RING_BYTES));
+        if (tracked) attr_set[ctx->device] = true;
+    }
+    const unsigned nitems = (unsigned)((size_t)nseg * (nseg + 1) / 2 * MV_NT);
+    SVM_CUDA(svm_launch_chained_smem(matvec_exact_tile_kernel<S>, dim3(nitems), dim3(MV_NT), (size_t)S::RING_BYTES, ctx->stream, a));
+    ctx->launches++;
+    ExactCombineArgs c;
+    c.wpart = s.wpart;
+    c.colchain = s.ex_colchain;
+    c.ld = ld;
+    c.nrows = n;
+    c.nrows_pad = nrows_pad;
+    c.nseg = nseg;
+    c.u_rows = du_rows;
+    c.w = dw;
+    c.denpart = ddenpart;
+    c.done = d_done;
+    SVM_CUDA(svm_launch_chained(matvec_exact_combine_kernel, dim3((unsigned)((n + MV_GROUP - 1) / MV_GROUP)), dim3(MV_NT),
+                                ctx->stream, c));
+    ctx->launches++;
+    return SVMB200_OK;
+}
+
+extern "C" int svmb200_matvec_exact(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw) {
+    SVM_TRY(svm_use(ctx));
+    SVM_CHECK_ARG(dQ != nullptr && du != nullptr && dw != nullptr, "null operand");
+    return launch_matvec_exact(ctx, dQ, n, ld, du, dw, nullptr, nullptr, nullptr);
+}
+
+extern "C" int svmb200_exact_symv_geometry(int64_t n, int64_t ld, int64_t* matrix_bytes, int64_t* scratch_bytes,
+                                           int64_t* items) {
+    SVM_CHECK_ARG(exact_shape_ok(n, ld), "the exact symmetric pass does not apply to this shape");
+    const int nseg = exact_nseg(ld);
+    int64_t elems = 0;
+    for (const int2 pr : exact_pairs(nseg)) {
+        const int64_t rowsA = std::min<int64_t>((int64_t)(pr.x + 1) * MV_SEG, n) - (int64_t)pr.x * MV_SEG;
+        const int64_t colsB = std::min<int64_t>((int64_t)(pr.y + 1) * MV_SEG, ld) - (int64_t)pr.y * MV_SEG;
+        elems += rowsA * colsB;
+    }
+    if (matrix_bytes) *matrix_bytes = 8 * elems;
+    if (scratch_bytes) *scratch_bytes = 2 * 8 * exact_colchain_off(nseg - 1, ld);   // written by the tile pass, read by the combine
+    if (items) *items = (int64_t)exact_pairs(nseg).size() * MV_NT;
+    return SVMB200_OK;
 }
 
 int svm_launch_matvec(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, const double* du, double* dw,
@@ -507,6 +638,7 @@ struct svmb200_pg {
     int64_t stride = 0;  // rows_per_rank results + rows_per_rank / MV_GROUP shares of u'w
     bool p2p = false;           // fused exchange through the peer arena instead of ncclAllGather
     bool symmetric = false;     // products from the upper triangle only (K2s; one rank holding the whole matrix)
+    bool exact = false;         // products from the upper triangle with K2's bits (K2e; svmb200_pg_set_self_gram)
     unsigned long long cur_seq = 0;  // sequence number of the product the next vector kernel consumes
     int nctas = 1;
     double *q = nullptr, *lb = nullptr, *ub = nullptr;
@@ -639,6 +771,9 @@ static int pg_product(svmb200_pg* pg, bool timed, int phase = 0) {
         if (pg->symmetric) {
             SVM_TRY(launch_symv(ctx, pg->dQ, pg->n, pg->ld, pg->n, pg->u, wshard, pg->u, wshard + pg->rows_per_rank,
                                 &pg->st->done));
+        } else if (pg->exact) {
+            SVM_TRY(launch_matvec_exact(ctx, pg->dQ, pg->n, pg->ld, pg->u, wshard, pg->u, wshard + pg->rows_per_rank,
+                                        &pg->st->done));
         } else {
             SVM_TRY(launch_matvec(ctx, pg->dQ, pg->nrows, pg->ld, pg->u, wshard, pg->u + pg->row0,
                                   wshard + pg->rows_per_rank, &pg->st->done));
@@ -1573,6 +1708,36 @@ extern "C" int svmb200_pg_set_profile(svmb200_pg* pg, int on) {
 extern "C" int svmb200_pg_is_symmetric(svmb200_pg* pg, int* on) {
     SVM_CHECK_ARG(pg != nullptr && on != nullptr, "null argument");
     *on = pg->symmetric ? 1 : 0;
+    return SVMB200_OK;
+}
+
+// The solver's matrix is a self-Gram svmb200_gram built (same = 1): exactly symmetric.  On one rank holding the whole
+// matrix, without the opt-in symmetric pass, the products then come from its upper triangle with K2's bits (K2e), which
+// reads ~60 % of the bytes at n = 50 000.  Products already taken by K2 (the first one, at creation) have the same bits.
+// SVMB200_EXACT_SYMV=0 keeps K2 (A/B runs).  When the scratch of the column chains cannot be allocated, the solver
+// keeps K2 as well.
+extern "C" int svmb200_pg_set_self_gram(svmb200_pg* pg, int on) {
+    SVM_CHECK_ARG(pg != nullptr, "null solver");
+    const char* ev = getenv("SVMB200_EXACT_SYMV");
+    const bool allowed = ev == nullptr || atoi(ev) != 0;
+    pg->exact = on != 0 && allowed && pg->solver != SOLVER_SMO && pg->ctx->nranks == 1 && pg->row0 == 0 &&
+                pg->nrows == pg->n && !pg->symmetric && exact_shape_ok(pg->n, pg->ld) &&
+                (reinterpret_cast<uintptr_t>(pg->dQ) & 15) == 0;
+    if (pg->exact) {
+        svmb200_ctx* ctx = pg->ctx;
+        SVM_TRY(svm_use(ctx));
+        if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
+        if (exact_scratch_reserve(ctx, *static_cast<MatvecScratch*>(ctx->matvec_scratch), pg->n, pg->ld) != SVMB200_OK) {
+            (void)cudaGetLastError();   // an out-of-memory error is not sticky
+            pg->exact = false;
+        }
+    }
+    return SVMB200_OK;
+}
+
+extern "C" int svmb200_pg_is_exact_symv(svmb200_pg* pg, int* on) {
+    SVM_CHECK_ARG(pg != nullptr && on != nullptr, "null argument");
+    *on = pg->exact ? 1 : 0;
     return SVMB200_OK;
 }
 

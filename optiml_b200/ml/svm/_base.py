@@ -206,6 +206,7 @@ class SVM(BaseEstimator):
                 N.call('svmb200_gram', part.ctx.handle, C.c_void_p(dXr.dptr), n, dXr.ld, C.c_void_p(dXr.dptr), n, dXr.ld, d, 1,
                        kid, gamma, coef0, degree, sp, sp, float(bias), part.row0, part.nrows, C.c_void_p(part.matrix.dptr),
                        part.ld)
+                part.matrix.self_gram = True
             ctx.group.sync()
             for m in copies + [v for v in sign_copies if v is not None]:
                 m.release()
@@ -214,6 +215,7 @@ class SVM(BaseEstimator):
             sp = C.c_void_p(dS.dptr) if dS is not None else None
             N.call('svmb200_gram', ctx.handle, C.c_void_p(dX.dptr), n, dX.ld, C.c_void_p(dX.dptr), n, dX.ld, d, 1, kid,
                    gamma, coef0, degree, sp, sp, float(bias), H.row0, H.nrows, C.c_void_p(H.matrix.dptr), H.ld)
+            H.matrix.self_gram = True
             ctx.sync()
             if dS is not None:
                 dS.release()

@@ -34,6 +34,8 @@ def create_solvers(symbol, H, tail):
             else:
                 N.call(symbol, *head, *tail(h))
             handles.append(h)
+            if getattr(part.matrix, 'self_gram', False):
+                N.call('svmb200_pg_set_self_gram', h, 1)
         if len(handles) == 1:
             return handles[0]
         arr = (C.c_void_p * len(handles))(*[h.value for h in handles])
@@ -79,6 +81,8 @@ class DeviceLoopMixin:
         sym = C.c_int(0)
         N.call('svmb200_pg_is_symmetric', h, C.byref(sym))
         self.symmetric_pass = bool(sym.value)   # products from the upper triangle only (runtime.use_symmetric_pass)
+        N.call('svmb200_pg_is_exact_symv', h, C.byref(sym))
+        self.exact_symv_pass = bool(sym.value)   # the full pass's bits from the upper triangle (a self-Gram on one GPU)
         return h, n
 
     @staticmethod

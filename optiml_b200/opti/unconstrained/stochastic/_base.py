@@ -105,6 +105,8 @@ class StochasticOptimizer(DeviceLoopMixin, Optimizer):
         sym = C.c_int(0)
         N.call('svmb200_pg_is_symmetric', h, C.byref(sym))
         self.symmetric_pass = bool(sym.value)
+        N.call('svmb200_pg_is_exact_symv', h, C.byref(sym))
+        self.exact_symv_pass = bool(sym.value)   # the full pass's bits from the upper triangle (a self-Gram on one GPU)
         return h, n
 
     def _pull_state(self, h, n):

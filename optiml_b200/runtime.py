@@ -221,6 +221,9 @@ class DeviceMatrix:
         self.ctx, self.rows, self.cols, self.ld = ctx, int(rows), int(cols), int(ld)
         self.nbytes = max(self.rows, 1) * self.ld * 8
         self.dptr = ctx.malloc(self.nbytes)
+        # rows of a self-Gram svmb200_gram built (same = 1): exactly symmetric, so a solver on one GPU may take its
+        # products from the upper triangle with the full pass's bits (svmb200_pg_set_self_gram)
+        self.self_gram = False
         self._finalizer = weakref.finalize(self, _free_quiet, ctx, self.dptr, self.nbytes)
 
     def release(self):
