@@ -194,10 +194,30 @@ int svmb200_fw_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
  * svmb200_pg_run (chunks of at most 65 536 iterations per launch, history storage grown with the iterations run),
  * _state (x = a, g = G = Qa + q, f = objective tracked per step, ng = gap), _history (f and gap per state), _scalars
  * ({f, gap, 0, 0, 0, 0}), _stats (passes = 0: an iteration reads two rows of Q) and _destroy apply; lockstep batches
- * and single-process groups do not.                                                                                 */
+ * of svmb200_pg_run_batch and single-process groups do not (svmb200_smo_run_batch below is SMO's batch).           */
 int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                        int hessian, const double* sign_host, const double* q_host, const double* ub_host, double tol,
                        int64_t max_iter, svmb200_pg** out);
+/* The same solver on a signed view of a shared, unsigned M (svmb200_gram with bias 0 and no signs): dQ holds M (n x n)
+ * and Q_st = (sign_s == sign_t ? M_st : -M_st) with s, t taken mod n, the signs being sign_host (SVC: the labels; SVR:
+ * e, which is the SVR read of svmb200_smo_create).  The diagonal is read unsigned.  svmb200_gram signs a matrix by
+ * flipping the sign bit of fl(K + bias), the same operation, so the solve is BIT-IDENTICAL to svmb200_smo_create on
+ * the signed Q svmb200_gram builds with these signs.  Arguments and answers as for svmb200_smo_create.             */
+int svmb200_smo_create_signed(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
+                              int hessian, const double* sign_host, const double* q_host, const double* ub_host,
+                              double tol, int64_t max_iter, svmb200_pg** out);
+/* K14: `count` fresh resident or signed-view SMO solvers (svmb200_smo_create / _create_signed, not run yet, none twice)
+ * on the same context, matrix, n, ld and layout, run to termination side by side: each problem gets its own range of
+ * CTAs of one cooperative launch (at most one CTA per SM), keeps its own tol, max_iter, state and history, and ends
+ * BIT-IDENTICAL to its own svmb200_pg_run.  Before every launch unfinished problems are admitted in index order while
+ * their minimum grids (slices of at most 4 714 variables) fit the SMs, and the SMs are split evenly among them (no
+ * problem above its own single-fit grid); a launch runs at most 4 096 iterations per problem; problems that finished give
+ * their SMs to the others at the next launch.  Afterwards every solver answers svmb200_pg_state / _history / _scalars
+ * / _stats (ms = the whole batch) as after svmb200_pg_run.  SVMB200_ERR_ARG for solvers of another kind, computed
+ * rows, mixed matrices or layouts, a solver listed twice or one that has run.  SVMB200_SMO_BATCH_SMS caps the SMs the
+ * batch uses, SVMB200_SMO_BATCH_CHUNK sets the iterations per launch (sweeps, tests).  iters / statuses: `count`
+ * entries each (may be NULL).                                                                                      */
+int svmb200_smo_run_batch(svmb200_pg* const* pgs, int count, int64_t* iters, int* statuses);
 /* K12: the same SMO solver for problems whose Hessian does not fit in HBM.  No matrix is stored: every row of Q the
  * solver needs is computed from X on the device, Q_st = sign_s sign_t k(x_{s mod n}, x_{t mod n}) (PLAIN: nvars = n,
  * SVC with sign = the labels; SVR: nvars = 2n, sign = e), with K1's arithmetic for the kernel value (svmb200_gram with

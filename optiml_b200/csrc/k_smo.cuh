@@ -41,6 +41,18 @@
 // A value is the same whether it was cached or computed, so hits and misses never change a bit of the trajectory.
 // Q_ij (phase 3) travels from j's owner, which holds Q_it for t = j in its part of row i, through a per-CTA slot
 // published beside the j candidate.
+//
+// SMO_ROWS_SIGNED reads a shared, unsigned resident M (bias 0) and applies the sign row on read, as K12 does:
+// Q_st = (sign_s == sign_t ? v : -v), v = M[s mod n][t mod n] (SVC: sign = the labels; SVR: sign = e, the SVR read above);
+// the diagonal is read unsigned.  K1 signs a matrix by flipping the sign bit of fl(K + bias), the same operation, so a
+// solve on the view is bit-identical to one on K1's signed Q, zeros included.  It is how the problems of one-vs-rest and
+// multi-target fits share one M in HBM.
+//
+// K14, smo_batch_kernel: several problems on one shared M in ONE cooperative launch.  Problem b runs on its own contiguous
+// range of CTAs with its own SmoArgs (state, candidate slots, histories) and its own grid barrier; the body below takes the
+// CTA's index and grid size inside its problem instead of blockIdx.x / gridDim.x.  A solve does not depend on its grid
+// (total-order reductions), so every problem follows the same bits whatever grid it is given, launch after launch.  The
+// computed form stays single-problem: its per-CTA cache tags assume one problem owns the CTA's slice.
 #pragma once
 #include "k_persistent.cuh"   // pk_grid_barrier
 #include "kernel_fn.cuh"      // kfn_value
@@ -48,7 +60,7 @@
 constexpr int SMO_NT = 256;
 constexpr int SMO_ARRAYS = 6;        // doubles of shared memory per owned variable: alpha, G, sign, Q_tt, C, Q_it
 constexpr double SMO_TAU = 1e-12;
-constexpr int SMO_ROWS_RESIDENT = 0, SMO_ROWS_COMPUTED = 1;
+constexpr int SMO_ROWS_RESIDENT = 0, SMO_ROWS_COMPUTED = 1, SMO_ROWS_SIGNED = 2;
 constexpr int SMO_CACHE_WAYS = 8;
 
 struct SmoCand {      // the winner of one CTA's slice (64 bytes)
@@ -92,14 +104,25 @@ __device__ __forceinline__ double smo_q(const SmoArgs& a, long long s, long long
     return s_lo == t_lo ? v : -v;
 }
 
+// SMO_ROWS_SIGNED: the unsigned M[s mod n][t mod n]
+__device__ __forceinline__ double smo_m(const SmoArgs& a, long long s, long long t) {
+    return __ldg(a.Q + (s < a.n ? s : s - a.n) * a.ld + (t < a.n ? t : t - a.n));
+}
+
+// SMO_ROWS_SIGNED: Q[s][t] from M and the signs of s and t
+__device__ __forceinline__ double smo_q_signed(const SmoArgs& a, long long s, long long t, double ys, double yt) {
+    const double v = smo_m(a, s, t);
+    return ys == yt ? v : -v;
+}
+
 // thread 0 of a CTA: the slot of sample r in this CTA's copy of the cache tags (LRU victim on a miss), -1 without cache
-__device__ __forceinline__ long long smo_cache_lookup(const SmoArgs& a, long long r, long long stamp, int& hit) {
+__device__ __forceinline__ long long smo_cache_lookup(const SmoArgs& a, unsigned cta, long long r, long long stamp, int& hit) {
     hit = 0;
     long long slot = -1;
     if (a.sets > 0) {
         const long long slots = a.sets * a.ways, base = (r % a.sets) * a.ways;
-        int* tags = a.tags + (size_t)blockIdx.x * slots;
-        long long* st = a.stamps + (size_t)blockIdx.x * slots;
+        int* tags = a.tags + (size_t)cta * slots;
+        long long* st = a.stamps + (size_t)cta * slots;
         // all ways are loaded before any is compared: independent loads, one round trip to L2 instead of `ways`
         int tg[SMO_CACHE_WAYS];
         long long sp[SMO_CACHE_WAYS];
@@ -123,7 +146,7 @@ __device__ __forceinline__ long long smo_cache_lookup(const SmoArgs& a, long lon
         tags[slot] = (int)r;
         st[slot] = stamp;
     }
-    if (blockIdx.x == 0) a.stats[hit ? 0 : 1] += 1;
+    if (cta == 0) a.stats[hit ? 0 : 1] += 1;
     return slot;
 }
 
@@ -200,8 +223,9 @@ __device__ __forceinline__ void smo_grid_reduce(const SmoCand* slots, unsigned g
     __syncthreads();
 }
 
+// the solve of one problem by CTA `cta` of the `grid` CTAs that run it
 template <int ROWS>
-__global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs a) {
+__device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, const unsigned grid) {
 #ifndef SVMB200_HOST_EMULATION
     extern __shared__ __align__(16) unsigned char smo_smem_raw[];
     double* sm = reinterpret_cast<double*>(smo_smem_raw);
@@ -213,10 +237,9 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
     __shared__ long long s_slot[2];   // computed rows: cache slot of row j (phase 1) and of row i (phase 2)
     __shared__ int s_hit[2];
     const int tid = threadIdx.x;
-    const unsigned grid = gridDim.x;
     const int S = a.slice;
     double *s_alpha = sm, *s_g = sm + S, *s_y = sm + 2 * S, *s_qd = sm + 3 * S, *s_c = sm + 4 * S, *s_qi = sm + 5 * S;
-    const long long t0 = (long long)blockIdx.x * S;
+    const long long t0 = (long long)cta * S;
     const int len = t0 >= a.nvars ? 0 : (int)(a.nvars - t0 < S ? a.nvars - t0 : S);
 
     for (int l = tid; l < len; l += SMO_NT) {
@@ -228,6 +251,8 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         if constexpr (ROWS == SMO_ROWS_COMPUTED) {
             const long long tm = t < a.n ? t : t - a.n;
             s_qd[l] = kfn_value(a.kf, tm, tm);
+        } else if constexpr (ROWS == SMO_ROWS_SIGNED) {
+            s_qd[l] = smo_m(a, t, t);
         } else {
             s_qd[l] = smo_q(a, t, t);
         }
@@ -253,6 +278,8 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
                 if constexpr (ROWS == SMO_ROWS_COMPUTED) {
                     const double v = smo_row_value(a, pj < a.n ? pj : pj - a.n, t, s_slot[0], s_hit[0]);
                     qjt = win_j.y == s_y[l] ? v : -v;
+                } else if constexpr (ROWS == SMO_ROWS_SIGNED) {
+                    qjt = smo_q_signed(a, pj, t, win_j.y, s_y[l]);
                 } else {
                     qjt = smo_q(a, pj, t);
                 }
@@ -278,7 +305,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
                 c.qd = s_qd[l];
                 c.c = s_c[l];
             }
-            slots_i[blockIdx.x] = c;
+            slots_i[cta] = c;
         }
         pk_grid_barrier(a.gbar, grid);
 
@@ -287,7 +314,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         const double m = win_i.key, yi = win_i.y, qii = win_i.qd;
         const long long i = (long long)win_i.idx;
         if constexpr (ROWS == SMO_ROWS_COMPUTED) {
-            if (tid == 0 && i >= 0) s_slot[1] = smo_cache_lookup(a, i < a.n ? i : i - a.n, 2 * k + 1, s_hit[1]);
+            if (tid == 0 && i >= 0) s_slot[1] = smo_cache_lookup(a, cta, i < a.n ? i : i - a.n, 2 * k + 1, s_hit[1]);
             __syncthreads();
         }
         key = -INFINITY;
@@ -301,6 +328,8 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
                     const double v = smo_row_value(a, i < a.n ? i : i - a.n, t, s_slot[1], s_hit[1]);
                     qit = yi == s_y[l] ? v : -v;
                 }
+            } else if constexpr (ROWS == SMO_ROWS_SIGNED) {
+                qit = i >= 0 ? smo_q_signed(a, i, t, yi, s_y[l]) : 0.0;
             } else {
                 qit = i >= 0 ? smo_q(a, i, t) : 0.0;
             }
@@ -332,9 +361,9 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
                 c.y = s_y[l];
                 c.qd = s_qd[l];
                 c.c = s_c[l];
-                if constexpr (ROWS == SMO_ROWS_COMPUTED) a.qij[(size_t)(k & 1) * grid + blockIdx.x] = s_qi[l];
+                if constexpr (ROWS == SMO_ROWS_COMPUTED) a.qij[(size_t)(k & 1) * grid + cta] = s_qi[l];
             }
-            slots_j[blockIdx.x] = c;
+            slots_j[cta] = c;
         }
         pk_grid_barrier(a.gbar, grid);
 
@@ -342,7 +371,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         smo_grid_reduce(slots_j, grid, S, red, &win_j);
         const long long j = (long long)win_j.idx;
         const double gap = __dsub_rn(m, win_j.mlow);
-        if (blockIdx.x == 0 && tid == 0) {
+        if (cta == 0 && tid == 0) {
             if (k < a.hist_cap) {
                 a.hist_f[k] = f;
                 a.hist_gap[k] = gap;
@@ -355,7 +384,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         if (j < 0 || gap < a.tol) stop = SVMB200_STATUS_OPTIMAL;
         else if (k >= a.max_iter) stop = SVMB200_STATUS_STOPPED;
         if (stop) {
-            if (blockIdx.x == 0 && tid == 0) {
+            if (cta == 0 && tid == 0) {
                 a.st->status = stop;
                 __threadfence();
                 a.st->done = 1;
@@ -369,6 +398,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         const double qjj = win_j.qd, gi = win_i.g, gj = win_j.g, ci = win_i.c, cj = win_j.c;
         double qij;
         if constexpr (ROWS == SMO_ROWS_COMPUTED) qij = __ldcg(a.qij + (size_t)(k & 1) * grid + j / S);
+        else if constexpr (ROWS == SMO_ROWS_SIGNED) qij = smo_q_signed(a, i, j, yi, win_j.y);
         else qij = smo_q(a, i, j);
         const double ai0 = win_i.alpha, aj0 = win_j.alpha;
         double ai = ai0, aj = aj0;
@@ -420,7 +450,7 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         pending = true;
         pj = j;
         if constexpr (ROWS == SMO_ROWS_COMPUTED) {
-            if (tid == 0) s_slot[0] = smo_cache_lookup(a, j < a.n ? j : j - a.n, 2 * (k + 1), s_hit[0]);
+            if (tid == 0) s_slot[0] = smo_cache_lookup(a, cta, j < a.n ? j : j - a.n, 2 * (k + 1), s_hit[0]);
         }
         __syncthreads();   // alpha of i / j in place for the next phase 1
     }
@@ -428,4 +458,35 @@ __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs
         a.x[t0 + l] = s_alpha[l];
         a.g[t0 + l] = s_g[l];
     }
+}
+
+template <int ROWS>
+__global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs a) {
+    smo_solve<ROWS>(a, blockIdx.x, gridDim.x);
+}
+
+// K14: one problem of a batch -- its arguments and its CTAs [cta0, cta0 + grid) of the launch
+struct SmoBatchProblem {
+    SmoArgs a;
+    int cta0, grid;
+};
+
+struct SmoBatchArgs {
+    const SmoBatchProblem* probs;   // in ascending cta0, the CTA ranges back to back from 0
+    int count;
+};
+
+template <int ROWS>
+__global__ void __launch_bounds__(SMO_NT, 1) smo_batch_kernel(const SmoBatchArgs b) {
+    __shared__ SmoArgs pa;   // the problem's arguments, read once per launch
+    __shared__ unsigned p_cta, p_grid;
+    if (threadIdx.x == 0) {
+        int p = 0;
+        while (p + 1 < b.count && (int)blockIdx.x >= b.probs[p + 1].cta0) ++p;
+        pa = b.probs[p].a;
+        p_cta = blockIdx.x - (unsigned)b.probs[p].cta0;
+        p_grid = (unsigned)b.probs[p].grid;
+    }
+    __syncthreads();
+    smo_solve<ROWS>(pa, p_cta, p_grid);
 }

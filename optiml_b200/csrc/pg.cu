@@ -19,6 +19,7 @@
 #include "k3_vector.cuh"   // K3 vector phases and kernel entry points (device code)
 #include "k_persistent.cuh"  // the whole loop in one cooperative kernel, matrix in shared memory (small problems)
 #include "k_smo.cuh"         // K11: SMO with the equality constraint, one cooperative kernel for many iterations
+#include <algorithm>
 #include <math.h>
 #include <stdlib.h>
 #include <memory>
@@ -617,7 +618,7 @@ enum SolverKind : int {
 struct SmoSolver {
     SmoArgs a = {};
     int grid = 0;
-    int rows = SMO_ROWS_RESIDENT;
+    int rows = SMO_ROWS_RESIDENT;   // SMO_ROWS_RESIDENT, _SIGNED (svmb200_smo_create_signed) or _COMPUTED
     void* rows_buf = nullptr;  // |x|^2 | Q_ij slots | tags | stamps | stats | cache
 };
 
@@ -1831,9 +1832,23 @@ struct SmoRowsSpec {
 
 extern "C" int64_t svmb200_smo_max_vars(int sm_count) { return SMO_SLICE_MAX * (int64_t)sm_count; }
 
+// the kernel of a row source, and its launch set-up
+static void (*smo_kernel(int rows))(SmoArgs) {
+    return rows == SMO_ROWS_COMPUTED ? smo_persistent_kernel<SMO_ROWS_COMPUTED>
+         : rows == SMO_ROWS_SIGNED   ? smo_persistent_kernel<SMO_ROWS_SIGNED>
+                                     : smo_persistent_kernel<SMO_ROWS_RESIDENT>;
+}
+
+static int smo_setup(svmb200_ctx* ctx, int rows, int grid, size_t smem, bool* fits) {
+    return rows == SMO_ROWS_COMPUTED ? cooperative_setup<smo_persistent_kernel<SMO_ROWS_COMPUTED>>(ctx, grid, SMO_NT, smem, fits)
+         : rows == SMO_ROWS_SIGNED   ? cooperative_setup<smo_persistent_kernel<SMO_ROWS_SIGNED>>(ctx, grid, SMO_NT, smem, fits)
+                                     : cooperative_setup<smo_persistent_kernel<SMO_ROWS_RESIDENT>>(ctx, grid, SMO_NT, smem, fits);
+}
+
+// rows: the computed form (K12), else null; signed_view: dQ is an unsigned M read with the signs (SMO_ROWS_SIGNED)
 static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int hessian, const double* sign_host,
                       const double* q_host, const double* ub_host, double tol, int64_t max_iter, const SmoRowsSpec* rows,
-                      svmb200_pg** out) {
+                      bool signed_view, svmb200_pg** out) {
     SVM_CHECK_ARG(max_iter > 0, "max_iter must be > 0");
     SVM_CHECK_ARG(tol >= 0.0, "tol must be >= 0");
     const int64_t nvars = hessian == SVMB200_HESSIAN_SVR ? 2 * n : n;
@@ -1875,10 +1890,9 @@ static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
     SmoArgs& a = smo.a;
     a.slice = (int)slice;
     smo.grid = (int)((nvars + slice - 1) / slice);
-    smo.rows = rows ? SMO_ROWS_COMPUTED : SMO_ROWS_RESIDENT;
+    smo.rows = rows ? SMO_ROWS_COMPUTED : signed_view ? SMO_ROWS_SIGNED : SMO_ROWS_RESIDENT;
     bool fits = false;
-    SVM_TRY((rows ? cooperative_setup<smo_persistent_kernel<SMO_ROWS_COMPUTED>>
-                  : cooperative_setup<smo_persistent_kernel<SMO_ROWS_RESIDENT>>)(ctx, smo.grid, SMO_NT, smo_smem_bytes(pg), &fits));
+    SVM_TRY(smo_setup(ctx, smo.rows, smo.grid, smo_smem_bytes(pg), &fits));
     if (!fits) {
         svmb200_set_error("SMO: %d CTAs of %zu bytes of shared memory cannot be co-resident", smo.grid, smo_smem_bytes(pg));
         return SVMB200_ERR_ARG;
@@ -1962,7 +1976,16 @@ extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n,
     SVM_TRY(check_create_args(__func__, ctx, out, dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr,
                               n, "Q is too small", ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
     SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
-    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, out);
+    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, false, out);
+}
+
+extern "C" int svmb200_smo_create_signed(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0,
+                                         int64_t nrows, int hessian, const double* sign_host, const double* q_host,
+                                         const double* ub_host, double tol, int64_t max_iter, svmb200_pg** out) {
+    SVM_TRY(check_create_args(__func__, ctx, out, dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr,
+                              n, "M is too small", ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
+    SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
+    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, true, out);
 }
 
 extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel,
@@ -1988,7 +2011,7 @@ extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64
     rows.kf.degree = degree;
     rows.kf.int_degree = svm_gram_int_degree(degree);
     rows.cache_bytes = cache_bytes;
-    return smo_create(ctx, nullptr, n, 0, hessian, sign_host, q_host, ub_host, tol, max_iter, &rows, out);
+    return smo_create(ctx, nullptr, n, 0, hessian, sign_host, q_host, ub_host, tol, max_iter, &rows, false, out);
 }
 
 extern "C" int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses) {
@@ -2037,9 +2060,8 @@ static int smo_launch(svmb200_pg* pg, int64_t niter) {
     a.hist_cap = pg->hist_cap;
     a.k0 = pg->k_next;
     a.niter = niter;
-    SVM_CUDA(svm_launch_cooperative(pg->smo.rows == SMO_ROWS_COMPUTED ? smo_persistent_kernel<SMO_ROWS_COMPUTED>
-                                                                        : smo_persistent_kernel<SMO_ROWS_RESIDENT>,
-                                    dim3((unsigned)pg->smo.grid), dim3(SMO_NT), smo_smem_bytes(pg), pg->ctx->stream, a));
+    SVM_CUDA(svm_launch_cooperative(smo_kernel(pg->smo.rows), dim3((unsigned)pg->smo.grid), dim3(SMO_NT), smo_smem_bytes(pg),
+                                    pg->ctx->stream, a));
     pg->ctx->launches++;
     return SVMB200_OK;
 }
@@ -2065,6 +2087,135 @@ static int smo_run(svmb200_pg* pg, int64_t max_new) {
     SVM_CUDA(cudaEventRecord(pg->ev1, ctx->stream));
     SVM_CUDA(cudaEventSynchronize(pg->ev1));
     SVM_CUDA(cudaEventElapsedTime(&pg->last_ms, pg->ev0, pg->ev1));
+    return SVMB200_OK;
+}
+
+// ------------------------------------------------------------------------------------------ K14: SMO batch (k_smo.cuh)
+// Several resident or signed-view SMO problems on one matrix share the GPU: an SMO iteration is bound by the latency of
+// two grid barriers, not by bandwidth, and a smaller grid costs a problem little (profiles/smo_grid_sweep.jsonl).  So
+// problems run side by side on disjoint ranges of CTAs, at most one CTA per SM, in one cooperative launch of at most
+// SMO_BATCH_CHUNK iterations per problem.  Before every launch the scheduler admits unfinished problems in index order
+// while their minimum grids (slices of at most SMO_SLICE_MAX variables) fit the SMs, and splits the SMs evenly among
+// them, no problem above its own single-fit grid; after it, one synchronisation reads every admitted problem's state.
+// Problems that finished give their SMs to the others at the next launch and waiting problems are admitted.  A solve
+// does not depend on its grid, so each problem ends bit for bit where its own svmb200_pg_run would.
+// SVMB200_SMO_BATCH_SMS caps the SMs a batch uses and SVMB200_SMO_BATCH_CHUNK sets the chunk (sweeps; tests on the host
+// emulation, which reports 148 SMs).
+constexpr int64_t SMO_BATCH_CHUNK = 4096;
+
+static int env_positive(const char* name, int64_t* value) {
+    if (const char* ev = getenv(name)) {
+        const long long v = atoll(ev);
+        if (v < 1) {
+            svmb200_set_error("%s must be >= 1", name);
+            return SVMB200_ERR_ARG;
+        }
+        *value = v;
+    }
+    return SVMB200_OK;
+}
+
+extern "C" int svmb200_smo_run_batch(svmb200_pg* const* pgs, int count, int64_t* iters, int* statuses) {
+    SVM_CHECK_ARG(pgs != nullptr && count >= 1 && count <= 65535, "bad argument");
+    svmb200_pg* p0 = pgs[0];
+    for (int b = 0; b < count; ++b) {
+        const svmb200_pg* p = pgs[b];
+        SVM_CHECK_ARG(p != nullptr && p0 != nullptr, "null solver");
+        SVM_CHECK_ARG(p->solver == SOLVER_SMO, "svmb200_smo_run_batch takes SMO solvers only");
+        SVM_CHECK_ARG(p->smo.rows != SMO_ROWS_COMPUTED, "an SMO solver with computed rows has no batch: run it alone");
+        SVM_CHECK_ARG(p->ctx == p0->ctx && p->dQ == p0->dQ && p->n == p0->n && p->ld == p0->ld && p->svr == p0->svr &&
+                          p->smo.rows == p0->smo.rows,
+                      "the solvers of a batch must share the resident matrix and its layout");
+        SVM_CHECK_ARG(p->k_next == 0 && !p->finished, "a batch takes solvers that have not run yet");
+        for (int c = 0; c < b; ++c) SVM_CHECK_ARG(pgs[c] != p, "a solver is listed twice");
+    }
+    svmb200_ctx* ctx = p0->ctx;
+    SVM_TRY(svm_use(ctx));
+    int64_t sms = ctx->sm_count > 0 ? ctx->sm_count : 1, chunk = SMO_BATCH_CHUNK;
+    int64_t cap = sms;
+    SVM_TRY(env_positive("SVMB200_SMO_BATCH_SMS", &cap));
+    SVM_TRY(env_positive("SVMB200_SMO_BATCH_CHUNK", &chunk));
+    if (cap < sms) sms = cap;
+    const int64_t nvars = p0->nvars, g_min = (nvars + SMO_SLICE_MAX - 1) / SMO_SLICE_MAX;
+    if (sms < g_min) sms = g_min;   // a cap below one problem's minimum grid still runs one problem at a time
+    const int64_t slots = std::min<int64_t>(count, sms / g_min);
+    // per launch: the problems' arguments, and one grid barrier (256 bytes) per admitted problem
+    const size_t probs_bytes = ((size_t)slots * sizeof(SmoBatchProblem) + 255) & ~size_t(255);
+    SVM_TRY(svm_scratch_reserve(ctx, &ctx->batch_buf, &ctx->batch_bytes, probs_bytes + (size_t)slots * 256));
+    SmoBatchProblem* dprobs = static_cast<SmoBatchProblem*>(ctx->batch_buf);
+    unsigned* bars = reinterpret_cast<unsigned*>(static_cast<unsigned char*>(ctx->batch_buf) + probs_bytes);
+    SVM_CUDA(cudaMemsetAsync(bars, 0, (size_t)slots * 256, ctx->stream));
+    for (int b = 0; b < count; ++b) reset_run_stats(pgs[b]);
+    SVM_CUDA(cudaEventRecord(p0->ev0, ctx->stream));
+    std::vector<SmoBatchProblem> hp((size_t)slots);
+    std::vector<int> admitted((size_t)slots);
+    std::vector<int64_t> nb((size_t)slots);
+    for (int next = 0;;) {
+        while (next < count && pgs[next]->finished) ++next;
+        int k = 0;
+        for (int b = next; b < count && k < slots; ++b)
+            if (!pgs[b]->finished) admitted[k++] = b;
+        if (k == 0) break;
+        int cta0 = 0;
+        size_t smem = 0;
+        for (int r = 0; r < k; ++r) {
+            svmb200_pg* pg = pgs[admitted[r]];
+            int64_t g = sms / k + (r < sms % k ? 1 : 0);
+            if (g > pg->smo.grid) g = pg->smo.grid;
+            const int64_t slice = (nvars + g - 1) / g;
+            const int64_t left = pg->max_iter - pg->k_next;
+            nb[r] = left < chunk ? left : chunk;
+            SVM_TRY(smo_hist_reserve(pg, pg->k_next + nb[r] + 1));
+            SmoBatchProblem& p = hp[r];
+            p.a = pg->smo.a;
+            p.a.slice = (int)slice;
+            p.a.gbar = bars + (size_t)r * 64;
+            p.a.hist_f = pg->hist_f;
+            p.a.hist_gap = pg->hist_ng;
+            p.a.hist_cap = pg->hist_cap;
+            p.a.k0 = pg->k_next;
+            p.a.niter = nb[r];
+            p.cta0 = cta0;
+            p.grid = (int)((nvars + slice - 1) / slice);
+            cta0 += p.grid;
+            smem = std::max(smem, (size_t)slice * SMO_ARRAYS * sizeof(double));
+        }
+        bool fits = false;
+        const bool sgn = p0->smo.rows == SMO_ROWS_SIGNED;
+        SVM_TRY(sgn ? cooperative_setup<smo_batch_kernel<SMO_ROWS_SIGNED>>(ctx, cta0, SMO_NT, smem, &fits)
+                    : cooperative_setup<smo_batch_kernel<SMO_ROWS_RESIDENT>>(ctx, cta0, SMO_NT, smem, &fits));
+        if (!fits) {
+            svmb200_set_error("SMO batch: %d CTAs of %zu bytes of shared memory cannot be co-resident", cta0, smem);
+            return SVMB200_ERR_STATE;
+        }
+        SVM_CUDA(cudaMemcpyAsync(dprobs, hp.data(), (size_t)k * sizeof(SmoBatchProblem), cudaMemcpyHostToDevice, ctx->stream));
+        SmoBatchArgs ba;
+        ba.probs = dprobs;
+        ba.count = k;
+        SVM_CUDA(svm_launch_cooperative(sgn ? smo_batch_kernel<SMO_ROWS_SIGNED> : smo_batch_kernel<SMO_ROWS_RESIDENT>,
+                                        dim3((unsigned)cta0), dim3(SMO_NT), smem, ctx->stream, ba));
+        ctx->launches++;
+        for (int r = 0; r < k; ++r) {
+            svmb200_pg* pg = pgs[admitted[r]];
+            SVM_CUDA(cudaMemcpyAsync(pg->st_host, pg->st, sizeof(PGDeviceState), cudaMemcpyDeviceToHost, ctx->stream));
+        }
+        SVM_CUDA(cudaStreamSynchronize(ctx->stream));
+        for (int r = 0; r < k; ++r) {
+            svmb200_pg* pg = pgs[admitted[r]];
+            if (pg->st_host->done) pg->finished = true;
+            pg->k_next = pg->finished ? pg->st_host->iter : pg->k_next + nb[r];
+        }
+    }
+    SVM_CUDA(cudaEventRecord(p0->ev1, ctx->stream));
+    SVM_CUDA(cudaEventSynchronize(p0->ev1));
+    float ms = 0.f;
+    SVM_CUDA(cudaEventElapsedTime(&ms, p0->ev0, p0->ev1));
+    for (int b = 0; b < count; ++b) {
+        svmb200_pg* pg = pgs[b];
+        pg->last_ms = ms;  // device time of the whole batch
+        if (iters) iters[b] = pg->st_host->iter;
+        if (statuses) statuses[b] = pg->st_host->status;
+    }
     return SVMB200_OK;
 }
 

@@ -11,6 +11,11 @@ bit-identical to what ``clone(estimator).fit(X, y_c)`` produces on the same GPU.
 
 ``MultiOutputRegressor`` is the same idea for ``SVR``: the targets only change the linear term q.
 
+``optimizer='smo'`` estimators share M too (bias 0, the signs applied on read), but their solvers run side by side on
+disjoint ranges of the GPU's SMs (``svmb200_smo_run_batch``) instead of in lockstep: an SMO iteration is bound by
+latency, not by bandwidth.  When M would not be resident (``smo.select_row_source`` picks computed rows) the clones are
+fitted one after the other, each choosing its own row source.
+
 Anything the lockstep driver cannot take (a generic callback, ``verbose``, an estimator of another type, fit
 parameters, a degenerate class column) goes through sklearn's own ``fit`` -- still on the GPU, one clone after
 the other.
@@ -33,7 +38,8 @@ __all__ = ['OneVsRestClassifier', 'MultiOutputRegressor', 'fit_shared_gram']
 
 def fit_shared_gram(estimator, X, targets):
     """Fit one clone of ``estimator`` (an ``SVC`` or ``SVR`` of this package on the dual path) per entry of ``targets``
-    (label / target vectors over the same rows of X) on ONE resident Gram matrix.  Returns the fitted clones."""
+    (label / target vectors over the same rows of X) on ONE resident Gram matrix.  Returns the fitted clones, which
+    report ``fit_times_['batch']``, the number of problems that shared the matrix."""
     if not isinstance(estimator, (SVC, SVR)):
         raise TypeError(f'{estimator} is not an SVC / SVR of optiml_b200')
     targets = [np.asarray(t) for t in targets]
@@ -42,10 +48,14 @@ def fit_shared_gram(estimator, X, targets):
     clones = [clone(estimator) for _ in targets]
     X, _ = _dense_f64(X, None, finite=False)  # the all-finite test runs on the device copy (_build_hessian)
     head = clones[0]
+    layout = 'svr' if isinstance(estimator, SVR) else 'plain'
     if head._bcqp_solver_class() is SMO:  # (raises for the branches outside the dual path before any device work)
-        raise NotImplementedError("optimizer='smo' has no lockstep batch: fit the clones one after the other")
+        n, d = X.shape
+        head._check_solver_scope(SMO, n)
+        if head._smo_row_source(n, d, layout)[0] != 'resident':
+            return [est.fit(X, t) for est, t in zip(clones, targets)]
     # K1 once: M = K + bias without label signs (SVC: the solvers apply them; SVR: the block signs are implicit)
-    shared = head._build_hessian(X, None, 'svr' if isinstance(estimator, SVR) else 'plain', None, head._bias())
+    shared = head._build_hessian(X, None, layout, None, head._bias())
     gram_s = head.fit_times_['gram_s']
     dX, owned = head._train_X_device   # every clone gathers its support vectors from this one copy of X in HBM
     try:
@@ -66,6 +76,17 @@ def fit_shared_gram(estimator, X, targets):
     return clones
 
 
+def _smo_batch_capable(estimator):
+    """An ``optimizer='smo'`` estimator whose clones ``fit_shared_gram`` can run as one SMO batch: nothing on the host
+    watches the solve.  (Sharded fits raise in ``fit_shared_gram``, as they do in a single fit.)"""
+    if not isinstance(estimator, (SVC, SVR)) or estimator.verbose:
+        return False
+    try:
+        return estimator._bcqp_solver_class() is SMO
+    except (NotImplementedError, TypeError):
+        return False
+
+
 def _lockstep_capable(estimator, n_samples=None):
     """The estimator runs a device-resident solver that nothing on the host has to watch (and the problem is not one a
     single-process device group shards over its GPUs: there the clones are fitted one after the other, each on all GPUs)."""
@@ -80,14 +101,15 @@ def _lockstep_capable(estimator, n_samples=None):
         solver_cls = estimator._bcqp_solver_class()
     except (NotImplementedError, TypeError):
         return False
-    return solver_cls is not SMO   # no lockstep SMO batch: sklearn's own fit, one clone after the other
+    return solver_cls is not SMO   # SMO batches are not lockstep ones: _smo_batch_capable
 
 
 class OneVsRestClassifier(_skmc.OneVsRestClassifier):
     """``sklearn.multiclass.OneVsRestClassifier`` whose binary ``SVC`` problems share one Gram matrix."""
 
     def fit(self, X, y, **fit_params):
-        if fit_params or not isinstance(self.estimator, SVC) or not _lockstep_capable(self.estimator, np.shape(X)[0]):
+        if fit_params or not isinstance(self.estimator, SVC) or \
+                not (_lockstep_capable(self.estimator, np.shape(X)[0]) or _smo_batch_capable(self.estimator)):
             return super().fit(X, y, **fit_params)
         self._validate_params()
         # label handling of sklearn/multiclass.py OneVsRestClassifier.fit
@@ -112,7 +134,8 @@ class MultiOutputRegressor(_skmo.MultiOutputRegressor):
     def fit(self, X, y, sample_weight=None, **fit_params):
         y_arr = np.asarray(y)
         if sample_weight is not None or fit_params or not isinstance(self.estimator, SVR) or \
-                not _lockstep_capable(self.estimator, np.shape(X)[0]) or y_arr.ndim != 2 or y_arr.shape[1] < 2:
+                not (_lockstep_capable(self.estimator, np.shape(X)[0]) or _smo_batch_capable(self.estimator)) or \
+                y_arr.ndim != 2 or y_arr.shape[1] < 2:
             return super().fit(X, y, sample_weight=sample_weight, **fit_params)
         self._validate_params()
         self.estimators_ = fit_shared_gram(self.estimator, X, [y_arr[:, i] for i in range(y_arr.shape[1])])

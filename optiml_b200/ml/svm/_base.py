@@ -224,6 +224,14 @@ class SVM(BaseEstimator):
         self.fit_times_ = {'gram_s': time.perf_counter() - t0}  # gamma + upload + Gram kernel (wall clock)
         return H
 
+    @staticmethod
+    def _smo_row_source(n, d, layout):
+        """``smo.select_row_source`` for an SMO fit of n samples with d features started now."""
+        ctx = default_context()
+        info = ctx.info()
+        info['free_bytes'] += ctx.pooled_bytes()   # parked buffers are given back when an allocation needs them
+        return select_row_source(n, 2 * n if layout == 'svr' else n, N.padded_ld(n), d, info)
+
     def _smo_hessian(self, X, signs, layout, X_device=None):
         """SMO's Hessian: resident (K1, as for the other solvers) when it fits in the free device memory, else computed
         rows (K12: no matrix, rows from X on the device, with a row cache) -- chosen by smo.select_row_source before
@@ -231,10 +239,7 @@ class SVM(BaseEstimator):
         import time
         ctx = default_context()
         n, d = X.shape
-        nvars = 2 * n if layout == 'svr' else n
-        info = ctx.info()
-        info['free_bytes'] += ctx.pooled_bytes()   # parked buffers are given back when an allocation needs them
-        source, cache_bytes = select_row_source(n, nvars, N.padded_ld(n), d, info)
+        source, cache_bytes = self._smo_row_source(n, d, layout)
         if source == 'resident':
             return self._build_hessian(X, signs, layout, X_device, 0.0)
         ctx.trim()   # the row cache is allocated by the solver, outside the pool

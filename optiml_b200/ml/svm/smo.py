@@ -112,12 +112,16 @@ class SMO(DeviceLoopMixin, Optimizer):
             return h, H.nvars
         if len(H.shards()) != 1 or H.nrows != H.n:
             raise NotImplementedError('SMO runs on one GPU: the Hessian must not be sharded')
-        if H.signs is not None:
-            raise NotImplementedError('SMO reads the signed matrix itself: signed views of a shared matrix are not supported')
         n = H.nvars
         layout = N.HESSIAN_SVR if H.layout == 'svr' else N.HESSIAN_PLAIN
+        symbol = 'svmb200_smo_create'
+        if H.signs is not None:
+            # Q = (s s') o M on a shared, unsigned M (one-vs-rest, ml/multiclass.py): the kernel signs what it reads
+            if not np.array_equal(y, H.signs):
+                raise ValueError('on a signed view the sign row y must be the signs of the view')
+            symbol = 'svmb200_smo_create_signed'
         h = C.c_void_p()
-        N.call('svmb200_smo_create', H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows, layout,
+        N.call(symbol, H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows, layout,
                N.ptr(y), N.ptr(q), N.ptr(ub), float(self.tol), int(self.max_iter), C.byref(h))
         self.row_source = 'resident'
         return h, n

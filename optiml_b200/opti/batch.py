@@ -7,16 +7,22 @@ label signs only, so here they share one unsigned ``M = K + bias`` in HBM (``Dev
 ``svmb200_pg_run_batch`` streams it once per iteration for up to four problems at a time.  Every solver ends with
 exactly the state its own ``minimize()`` would have produced (the multi-vector pass reproduces the single-vector
 reductions bit for bit), so this is a scheduling decision, not a different algorithm.
+
+SMO solvers (ml/svm/smo.py) batch differently: an SMO iteration reads two rows and is bound by the latency of its grid
+barriers, so ``svmb200_smo_run_batch`` runs the problems side by side on disjoint ranges of the GPU's SMs, each with its
+own tol and max_iter, and each again ends bit for bit where its own ``minimize()`` would.
 """
 import ctypes as C
 
 from .. import _native as N
+from ..runtime import KernelRowsHessian
 from .constrained._device_loop import DeviceLoopMixin
 
 
 def batchable(solvers):
-    """True when ``minimize_batch`` can run the solvers in lockstep: device-resident solvers of one class on the same
-    resident matrix, same iteration limit, nothing to run on the host between iterations."""
+    """True when ``minimize_batch`` can run the solvers together: device-resident solvers of one class on the same
+    resident matrix, same iteration limit (SMO: each keeps its own), nothing to run on the host between iterations."""
+    from ..ml.svm.smo import SMO
     solvers = list(solvers)
     if len(solvers) < 2:
         return False
@@ -25,9 +31,11 @@ def batchable(solvers):
         return False
     if not all(s._resident_ok() and not getattr(s, 'profile', False) for s in solvers):
         return False
-    if len({int(s.max_iter) for s in solvers}) != 1:
+    if not isinstance(first, SMO) and len({int(s.max_iter) for s in solvers}) != 1:
         return False
     H0 = first.f.device_hessian()
+    if isinstance(H0, KernelRowsHessian):
+        return False   # SMO with computed rows has no batch
     if len(H0.shards()) != 1:
         return False   # a single-process device group advances one problem at a time (no lockstep batches there)
     for s in solvers:
@@ -41,6 +49,7 @@ def minimize_batch(solvers):
     """``[s.minimize() for s in solvers]`` with the streaming passes shared.  Falls back to exactly that loop (still on
     the device, one solver after the other) when the solvers cannot advance in lockstep -- generic callbacks,
     ``verbose``, different matrices or solver classes."""
+    from ..ml.svm.smo import SMO
     solvers = list(solvers)
     if not batchable(solvers):
         for s in solvers:
@@ -69,7 +78,8 @@ def minimize_batch(solvers):
         count = len(created)
         handles = (C.c_void_p * count)(*[h.value for h, _ in created])
         iters, statuses = (C.c_int64 * count)(), (C.c_int * count)()
-        N.call('svmb200_pg_run_batch', handles, count, iters, statuses)
+        N.call('svmb200_smo_run_batch' if isinstance(solvers[0], SMO) else 'svmb200_pg_run_batch', handles, count, iters,
+               statuses)
         for s, (h, n), it, st in zip(solvers, created, iters, statuses):
             s._finish_resident(h, n, int(it), N.STATUS[int(st)])
             s._after_run(h, n)       # device_ms / q_passes are those of the whole batch
