@@ -115,6 +115,19 @@ static inline int svm_use(svmb200_ctx* ctx) {
 
 static inline int64_t round_up64(int64_t a, int64_t b) { return (a + b - 1) / b * b; }
 
+// Opt `kernel` in to `bytes` of dynamic shared memory, above the default 48 KB.  The attribute belongs to the device (a
+// single-process device group launches one kernel on every GPU of the box from one process): set once per device index
+// below 64, and on every call for any other index.
+template <auto kernel>
+static inline int svm_opt_in_smem(const svmb200_ctx* ctx, int bytes) {
+    static bool done[64] = {};
+    const bool tracked = ctx->device >= 0 && ctx->device < 64;
+    if (tracked && done[ctx->device]) return SVMB200_OK;
+    SVM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    if (tracked) done[ctx->device] = true;
+    return SVMB200_OK;
+}
+
 // ---- programmatic dependent launch (PDL): the kernels of the solver loop form a strict chain (K2 -> K3 -> K2 ...), each
 // a few hundred microseconds or less at 8 GPUs, so the 2-3 us between the end of one grid and the first instruction of the
 // next are paid twice per iteration.  A kernel launched with the programmatic-serialisation attribute may be SCHEDULED

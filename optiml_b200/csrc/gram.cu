@@ -591,14 +591,7 @@ int make_tensor_map(svmb200_ctx* ctx, CUtensorMap* map, const double* base, int6
 
 template <int KERNEL>
 int launch_gram(svmb200_ctx* ctx, const CUtensorMap& ma, const CUtensorMap& mb, const GramArgs& args) {
-    // the opt-in to > 48 KB of dynamic shared memory is a PER-DEVICE function attribute (a single-process device group
-    // launches this kernel on every GPU of the box from one process)
-    static bool configured[64] = {};
-    const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
-    if (!configured[dev]) {
-        SVM_CUDA(cudaFuncSetAttribute(gram_kernel<KERNEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, GRAM_SMEM));
-        configured[dev] = true;
-    }
+    SVM_TRY(svm_opt_in_smem<gram_kernel<KERNEL>>(ctx, GRAM_SMEM));
     const int ntiles = args.tiles_m * args.tiles_n;
     const int grid = ntiles < ctx->sm_count ? ntiles : ctx->sm_count;
     gram_kernel<KERNEL><<<grid, GRAM_THREADS, GRAM_SMEM, ctx->stream>>>(ma, mb, args);

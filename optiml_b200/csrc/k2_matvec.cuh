@@ -83,19 +83,6 @@ __device__ __forceinline__ double2 ld_stream_f64x2(const double2* p) {
     asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p));
     return r;
 }
-// the same load with an evict-first L2 policy: the matrix is touched once per pass, while the vectors of the iteration
-// (u, x, g, d, q, bounds: ~3 MB) and the segment partials are re-read every few hundred microseconds and should survive
-// the 2.5 - 20 GB that stream through the 126 MB L2 in between (A/B: SVMB200_MATVEC_L2_HINT)
-__device__ __forceinline__ unsigned long long l2_evict_first_policy_mv() {
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-__device__ __forceinline__ double2 ld_stream_hint_f64x2(const double2* p, unsigned long long pol) {
-    double2 r;
-    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(r.x), "=d"(r.y) : "l"(p), "l"(pol));
-    return r;
-}
 #else
 // tests/cuda_emu compiles this file for the host (the kernels run thread by thread on fibers, ranks are host threads):
 // same entry format, same wait-until-both-tags-match protocol, without the PTX
@@ -119,11 +106,8 @@ __device__ __forceinline__ double ll_load(const ulonglong2* p, unsigned tag, int
     return __longlong_as_double((long long)((w1 << 32) | (w0 & 0xffffffffull)));
 }
 __device__ __forceinline__ double2 ld_stream_f64x2(const double2* p) { return *p; }
-__device__ __forceinline__ unsigned long long l2_evict_first_policy_mv() { return 0; }
-__device__ __forceinline__ double2 ld_stream_hint_f64x2(const double2* p, unsigned long long) { return *p; }
 #endif
 
-template <bool L2HINT>
 __global__ void __launch_bounds__(MV_NT, MV_MINB) matvec_seg_kernel(const MatvecArgs a) {
     pdl_wait();               // u (and the done flag) come from the vector launch before this one
     pdl_launch_dependents();  // once every CTA of this grid has started, the vector launch may be scheduled behind it
@@ -171,7 +155,6 @@ __global__ void __launch_bounds__(MV_NT, MV_MINB) matvec_seg_kernel(const Matvec
         double acc[R];
 #pragma unroll
         for (int r = 0; r < R; ++r) acc[r] = 0.0;
-        const unsigned long long pol = L2HINT ? l2_evict_first_policy_mv() : 0ull;
 
         int c = threadIdx.x;
         for (; c + (U - 1) * NT < nvec; c += U * NT) {
@@ -180,8 +163,7 @@ __global__ void __launch_bounds__(MV_NT, MV_MINB) matvec_seg_kernel(const Matvec
 #pragma unroll
             for (int j = 0; j < U; ++j) {
 #pragma unroll
-                for (int r = 0; r < R; ++r)
-                    qv[j][r] = L2HINT ? ld_stream_hint_f64x2(rows[r] + c + j * NT, pol) : ld_stream_f64x2(rows[r] + c + j * NT);
+                for (int r = 0; r < R; ++r) qv[j][r] = ld_stream_f64x2(rows[r] + c + j * NT);
             }
 #pragma unroll
             for (int j = 0; j < U; ++j) uv[j] = __ldg(u2 + c + j * NT);
@@ -197,7 +179,7 @@ __global__ void __launch_bounds__(MV_NT, MV_MINB) matvec_seg_kernel(const Matvec
         for (; c < nvec; c += NT) {
             double2 qv[R];
 #pragma unroll
-            for (int r = 0; r < R; ++r) qv[r] = L2HINT ? ld_stream_hint_f64x2(rows[r] + c, pol) : ld_stream_f64x2(rows[r] + c);
+            for (int r = 0; r < R; ++r) qv[r] = ld_stream_f64x2(rows[r] + c);
             const double2 uv = __ldg(u2 + c);
 #pragma unroll
             for (int r = 0; r < R; ++r) {

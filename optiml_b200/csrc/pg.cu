@@ -24,49 +24,79 @@
 #include <stdlib.h>
 #include <memory>
 
-// ------------------------------------------------------------------------------------------ K2 launchers
+// ------------------------------------------------------------------------------------------ product launchers
+// Every product w = Q u of a solver runs one of three passes over the matrix: K2 (the full pass), K2s (the upper triangle,
+// opt-in) or K2e (the upper triangle with K2's bits, for exactly symmetric self-Grams).  launch_product checks the
+// operands and runs the pass a solver chose at creation (product_pass).
+enum ProductPass : int { PASS_FULL, PASS_SYMMETRIC, PASS_EXACT };
+
+// a grow-only device buffer of the context's product scratch
+struct ScratchBuf {
+    void* p = nullptr;
+    size_t bytes = 0;
+    template <typename T>
+    T* as() const { return static_cast<T*>(p); }
+};
+
 struct MatvecScratch {
-    double* wpart = nullptr;
-    unsigned* tickets = nullptr;
-    size_t wpart_elems = 0, ticket_elems = 0;
-    // symmetric pass (K2s): row / column partials and the plan of the (n, ld, rank, ranks) it was last built for
-    double* sy_rowpart = nullptr;
-    double* sy_colpart = nullptr;
-    SymvItem* sy_items = nullptr;
-    int* sy_nseg = nullptr;     // per band: row-sum slots; behind them: band of every `unit` rows
-    size_t sy_row_elems = 0, sy_col_elems = 0, sy_item_cap = 0, sy_nseg_cap = 0;
+    ScratchBuf wpart, tickets;   // segment partials (K2, K2 x NB, K2e); one ticket per row group (K2), zero between passes
+    // K2s: row / column partials, work items, row-sum slots + band of every `unit` rows, and the plan of the
+    // (n, ld, rank, ranks) they were last built for
+    ScratchBuf sy_rowpart, sy_colpart, sy_items, sy_tables;
     int64_t sy_n = -1, sy_ld = -1;
     int sy_rank = -1, sy_P = -1;
     SymvPlan sy_plan;
     // K2e: column chains and the (A, B) segment pairs of the grid, for ex_nseg segments
-    double* ex_colchain = nullptr;
-    int2* ex_pairs = nullptr;
-    size_t ex_cc_elems = 0, ex_pair_cap = 0;
+    ScratchBuf ex_colchain, ex_pairs;
     int ex_nseg = -1;
 };
 
+static MatvecScratch& matvec_scratch(svmb200_ctx* ctx) {
+    if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
+    return *static_cast<MatvecScratch*>(ctx->matvec_scratch);
+}
+
+void svm_release_matvec_scratch(svmb200_ctx* ctx) {
+    MatvecScratch* s = static_cast<MatvecScratch*>(ctx->matvec_scratch);
+    if (!s) return;
+    for (ScratchBuf* b : {&s->wpart, &s->tickets, &s->sy_rowpart, &s->sy_colpart, &s->sy_items, &s->sy_tables,
+                          &s->ex_colchain, &s->ex_pairs})
+        if (b->p) cudaFree(b->p);
+    delete s;
+    ctx->matvec_scratch = nullptr;
+}
+
+// `count` elements of T at least, and never an empty buffer (the kernels take its address either way)
+template <typename T>
+static int reserve(svmb200_ctx* ctx, ScratchBuf& b, size_t count) {
+    return svm_scratch_reserve(ctx, &b.p, &b.bytes, (count ? count : 1) * sizeof(T));
+}
+
+static int mv_nseg(int64_t ld) { return (int)((ld + MV_SEG - 1) / MV_SEG); }
+
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// the context's sticky exchange-fault flag (see ll_load)
+static int* exchange_fault(svmb200_ctx* ctx) { return reinterpret_cast<int*>(ctx->arena + ARENA_LOCAL_OFF + 8); }
+
+// the checks of every product: the leading dimension against the rule of its pass, 16-byte matrix and vectors
+static int check_operands(bool ld_ok, const char* ld_rule, bool aligned) {
+    if (!ld_ok) {
+        svmb200_set_error("product: ld must be %s", ld_rule);
+        return SVMB200_ERR_ARG;
+    }
+    if (!aligned) {
+        svmb200_set_error("product: operands must be 16-byte aligned");
+        return SVMB200_ERR_ARG;
+    }
+    return SVMB200_OK;
+}
+
 static int matvec_scratch_reserve(svmb200_ctx* ctx, MatvecScratch& s, int64_t nrows, int64_t ld, int nvec = 1) {
-    const int nseg = (int)((ld + MV_SEG - 1) / MV_SEG);
-    const size_t nrows_pad = (size_t)round_up64(nrows, 16);
-    const size_t need_w = (size_t)nvec * nseg * nrows_pad;
-    const size_t need_t = (size_t)((nrows + MV_GROUP - 1) / MV_GROUP);
-    if (need_w > s.wpart_elems) {
-        SVM_CUDA(cudaStreamSynchronize(ctx->stream));
-        if (s.wpart) cudaFree(s.wpart);
-        s.wpart = nullptr;
-        s.wpart_elems = 0;
-        SVM_CUDA(cudaMalloc(&s.wpart, need_w * sizeof(double)));
-        s.wpart_elems = need_w;
-    }
-    if (need_t > s.ticket_elems) {
-        SVM_CUDA(cudaStreamSynchronize(ctx->stream));
-        if (s.tickets) cudaFree(s.tickets);
-        s.tickets = nullptr;
-        s.ticket_elems = 0;
-        SVM_CUDA(cudaMalloc(&s.tickets, need_t * sizeof(unsigned)));
-        SVM_CUDA(cudaMemsetAsync(s.tickets, 0, need_t * sizeof(unsigned), ctx->stream));
-        s.ticket_elems = need_t;
-    }
+    SVM_TRY(reserve<double>(ctx, s.wpart, (size_t)nvec * mv_nseg(ld) * (size_t)round_up64(nrows, 16)));
+    const size_t had = s.tickets.bytes;
+    SVM_TRY(reserve<unsigned>(ctx, s.tickets, (size_t)((nrows + MV_GROUP - 1) / MV_GROUP)));
+    if (s.tickets.bytes != had) SVM_CUDA(cudaMemsetAsync(s.tickets.p, 0, s.tickets.bytes, ctx->stream));
     return SVMB200_OK;
 }
 
@@ -76,65 +106,65 @@ struct ExchangeTargets {
     ulonglong2* peer_w[SVM_MAX_RANKS] = {};
 };
 
-static int launch_matvec(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, const double* du, double* dw,
-                         const double* du_rows, double* ddenpart, const int* d_done,
-                         const ExchangeTargets* xt = nullptr) {
-    if (nrows <= 0) return SVMB200_OK;  // an empty shard has nothing to compute or to send
-    if (ld % 2 != 0 || ld <= 0) {
-        svmb200_set_error("matvec: ld must be a positive multiple of 2");
-        return SVMB200_ERR_ARG;
-    }
-    if ((reinterpret_cast<uintptr_t>(dQ) & 15) || (reinterpret_cast<uintptr_t>(du) & 15)) {
-        svmb200_set_error("matvec: operands must be 16-byte aligned");
-        return SVMB200_ERR_ARG;
-    }
-    if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
-    MatvecScratch& s = *static_cast<MatvecScratch*>(ctx->matvec_scratch);
-    SVM_TRY(matvec_scratch_reserve(ctx, s, nrows, ld));
+// One product: w = Q u over the n x ld matrix, or over this rank's shard of nrows rows (K2).  With u_rows / denpart, also
+// the shares of u'w per 64-row group; with `done`, nothing runs once the solver's device state says so.  With xt, the
+// results go straight into every rank's gathered buffer (fused exchange; w and denpart then only carry the slot
+// geometry), under sequence number seq; rpr is the rows per rank of that exchange.  phase: see launch_symv.
+struct ProductOperands {
+    const double* Q = nullptr;
+    int64_t n = 0, nrows = 0, ld = 0, rpr = 0;
+    const double* u = nullptr;
+    double* w = nullptr;
+    const double* u_rows = nullptr;
+    double* denpart = nullptr;
+    const int* done = nullptr;
+    const ExchangeTargets* xt = nullptr;
+    unsigned long long seq = 0;
+    int phase = 0;
+};
+
+static int launch_matvec(svmb200_ctx* ctx, const ProductOperands& op) {
+    MatvecScratch& s = matvec_scratch(ctx);
+    SVM_TRY(matvec_scratch_reserve(ctx, s, op.nrows, op.ld));
     MatvecArgs a;
-    a.Q = dQ;
-    a.ld = ld;
-    a.nrows = nrows;
-    a.u = du;
-    a.w = dw;
-    a.wpart = s.wpart;
-    a.nrows_pad = round_up64(nrows, 16);
-    a.tickets = s.tickets;
-    a.u_rows = du_rows;
-    a.denpart = ddenpart;
-    a.nseg = (int)((ld + MV_SEG - 1) / MV_SEG);
-    a.done = d_done;
-    const int64_t ngroups = (nrows + MV_GROUP - 1) / MV_GROUP;
+    a.Q = op.Q;
+    a.ld = op.ld;
+    a.nrows = op.nrows;
+    a.u = op.u;
+    a.w = op.w;
+    a.wpart = s.wpart.as<double>();
+    a.nrows_pad = round_up64(op.nrows, 16);
+    a.tickets = s.tickets.as<unsigned>();
+    a.u_rows = op.u_rows;
+    a.denpart = op.denpart;
+    a.nseg = mv_nseg(op.ld);
+    a.done = op.done;
+    const int64_t ngroups = (op.nrows + MV_GROUP - 1) / MV_GROUP;
     a.nranks_x = 0;
     a.tag = 0;
     a.fault = nullptr;
-    if (xt != nullptr) {
-        a.nranks_x = xt->nranks;
-        a.tag = xt->tag;
-        a.fault = reinterpret_cast<const int*>(ctx->arena + ARENA_LOCAL_OFF + 8);
-        for (int r = 0; r < xt->nranks; ++r) a.peer_w[r] = xt->peer_w[r];
+    if (op.xt != nullptr) {
+        a.nranks_x = op.xt->nranks;
+        a.tag = op.xt->tag;
+        a.fault = exchange_fault(ctx);
+        for (int r = 0; r < op.xt->nranks; ++r) a.peer_w[r] = op.xt->peer_w[r];
     }
     const int64_t nitems = ngroups * MV_BPG * a.nseg;
     if (nitems >= (1ll << 31)) {
         svmb200_set_error("matvec: grid too large");
         return SVMB200_ERR_ARG;
     }
-    static const bool l2_hint = [] {
-        const char* ev = getenv("SVMB200_MATVEC_L2_HINT");
-        return ev != nullptr && atoi(ev) != 0;
-    }();
-    if (l2_hint) SVM_CUDA(svm_launch_chained(matvec_seg_kernel<true>, dim3((unsigned)nitems), dim3(MV_NT), ctx->stream, a));
-    else SVM_CUDA(svm_launch_chained(matvec_seg_kernel<false>, dim3((unsigned)nitems), dim3(MV_NT), ctx->stream, a));
+    SVM_CUDA(svm_launch_chained(matvec_seg_kernel, dim3((unsigned)nitems), dim3(MV_NT), ctx->stream, a));
     ctx->launches++;
     return SVMB200_OK;
 }
 
 // ------------------------------------------------------------------------------------------ K2s launcher
-// w = Q u from the upper triangle of the symmetric matrix (see k2_symv.cuh); same outputs as launch_matvec (w, and the
-// shares of u'w per 64-row group when du_rows / ddenpart are given).  One rank holding the whole matrix, or the ranks of
-// a fused peer exchange (xt != null): `phase` 1 = tile pass + the column sums for the other ranks, 2 = combine (waits
-// for the column sums of the others), 0 = both.  A single host thread that drives several ranks issues phase 1 for all
-// of them before phase 2 (the host emulation runs launches synchronously; on hardware the order is immaterial).
+// w = Q u from the upper triangle of the symmetric matrix (see k2_symv.cuh); same outputs as launch_matvec.  One rank
+// holding the whole matrix, or the ranks of a fused peer exchange (op.xt != null): `phase` 1 = tile pass + the column sums
+// for the other ranks, 2 = combine (waits for the column sums of the others), 0 = both.  A single host thread that drives
+// several ranks issues phase 1 for all of them before phase 2 (the host emulation runs launches synchronously; on hardware
+// the order is immaterial).
 constexpr size_t symv_inbox_bytes(int64_t rpr, int P) { return (size_t)P * (size_t)rpr * sizeof(ulonglong2); }
 static size_t symv_inbox_off(const svmb200_ctx* ctx) { return ctx->arena_bytes / 2; }
 
@@ -149,55 +179,28 @@ static int symv_plan_slots(int sm_count) {
 #endif
 }
 
-static int launch_symv(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t rpr, const double* du, double* dw,
-                       const double* du_rows, double* ddenpart, const int* d_done, const ExchangeTargets* xt = nullptr,
-                       unsigned long long seq = 0, int phase = 0) {
+static int launch_symv(svmb200_ctx* ctx, const ProductOperands& op) {
     using S = SymvDefault;
-    if (n <= 0) return SVMB200_OK;
-    if (ld % 2 != 0 || ld < n) {
-        svmb200_set_error("symv: ld must be even and at least n");
-        return SVMB200_ERR_ARG;
-    }
-    if ((reinterpret_cast<uintptr_t>(dQ) & 15) || (reinterpret_cast<uintptr_t>(du) & 15)) {
-        svmb200_set_error("symv: operands must be 16-byte aligned");
-        return SVMB200_ERR_ARG;
-    }
+    const ExchangeTargets* xt = op.xt;
+    const int64_t n = op.n, ld = op.ld, rpr = op.rpr;
     const int P = xt ? xt->nranks : 1, rank = xt ? ctx->rank : 0;
-    if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
-    MatvecScratch& s = *static_cast<MatvecScratch*>(ctx->matvec_scratch);
+    MatvecScratch& s = matvec_scratch(ctx);
     if (s.sy_n != n || s.sy_ld != ld || s.sy_rank != rank || s.sy_P != P) {
+        s.sy_n = -1;   // until the tables of the new plan are on the device
         SymvPlan& plan = s.sy_plan;
         symv_build_plan<S>(n, ld, rank, P, P == 1 ? n : rpr, plan, symv_plan_slots(ctx->sm_count));
-        const size_t n_pad = (size_t)round_up64(plan.nrows, 16);
-        const size_t need_r = (size_t)plan.nseg_max * n_pad, need_c = (size_t)plan.nbands * ld;
-        const size_t need_t = plan.nseg.size() + plan.band_of_unit.size();
-        if (need_r > s.sy_row_elems || need_c > s.sy_col_elems || plan.items.size() > s.sy_item_cap || need_t > s.sy_nseg_cap) {
-            SVM_CUDA(cudaStreamSynchronize(ctx->stream));
-            if (s.sy_rowpart) cudaFree(s.sy_rowpart);
-            if (s.sy_colpart) cudaFree(s.sy_colpart);
-            if (s.sy_items) cudaFree(s.sy_items);
-            if (s.sy_nseg) cudaFree(s.sy_nseg);
-            s.sy_rowpart = s.sy_colpart = nullptr;
-            s.sy_items = nullptr;
-            s.sy_nseg = nullptr;
-            s.sy_row_elems = s.sy_col_elems = s.sy_item_cap = s.sy_nseg_cap = 0;
-            s.sy_n = s.sy_ld = -1;
-            SVM_CUDA(cudaMalloc(&s.sy_rowpart, (need_r ? need_r : 1) * sizeof(double)));
-            s.sy_row_elems = need_r;
-            SVM_CUDA(cudaMalloc(&s.sy_colpart, (need_c ? need_c : 1) * sizeof(double)));
-            s.sy_col_elems = need_c;
-            SVM_CUDA(cudaMalloc(&s.sy_items, (plan.items.size() + 1) * sizeof(SymvItem)));
-            s.sy_item_cap = plan.items.size();
-            SVM_CUDA(cudaMalloc(&s.sy_nseg, (need_t + 1) * sizeof(int)));
-            s.sy_nseg_cap = need_t;
-        }
+        SVM_TRY(reserve<double>(ctx, s.sy_rowpart, (size_t)plan.nseg_max * (size_t)round_up64(plan.nrows, 16)));
+        SVM_TRY(reserve<double>(ctx, s.sy_colpart, (size_t)plan.nbands * ld));
+        SVM_TRY(reserve<SymvItem>(ctx, s.sy_items, plan.items.size()));
+        SVM_TRY(reserve<int>(ctx, s.sy_tables, plan.nseg.size() + plan.band_of_unit.size()));
         if (!plan.items.empty())
-            SVM_CUDA(cudaMemcpyAsync(s.sy_items, plan.items.data(), plan.items.size() * sizeof(SymvItem), cudaMemcpyHostToDevice, ctx->stream));
+            SVM_CUDA(cudaMemcpyAsync(s.sy_items.p, plan.items.data(), plan.items.size() * sizeof(SymvItem), cudaMemcpyHostToDevice,
+                                     ctx->stream));
         if (!plan.nseg.empty())
-            SVM_CUDA(cudaMemcpyAsync(s.sy_nseg, plan.nseg.data(), plan.nseg.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+            SVM_CUDA(cudaMemcpyAsync(s.sy_tables.p, plan.nseg.data(), plan.nseg.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
         if (!plan.band_of_unit.empty())
-            SVM_CUDA(cudaMemcpyAsync(s.sy_nseg + plan.nseg.size(), plan.band_of_unit.data(), plan.band_of_unit.size() * sizeof(int),
-                                     cudaMemcpyHostToDevice, ctx->stream));
+            SVM_CUDA(cudaMemcpyAsync(s.sy_tables.as<int>() + plan.nseg.size(), plan.band_of_unit.data(),
+                                     plan.band_of_unit.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
         SVM_CUDA(cudaStreamSynchronize(ctx->stream));  // once per problem size; the tables stay valid for every later pass
         s.sy_n = n;
         s.sy_ld = ld;
@@ -207,34 +210,29 @@ static int launch_symv(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
     const SymvPlan& plan = s.sy_plan;
     if (plan.nrows <= 0) return SVMB200_OK;
     const long long n_pad = round_up64(plan.nrows, 16);
-    const int* fault = xt ? reinterpret_cast<const int*>(ctx->arena + ARENA_LOCAL_OFF + 8) : nullptr;
+    int* fault = xt ? exchange_fault(ctx) : nullptr;
     const unsigned tag = xt ? xt->tag : 0u;
-    const size_t inbox_par = xt ? symv_inbox_off(ctx) + (size_t)(seq & 1) * symv_inbox_bytes(rpr, P) : 0;
-    if (phase == 0 || phase == 1) {
+    const size_t inbox_par = xt ? symv_inbox_off(ctx) + (size_t)(op.seq & 1) * symv_inbox_bytes(rpr, P) : 0;
+    if (op.phase == 0 || op.phase == 1) {
         SymvArgs a;
-        a.Q = dQ;
+        a.Q = op.Q;
         a.ld = ld;
         a.nrows = plan.nrows;
         a.row0 = plan.row0;
         a.n_pad = n_pad;
-        a.u = du;
-        a.rowpart = s.sy_rowpart;
-        a.colpart = s.sy_colpart;
-        a.items = s.sy_items;
-        a.done = d_done;
+        a.u = op.u;
+        a.rowpart = s.sy_rowpart.as<double>();
+        a.colpart = s.sy_colpart.as<double>();
+        a.items = s.sy_items.as<SymvItem>();
+        a.done = op.done;
         a.fault = fault;
-        static bool attr_set[64] = {};   // per device: the ring needs more than the default 48 KB of dynamic shared memory
-        const bool tracked = ctx->device >= 0 && ctx->device < 64;
-        if (!tracked || !attr_set[ctx->device]) {
-            SVM_CUDA(cudaFuncSetAttribute(symv_tile_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::RING_BYTES));
-            if (tracked) attr_set[ctx->device] = true;
-        }
+        SVM_TRY(svm_opt_in_smem<symv_tile_kernel<S>>(ctx, S::RING_BYTES));
         SVM_CUDA(svm_launch_chained_smem(symv_tile_kernel<S>, dim3((unsigned)plan.items.size()), dim3(SY_NT),
                                          (size_t)S::RING_BYTES, ctx->stream, a));
         ctx->launches++;
         if (!plan.sends.empty()) {
             SymvSendArgs sa = {};
-            sa.colpart = s.sy_colpart;
+            sa.colpart = s.sy_colpart.as<double>();
             sa.ld = ld;
             sa.nsend = (int)plan.sends.size();
             long long total = 0;
@@ -244,36 +242,36 @@ static int launch_symv(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
                 total += plan.sends[(size_t)i].ncols;
             }
             sa.tag = tag;
-            sa.done = d_done;
+            sa.done = op.done;
             sa.fault = fault;
             SVM_CUDA(svm_launch_chained(symv_send_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), ctx->stream, sa));
             ctx->launches++;
         }
     }
-    if (phase == 0 || phase == 2) {
+    if (op.phase == 0 || op.phase == 2) {
         SymvCombineArgs c = {};
-        c.rowpart = s.sy_rowpart;
-        c.colpart = s.sy_colpart;
+        c.rowpart = s.sy_rowpart.as<double>();
+        c.colpart = s.sy_colpart.as<double>();
         c.ld = ld;
         c.nrows = plan.nrows;
         c.row0 = plan.row0;
         c.n_pad = n_pad;
         c.unit = plan.unit;
-        c.band_of_unit = s.sy_nseg + plan.nseg.size();
-        c.nseg = s.sy_nseg;
-        c.u_rows = du_rows;
-        c.w = dw;
-        c.denpart = ddenpart;
-        c.done = d_done;
+        c.band_of_unit = s.sy_tables.as<int>() + plan.nseg.size();
+        c.nseg = s.sy_tables.as<int>();
+        c.u_rows = op.u_rows;
+        c.w = op.w;
+        c.denpart = op.denpart;
+        c.done = op.done;
         c.nrecv = (int)plan.recvs.size();
         for (int i = 0; i < c.nrecv; ++i) c.recvs[i] = plan.recvs[(size_t)i];
         c.inbox = xt ? reinterpret_cast<const ulonglong2*>(ctx->arena + inbox_par) : nullptr;
         c.rpr = rpr;
         c.tag = tag;
-        c.fault = const_cast<int*>(fault);
+        c.fault = fault;
         if (xt != nullptr) {
             c.nranks_x = xt->nranks;
-            c.share_off = (long long)(ddenpart - dw);
+            c.share_off = (long long)(op.denpart - op.w);
             for (int r = 0; r < xt->nranks; ++r) c.peer_w[r] = xt->peer_w[r];
         }
         const int64_t ngroups = (plan.nrows + MV_GROUP - 1) / MV_GROUP;
@@ -281,13 +279,6 @@ static int launch_symv(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
         ctx->launches++;
     }
     return SVMB200_OK;
-}
-
-// w = Q u for a symmetric n x n matrix from its upper triangle (the lower one is never read)
-extern "C" int svmb200_symv(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw) {
-    SVM_TRY(svm_use(ctx));
-    SVM_CHECK_ARG(dQ != nullptr && du != nullptr && dw != nullptr && n >= 0, "bad argument");
-    return launch_symv(ctx, dQ, n, ld, n, du, dw, nullptr, nullptr, nullptr);
 }
 
 // bytes of the matrix one symmetric pass streams (diagonal blocks in full + everything to their right) and the shape of
@@ -353,31 +344,14 @@ extern "C" int svmb200_symv_plan_items(int64_t n, int64_t ld, int rank, int nran
     return SVMB200_OK;
 }
 
-void svm_release_matvec_scratch(svmb200_ctx* ctx) {
-    if (ctx->matvec_scratch) {
-        MatvecScratch* s = static_cast<MatvecScratch*>(ctx->matvec_scratch);
-        if (s->wpart) cudaFree(s->wpart);
-        if (s->tickets) cudaFree(s->tickets);
-        if (s->sy_rowpart) cudaFree(s->sy_rowpart);
-        if (s->sy_colpart) cudaFree(s->sy_colpart);
-        if (s->sy_items) cudaFree(s->sy_items);
-        if (s->sy_nseg) cudaFree(s->sy_nseg);
-        if (s->ex_colchain) cudaFree(s->ex_colchain);
-        if (s->ex_pairs) cudaFree(s->ex_pairs);
-        delete s;
-        ctx->matvec_scratch = nullptr;
-    }
-}
-
 // ------------------------------------------------------------------------------------------ K2e launcher
 // w = Q u with K2's bits from the upper triangle of an exactly symmetric n x n matrix (see k2_exact.cuh); same outputs as
-// launch_matvec on one rank (w, and the shares of u'w per 64-row group when du_rows / ddenpart are given).
-static int exact_nseg(int64_t ld) { return (int)((ld + MV_SEG - 1) / MV_SEG); }
+// launch_matvec on one rank.
 
 // at least two segments, and every segment but the last one made of real rows (the column chains of a segment cover all
 // of its rows)
 static bool exact_shape_ok(int64_t n, int64_t ld) {
-    const int nseg = exact_nseg(ld);
+    const int nseg = mv_nseg(ld);
     return n > 0 && ld >= n && ld % 2 == 0 && nseg >= 2 && n > (int64_t)(nseg - 1) * MV_SEG;
 }
 
@@ -393,93 +367,110 @@ static std::vector<int2> exact_pairs(int nseg) {
 
 static int exact_scratch_reserve(svmb200_ctx* ctx, MatvecScratch& s, int64_t n, int64_t ld) {
     SVM_TRY(matvec_scratch_reserve(ctx, s, n, ld));
-    const int nseg = exact_nseg(ld);
-    const size_t need_c = (size_t)exact_colchain_off(nseg - 1, ld), need_p = (size_t)nseg * (nseg + 1) / 2;
-    if (need_c > s.ex_cc_elems || need_p > s.ex_pair_cap) {
-        SVM_CUDA(cudaStreamSynchronize(ctx->stream));
-        if (s.ex_colchain) cudaFree(s.ex_colchain);
-        if (s.ex_pairs) cudaFree(s.ex_pairs);
-        s.ex_colchain = nullptr;
-        s.ex_pairs = nullptr;
-        s.ex_cc_elems = s.ex_pair_cap = 0;
-        s.ex_nseg = -1;
-        SVM_CUDA(cudaMalloc(&s.ex_colchain, need_c * sizeof(double)));
-        s.ex_cc_elems = need_c;
-        SVM_CUDA(cudaMalloc(&s.ex_pairs, need_p * sizeof(int2)));
-        s.ex_pair_cap = need_p;
-    }
+    const int nseg = mv_nseg(ld);
+    SVM_TRY(reserve<double>(ctx, s.ex_colchain, (size_t)exact_colchain_off(nseg - 1, ld)));
     if (s.ex_nseg != nseg) {
+        s.ex_nseg = -1;   // until the new table is on the device
         const std::vector<int2> pairs = exact_pairs(nseg);
-        SVM_CUDA(cudaMemcpyAsync(s.ex_pairs, pairs.data(), pairs.size() * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream));
+        SVM_TRY(reserve<int2>(ctx, s.ex_pairs, pairs.size()));
+        SVM_CUDA(cudaMemcpyAsync(s.ex_pairs.p, pairs.data(), pairs.size() * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream));
         SVM_CUDA(cudaStreamSynchronize(ctx->stream));  // once per segment count; the table stays valid for every later pass
         s.ex_nseg = nseg;
     }
     return SVMB200_OK;
 }
 
-static int launch_matvec_exact(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw,
-                               const double* du_rows, double* ddenpart, const int* d_done) {
+static int launch_matvec_exact(svmb200_ctx* ctx, const ProductOperands& op) {
     using S = ExactDefault;
-    if (!exact_shape_ok(n, ld)) {
-        svmb200_set_error("matvec_exact: needs an even ld >= n, two segments of %d columns or more and n > ld - %d",
-                          MV_SEG, MV_SEG);
-        return SVMB200_ERR_ARG;
-    }
-    if ((reinterpret_cast<uintptr_t>(dQ) & 15) || (reinterpret_cast<uintptr_t>(du) & 15)) {
-        svmb200_set_error("matvec_exact: operands must be 16-byte aligned");
-        return SVMB200_ERR_ARG;
-    }
-    if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
-    MatvecScratch& s = *static_cast<MatvecScratch*>(ctx->matvec_scratch);
-    SVM_TRY(exact_scratch_reserve(ctx, s, n, ld));
-    const int nseg = exact_nseg(ld);
-    const long long nrows_pad = round_up64(n, 16);
+    MatvecScratch& s = matvec_scratch(ctx);
+    SVM_TRY(exact_scratch_reserve(ctx, s, op.n, op.ld));
+    const int nseg = mv_nseg(op.ld);
+    const long long nrows_pad = round_up64(op.n, 16);
     ExactArgs a;
-    a.Q = dQ;
-    a.ld = ld;
-    a.n = n;
+    a.Q = op.Q;
+    a.ld = op.ld;
+    a.n = op.n;
     a.nrows_pad = nrows_pad;
-    a.u = du;
-    a.wpart = s.wpart;
-    a.colchain = s.ex_colchain;
-    a.pairs = s.ex_pairs;
-    a.done = d_done;
-    static bool attr_set[64] = {};   // per device: the ring needs more than the default 48 KB of dynamic shared memory
-    const bool tracked = ctx->device >= 0 && ctx->device < 64;
-    if (!tracked || !attr_set[ctx->device]) {
-        SVM_CUDA(cudaFuncSetAttribute(matvec_exact_tile_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::RING_BYTES));
-        if (tracked) attr_set[ctx->device] = true;
-    }
+    a.u = op.u;
+    a.wpart = s.wpart.as<double>();
+    a.colchain = s.ex_colchain.as<double>();
+    a.pairs = s.ex_pairs.as<int2>();
+    a.done = op.done;
+    SVM_TRY(svm_opt_in_smem<matvec_exact_tile_kernel<S>>(ctx, S::RING_BYTES));
     const unsigned nitems = (unsigned)((size_t)nseg * (nseg + 1) / 2 * MV_NT);
     SVM_CUDA(svm_launch_chained_smem(matvec_exact_tile_kernel<S>, dim3(nitems), dim3(MV_NT), (size_t)S::RING_BYTES, ctx->stream, a));
     ctx->launches++;
     ExactCombineArgs c;
-    c.wpart = s.wpart;
-    c.colchain = s.ex_colchain;
-    c.ld = ld;
-    c.nrows = n;
+    c.wpart = s.wpart.as<double>();
+    c.colchain = s.ex_colchain.as<double>();
+    c.ld = op.ld;
+    c.nrows = op.n;
     c.nrows_pad = nrows_pad;
     c.nseg = nseg;
-    c.u_rows = du_rows;
-    c.w = dw;
-    c.denpart = ddenpart;
-    c.done = d_done;
-    SVM_CUDA(svm_launch_chained(matvec_exact_combine_kernel, dim3((unsigned)((n + MV_GROUP - 1) / MV_GROUP)), dim3(MV_NT),
+    c.u_rows = op.u_rows;
+    c.w = op.w;
+    c.denpart = op.denpart;
+    c.done = op.done;
+    SVM_CUDA(svm_launch_chained(matvec_exact_combine_kernel, dim3((unsigned)((op.n + MV_GROUP - 1) / MV_GROUP)), dim3(MV_NT),
                                 ctx->stream, c));
     ctx->launches++;
     return SVMB200_OK;
 }
 
+// ------------------------------------------------------------------------------------------ one launch path
+static int launch_product(svmb200_ctx* ctx, ProductPass pass, const ProductOperands& op) {
+    static const char* const ld_rule[] = {"a positive multiple of 2", "even and at least n",
+                                          "even and at least n, with n reaching into the last of two or more column segments"};
+    if (pass == PASS_FULL ? op.nrows <= 0 : pass == PASS_SYMMETRIC && op.n <= 0)
+        return SVMB200_OK;   // an empty shard has nothing to compute or to send
+    const bool ld_ok = pass == PASS_FULL      ? op.ld > 0 && op.ld % 2 == 0
+                     : pass == PASS_SYMMETRIC ? op.ld % 2 == 0 && op.ld >= op.n
+                                              : exact_shape_ok(op.n, op.ld);
+    SVM_TRY(check_operands(ld_ok, ld_rule[pass], aligned16(op.Q) && aligned16(op.u)));
+    return pass == PASS_FULL ? launch_matvec(ctx, op) : pass == PASS_SYMMETRIC ? launch_symv(ctx, op) : launch_matvec_exact(ctx, op);
+}
+
+// w = Q u over an n x ld matrix (K2: over nrows = n rows of it) with no exchange, no shares of u'w
+static int launch_plain(svmb200_ctx* ctx, ProductPass pass, const double* dQ, int64_t n, int64_t ld, const double* du,
+                        double* dw, const int* d_done = nullptr) {
+    ProductOperands op;
+    op.Q = dQ;
+    op.n = op.nrows = op.rpr = n;
+    op.ld = ld;
+    op.u = du;
+    op.w = dw;
+    op.done = d_done;
+    return launch_product(ctx, pass, op);
+}
+
+int svm_launch_matvec(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, const double* du, double* dw,
+                      const int* d_done) {
+    return launch_plain(ctx, PASS_FULL, dQ, nrows, ld, du, dw, d_done);
+}
+
+extern "C" int svmb200_matvec(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, const double* du,
+                              double* dw) {
+    SVM_TRY(svm_use(ctx));
+    return launch_plain(ctx, PASS_FULL, dQ, nrows, ld, du, dw);
+}
+
+// w = Q u for a symmetric n x n matrix from its upper triangle (the lower one is never read)
+extern "C" int svmb200_symv(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw) {
+    SVM_TRY(svm_use(ctx));
+    SVM_CHECK_ARG(dQ != nullptr && du != nullptr && dw != nullptr && n >= 0, "bad argument");
+    return launch_plain(ctx, PASS_SYMMETRIC, dQ, n, ld, du, dw);
+}
+
 extern "C" int svmb200_matvec_exact(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, const double* du, double* dw) {
     SVM_TRY(svm_use(ctx));
     SVM_CHECK_ARG(dQ != nullptr && du != nullptr && dw != nullptr, "null operand");
-    return launch_matvec_exact(ctx, dQ, n, ld, du, dw, nullptr, nullptr, nullptr);
+    return launch_plain(ctx, PASS_EXACT, dQ, n, ld, du, dw);
 }
 
 extern "C" int svmb200_exact_symv_geometry(int64_t n, int64_t ld, int64_t* matrix_bytes, int64_t* scratch_bytes,
                                            int64_t* items) {
     SVM_CHECK_ARG(exact_shape_ok(n, ld), "the exact symmetric pass does not apply to this shape");
-    const int nseg = exact_nseg(ld);
+    const int nseg = mv_nseg(ld);
     int64_t elems = 0;
     for (const int2 pr : exact_pairs(nseg)) {
         const int64_t rowsA = std::min<int64_t>((int64_t)(pr.x + 1) * MV_SEG, n) - (int64_t)pr.x * MV_SEG;
@@ -492,17 +483,6 @@ extern "C" int svmb200_exact_symv_geometry(int64_t n, int64_t ld, int64_t* matri
     return SVMB200_OK;
 }
 
-int svm_launch_matvec(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, const double* du, double* dw,
-                      const int* d_done) {
-    return launch_matvec(ctx, dQ, nrows, ld, du, dw, nullptr, nullptr, d_done);
-}
-
-extern "C" int svmb200_matvec(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, const double* du,
-                              double* dw) {
-    SVM_TRY(svm_use(ctx));
-    return svm_launch_matvec(ctx, dQ, nrows, ld, du, dw, nullptr);
-}
-
 static int launch_matvec_multi(svmb200_ctx* ctx, const double* dQ, int64_t nrows, int64_t ld, int nb,
                                const double* const* du, double* const* dw, const double* const* du_rows,
                                double* const* ddenpart, const int* const* d_done, const ExchangeTargets* xt = nullptr,
@@ -512,30 +492,20 @@ static int launch_matvec_multi(svmb200_ctx* ctx, const double* dQ, int64_t nrows
         svmb200_set_error("matvec_multi: between 1 and %d vectors per launch", MV_MULTI_MAX);
         return SVMB200_ERR_ARG;
     }
-    if (ld % 2 != 0 || ld <= 0) {
-        svmb200_set_error("matvec: ld must be a positive multiple of 2");
-        return SVMB200_ERR_ARG;
-    }
-    if (reinterpret_cast<uintptr_t>(dQ) & 15) {
-        svmb200_set_error("matvec: operands must be 16-byte aligned");
-        return SVMB200_ERR_ARG;
-    }
-    if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
-    MatvecScratch& s = *static_cast<MatvecScratch*>(ctx->matvec_scratch);
+    bool aligned = aligned16(dQ);
+    for (int b = 0; b < nb; ++b) aligned = aligned && aligned16(du[b]);
+    SVM_TRY(check_operands(ld > 0 && ld % 2 == 0, "a positive multiple of 2", aligned));
+    MatvecScratch& s = matvec_scratch(ctx);
     SVM_TRY(matvec_scratch_reserve(ctx, s, nrows, ld, nb));
     MatvecMultiArgs a = {};
     a.Q = dQ;
     a.ld = ld;
     a.nrows = nrows;
     a.nrows_pad = round_up64(nrows, 16);
-    a.wpart = s.wpart;
-    a.tickets = s.tickets;
-    a.nseg = (int)((ld + MV_SEG - 1) / MV_SEG);
+    a.wpart = s.wpart.as<double>();
+    a.tickets = s.tickets.as<unsigned>();
+    a.nseg = mv_nseg(ld);
     for (int b = 0; b < nb; ++b) {
-        if (reinterpret_cast<uintptr_t>(du[b]) & 15) {
-            svmb200_set_error("matvec: operands must be 16-byte aligned");
-            return SVMB200_ERR_ARG;
-        }
         a.u[b] = du[b];
         a.w[b] = dw[b];
         a.u_rows[b] = du_rows ? du_rows[b] : nullptr;
@@ -547,7 +517,7 @@ static int launch_matvec_multi(svmb200_ctx* ctx, const double* dQ, int64_t nrows
         a.tag = xt->tag;
         a.xstride = xstride;
         a.share_off = share_off;
-        a.fault = reinterpret_cast<const int*>(ctx->arena + ARENA_LOCAL_OFF + 8);
+        a.fault = exchange_fault(ctx);
         for (int r = 0; r < xt->nranks; ++r) a.peer_w[r] = xt->peer_w[r];
     }
     const int64_t ngroups = (nrows + MV_GROUP - 1) / MV_GROUP;
@@ -638,8 +608,7 @@ struct svmb200_pg {
     double *x = nullptr, *g = nullptr, *d = nullptr, *u = nullptr, *w = nullptr;  // w: gathered [P][stride]
     int64_t stride = 0;  // rows_per_rank results + rows_per_rank / MV_GROUP shares of u'w
     bool p2p = false;           // fused exchange through the peer arena instead of ncclAllGather
-    bool symmetric = false;     // products from the upper triangle only (K2s; one rank holding the whole matrix)
-    bool exact = false;         // products from the upper triangle with K2's bits (K2e; svmb200_pg_set_self_gram)
+    ProductPass pass = PASS_FULL;   // the pass of its products (product_pass)
     unsigned long long cur_seq = 0;  // sequence number of the product the next vector kernel consumes
     int nctas = 1;
     double *q = nullptr, *lb = nullptr, *ub = nullptr;
@@ -689,7 +658,7 @@ static VecArgs make_vec_args(svmb200_pg* pg) {
         const size_t bufbytes = (size_t)pg->stride * ctx->nranks * sizeof(ulonglong2);
         a.gathered_ll = reinterpret_cast<const ulonglong2*>(ctx->arena + ARENA_DATA_OFF + (pg->cur_seq & 1) * bufbytes);
         a.tag = exchange_tag(pg->cur_seq);
-        a.fault = reinterpret_cast<int*>(ctx->arena + ARENA_LOCAL_OFF + 8);
+        a.fault = exchange_fault(ctx);
     }
     a.rpr = pg->rows_per_rank;
     a.stride = pg->stride;
@@ -727,7 +696,7 @@ static cudaEvent_t pooled_event(svmb200_ctx* ctx);
 static int pg_product(svmb200_pg* pg, bool timed, int phase = 0) {
     // w[row0 : row0+nrows] = Q_shard u, then all ranks exchange their shards (K4)
     svmb200_ctx* ctx = pg->ctx;
-    const bool split = pg->symmetric && pg->p2p;
+    const bool split = pg->pass == PASS_SYMMETRIC && pg->p2p;
     if (phase == 2 && !split) return SVMB200_OK;
     if (phase == 1 && !split) phase = 0;
     cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
@@ -747,9 +716,19 @@ static int pg_product(svmb200_pg* pg, bool timed, int phase = 0) {
         e1 = pg->mv_ev[pg->mv_ev.size() - 2];
         e2 = pg->mv_ev[pg->mv_ev.size() - 1];
     }
+    ProductOperands op;
+    op.Q = pg->dQ;
+    op.n = pg->n;
+    op.nrows = pg->nrows;
+    op.ld = pg->ld;
+    op.rpr = pg->rows_per_rank;
+    op.u = pg->u;
+    op.u_rows = pg->u + pg->row0;
+    op.done = &pg->st->done;
+    op.phase = phase;
+    ExchangeTargets xt;
     if (pg->p2p) {
         // K2 + K4 fused: results go straight into every rank's gathered buffer (parity = seq & 1)
-        ExchangeTargets xt;
         xt.nranks = ctx->nranks;
         const unsigned long long seq = phase == 2 ? pg->cur_seq : ++ctx->xseq;
         pg->cur_seq = seq;
@@ -758,30 +737,16 @@ static int pg_product(svmb200_pg* pg, bool timed, int phase = 0) {
         const size_t slot = ARENA_DATA_OFF + (seq & 1) * bufbytes + (size_t)ctx->rank * pg->stride * sizeof(ulonglong2);
         for (int r = 0; r < ctx->nranks; ++r) xt.peer_w[r] = reinterpret_cast<ulonglong2*>(ctx->peer_arena[r] + slot);
         // the plain pointers only carry the slot geometry (w at [0, rpr), shares at [rpr, stride)) in this mode
-        double* geom = reinterpret_cast<double*>(ctx->arena);
-        if (pg->symmetric) {
-            SVM_TRY(launch_symv(ctx, pg->dQ, pg->n, pg->ld, pg->rows_per_rank, pg->u, geom, pg->u + pg->row0,
-                                geom + pg->rows_per_rank, &pg->st->done, &xt, seq, phase));
-        } else {
-            SVM_TRY(launch_matvec(ctx, pg->dQ, pg->nrows, pg->ld, pg->u, geom, pg->u + pg->row0, geom + pg->rows_per_rank,
-                                  &pg->st->done, &xt));
-        }
-        if (e1 && phase != 1) SVM_CUDA(cudaEventRecord(e1, ctx->stream));
+        op.w = reinterpret_cast<double*>(ctx->arena);
+        op.xt = &xt;
+        op.seq = seq;
     } else {
-        double* wshard = pg->w + (size_t)ctx->rank * pg->stride;
-        if (pg->symmetric) {
-            SVM_TRY(launch_symv(ctx, pg->dQ, pg->n, pg->ld, pg->n, pg->u, wshard, pg->u, wshard + pg->rows_per_rank,
-                                &pg->st->done));
-        } else if (pg->exact) {
-            SVM_TRY(launch_matvec_exact(ctx, pg->dQ, pg->n, pg->ld, pg->u, wshard, pg->u, wshard + pg->rows_per_rank,
-                                        &pg->st->done));
-        } else {
-            SVM_TRY(launch_matvec(ctx, pg->dQ, pg->nrows, pg->ld, pg->u, wshard, pg->u + pg->row0,
-                                  wshard + pg->rows_per_rank, &pg->st->done));
-        }
-        if (e1) SVM_CUDA(cudaEventRecord(e1, ctx->stream));
-        if (ctx->nranks > 1) SVM_TRY(svm_comm_allgather(ctx, pg->w, pg->stride));
+        op.w = pg->w + (size_t)ctx->rank * pg->stride;   // this rank's shard, then the all-gather
     }
+    op.denpart = op.w + pg->rows_per_rank;
+    SVM_TRY(launch_product(ctx, pg->pass, op));
+    if (e1 && phase != 1) SVM_CUDA(cudaEventRecord(e1, ctx->stream));
+    if (!pg->p2p && ctx->nranks > 1) SVM_TRY(svm_comm_allgather(ctx, pg->w, pg->stride));
     if (e2 && phase != 1) SVM_CUDA(cudaEventRecord(e2, ctx->stream));
     if (phase != 2) pg->last_passes++;
     return SVMB200_OK;
@@ -919,6 +884,34 @@ static int check_create_args(const char* fn, svmb200_ctx* ctx, svmb200_pg** out,
     return SVMB200_OK;
 }
 
+// The pass of a solver's products, decided at creation and again by svmb200_pg_set_self_gram.  symmetric: the context
+// asked for K2s when the solver was created; self_gram: the matrix is a self-Gram svmb200_gram built, exactly symmetric.
+//   K2s  one rank holding the whole matrix, or the ranks of a fused peer exchange whose arena also holds the inboxes of
+//        the column sums (two parities x P senders x rows_per_rank tagged entries in its upper half)
+//   K2e  a self-Gram held whole by one rank, a solver with products (not SMO), a shape K2e covers and a 16-byte aligned
+//        matrix; it reads ~60 % of K2's bytes at n = 50 000.  SVMB200_EXACT_SYMV=0 keeps K2 (A/B runs), and so does a
+//        scratch for the column chains that cannot be allocated.
+//   K2   every other solver.
+// The persistent loop (K8) and lockstep batches (K2 x NB) are run modes of their own that bypass the pass.
+static ProductPass product_pass(svmb200_pg* pg, bool symmetric, bool self_gram) {
+    svmb200_ctx* ctx = pg->ctx;
+    const int P = ctx->nranks;
+    const bool whole = P == 1 && pg->row0 == 0 && pg->nrows == pg->n;
+    const size_t inbox = symv_inbox_off(ctx);
+    if (symmetric && (whole || (pg->p2p && ARENA_DATA_OFF + 2 * (size_t)pg->stride * P * sizeof(ulonglong2) <= inbox &&
+                                inbox % 16 == 0 && 2 * symv_inbox_bytes(pg->rows_per_rank, P) <= ctx->arena_bytes - inbox)))
+        return PASS_SYMMETRIC;
+    if (!self_gram || pg->solver == SOLVER_SMO || !whole || !exact_shape_ok(pg->n, pg->ld) || !aligned16(pg->dQ))
+        return PASS_FULL;
+    const char* ev = getenv("SVMB200_EXACT_SYMV");
+    if (ev != nullptr && atoi(ev) == 0) return PASS_FULL;
+    if (exact_scratch_reserve(ctx, matvec_scratch(ctx), pg->n, pg->ld) != SVMB200_OK) {
+        (void)cudaGetLastError();   // an out-of-memory error is not sticky
+        return PASS_FULL;
+    }
+    return PASS_EXACT;
+}
+
 // host-side description of an augmented-Lagrangian solve (SOLVER_AL)
 struct ALSpec {
     ALParams p;
@@ -1001,17 +994,12 @@ static int bcqp_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
     const bool every_rank_owns_rows = (int64_t)(P - 1) * rpr < n;
     pg->p2p = ctx->p2p_enabled && P > 1 && every_rank_owns_rows &&
               ARENA_DATA_OFF + 2 * (size_t)pg->stride * P * sizeof(ulonglong2) <= ctx->arena_bytes;
-    // symmetric pass: one rank with the whole matrix, or the ranks of a fused peer exchange whose arena also holds the
-    // inboxes of the column sums (two parities x P senders x rows_per_rank tagged entries in its upper half)
-    pg->symmetric = ctx->symmetric &&
-                    ((P == 1 && row0 == 0 && nrows == n) ||
-                     (pg->p2p && ARENA_DATA_OFF + 2 * (size_t)pg->stride * P * sizeof(ulonglong2) <= symv_inbox_off(ctx) &&
-                      symv_inbox_off(ctx) % 16 == 0 && 2 * symv_inbox_bytes(rpr, P) <= ctx->arena_bytes - symv_inbox_off(ctx)));
     pg->nctas = (int)((n + VP_ELEMS - 1) / VP_ELEMS);
     if (pg->nctas > VP_MAXC) pg->nctas = VP_MAXC;
     if (pg->nctas < 1) pg->nctas = 1;
     pg->eps = eps;
     pg->solver = solver;
+    pg->pass = product_pass(pg, ctx->symmetric, false);
     pg->fw_t = fw_t;
     pg->max_iter = max_iter;
     pg->hist_cap = max_iter + 1 < (1ll << 24) ? max_iter + 1 : (1ll << 24);
@@ -1136,7 +1124,7 @@ static int poll_enqueue(svmb200_pg* pg, int slot) {
     int* fault = reinterpret_cast<int*>(dst + POLL_SLOT_BYTES - sizeof(int));
     *fault = 0;
     if (pg->p2p)
-        SVM_CUDA(cudaMemcpyAsync(fault, pg->ctx->arena + ARENA_LOCAL_OFF + 8, sizeof(int), cudaMemcpyDeviceToHost, s));
+        SVM_CUDA(cudaMemcpyAsync(fault, exchange_fault(pg->ctx), sizeof(int), cudaMemcpyDeviceToHost, s));
     SVM_CUDA(cudaEventRecord(pg->ev_poll[slot], s));
     return SVMB200_OK;
 }
@@ -1163,18 +1151,13 @@ static int poll_wait(svmb200_pg* pg, int slot) {
 constexpr size_t COOP_SMEM_MAX = 221 * 1024;
 
 // Ready a cooperative launch of `kernel` on `grid` CTAs of `block` threads and `smem` bytes of dynamic shared memory: the
-// opt-in to COOP_SMEM_MAX (once per device and kernel), the check that such a grid can be co-resident (it cannot on a
-// partitioned GPU), and the context's grid barrier.  *fits tells whether the grid can run.
+// opt-in to COOP_SMEM_MAX, the check that such a grid can be co-resident (it cannot on a partitioned GPU), and the
+// context's grid barrier.  *fits tells whether the grid can run.
 template <auto kernel>
 static int cooperative_setup(svmb200_ctx* ctx, int grid, int block, size_t smem, bool* fits) {
     *fits = true;
 #ifndef SVMB200_HOST_EMULATION
-    static bool configured[64] = {};
-    const int dev = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
-    if (!configured[dev]) {
-        SVM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM_MAX));
-        configured[dev] = true;
-    }
+    SVM_TRY(svm_opt_in_smem<kernel>(ctx, (int)COOP_SMEM_MAX));
     int per_sm = 0;
     SVM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, block, smem));
     *fits = (long long)per_sm * ctx->sm_count >= grid;
@@ -1516,7 +1499,7 @@ static int batch_poll(svmb200_ctx* ctx, svmb200_pg* const* pgs, int count, int* 
     SVM_CUDA(cudaStreamSynchronize(ctx->stream));
     if (bx.p2p) {
         int fault = 0;
-        SVM_CUDA(cudaMemcpy(&fault, ctx->arena + ARENA_LOCAL_OFF + 8, sizeof(int), cudaMemcpyDeviceToHost));
+        SVM_CUDA(cudaMemcpy(&fault, exchange_fault(ctx), sizeof(int), cudaMemcpyDeviceToHost));
         if (fault) {
             svmb200_set_error("peer exchange timed out: a rank stopped publishing its product shards");
             return SVMB200_ERR_STATE;
@@ -1576,7 +1559,7 @@ extern "C" int svmb200_pg_run_batch(svmb200_pg* const* pgs, int count, int64_t* 
             if (bx.p2p) {
                 hv[b].gathered_ll = reinterpret_cast<const ulonglong2*>(ctx->arena + bx.base + (size_t)b * bx.bufbytes);
                 hv[b].ll_pstride = (long long)((size_t)count * bx.bufbytes / sizeof(ulonglong2));
-                hv[b].fault = reinterpret_cast<int*>(ctx->arena + ARENA_LOCAL_OFF + 8);
+                hv[b].fault = exchange_fault(ctx);
             }
         }
         SVM_CUDA(cudaMemcpyAsync(dva, hv.data(), (size_t)count * sizeof(VecArgs), cudaMemcpyHostToDevice, ctx->stream));
@@ -1705,40 +1688,25 @@ extern "C" int svmb200_pg_set_profile(svmb200_pg* pg, int on) {
 }
 
 // 1 when the solver's products come from the upper triangle alone (svmb200_ctx_set_symmetric was on at its creation and
-// it holds the whole matrix on one rank)
+// it holds the whole matrix on one rank, or exchanges its shard through the peer arena)
 extern "C" int svmb200_pg_is_symmetric(svmb200_pg* pg, int* on) {
     SVM_CHECK_ARG(pg != nullptr && on != nullptr, "null argument");
-    *on = pg->symmetric ? 1 : 0;
+    *on = pg->pass == PASS_SYMMETRIC ? 1 : 0;
     return SVMB200_OK;
 }
 
-// The solver's matrix is a self-Gram svmb200_gram built (same = 1): exactly symmetric.  On one rank holding the whole
-// matrix, without the opt-in symmetric pass, the products then come from its upper triangle with K2's bits (K2e), which
-// reads ~60 % of the bytes at n = 50 000.  Products already taken by K2 (the first one, at creation) have the same bits.
-// SVMB200_EXACT_SYMV=0 keeps K2 (A/B runs).  When the scratch of the column chains cannot be allocated, the solver
-// keeps K2 as well.
+// The solver's matrix is a self-Gram svmb200_gram built (same = 1): exactly symmetric, and the solver may take K2e
+// (product_pass).  Products already taken by K2 (the first one, at creation) have the same bits.
 extern "C" int svmb200_pg_set_self_gram(svmb200_pg* pg, int on) {
     SVM_CHECK_ARG(pg != nullptr, "null solver");
-    const char* ev = getenv("SVMB200_EXACT_SYMV");
-    const bool allowed = ev == nullptr || atoi(ev) != 0;
-    pg->exact = on != 0 && allowed && pg->solver != SOLVER_SMO && pg->ctx->nranks == 1 && pg->row0 == 0 &&
-                pg->nrows == pg->n && !pg->symmetric && exact_shape_ok(pg->n, pg->ld) &&
-                (reinterpret_cast<uintptr_t>(pg->dQ) & 15) == 0;
-    if (pg->exact) {
-        svmb200_ctx* ctx = pg->ctx;
-        SVM_TRY(svm_use(ctx));
-        if (!ctx->matvec_scratch) ctx->matvec_scratch = new MatvecScratch();
-        if (exact_scratch_reserve(ctx, *static_cast<MatvecScratch*>(ctx->matvec_scratch), pg->n, pg->ld) != SVMB200_OK) {
-            (void)cudaGetLastError();   // an out-of-memory error is not sticky
-            pg->exact = false;
-        }
-    }
+    SVM_TRY(svm_use(pg->ctx));
+    pg->pass = product_pass(pg, pg->pass == PASS_SYMMETRIC, on != 0);
     return SVMB200_OK;
 }
 
 extern "C" int svmb200_pg_is_exact_symv(svmb200_pg* pg, int* on) {
     SVM_CHECK_ARG(pg != nullptr && on != nullptr, "null argument");
-    *on = pg->exact ? 1 : 0;
+    *on = pg->pass == PASS_EXACT ? 1 : 0;
     return SVMB200_OK;
 }
 

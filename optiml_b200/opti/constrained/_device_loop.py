@@ -76,14 +76,18 @@ class DeviceLoopMixin:
         h = create_solvers(self._create_symbol, H,
                            lambda hh: (N.ptr(q), N.ptr(lb), N.ptr(ub), N.ptr(x0), float(self.eps), int(self.max_iter),
                                        *self._extra_create_args(), C.byref(hh)))
+        self._after_create(h, profile)
+        return h, n
+
+    def _after_create(self, h, profile):
+        """Profiling on request, and which pass the solver's products take (csrc/pg.cu, product_pass)."""
         if profile:
             N.call('svmb200_pg_set_profile', h, 1)
-        sym = C.c_int(0)
-        N.call('svmb200_pg_is_symmetric', h, C.byref(sym))
-        self.symmetric_pass = bool(sym.value)   # products from the upper triangle only (runtime.use_symmetric_pass)
-        N.call('svmb200_pg_is_exact_symv', h, C.byref(sym))
-        self.exact_symv_pass = bool(sym.value)   # the full pass's bits from the upper triangle (a self-Gram on one GPU)
-        return h, n
+        on = C.c_int(0)
+        N.call('svmb200_pg_is_symmetric', h, C.byref(on))
+        self.symmetric_pass = bool(on.value)   # products from the upper triangle only (runtime.use_symmetric_pass)
+        N.call('svmb200_pg_is_exact_symv', h, C.byref(on))
+        self.exact_symv_pass = bool(on.value)   # the full pass's bits from the upper triangle (a self-Gram on one GPU)
 
     @staticmethod
     def _run(h, max_new):

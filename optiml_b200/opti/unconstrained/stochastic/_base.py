@@ -100,13 +100,7 @@ class StochasticOptimizer(DeviceLoopMixin, Optimizer):
             N.ptr(q), N.ptr(lb), N.ptr(ub), N.ptr(x0), N.ptr(a), b, float(f.rho), N.RULES[self._rule],
             N.MOMENTUM[momentum_type], N.ptr(lr), N.ptr(mom), float(k['decay']), float(k['beta1']), float(k['beta2']),
             float(k['offset']), float(self.tol), int(self.epochs), C.byref(hh)))
-        if profile:
-            N.call('svmb200_pg_set_profile', h, 1)
-        sym = C.c_int(0)
-        N.call('svmb200_pg_is_symmetric', h, C.byref(sym))
-        self.symmetric_pass = bool(sym.value)
-        N.call('svmb200_pg_is_exact_symv', h, C.byref(sym))
-        self.exact_symv_pass = bool(sym.value)   # the full pass's bits from the upper triangle (a self-Gram on one GPU)
+        self._after_create(h, profile)
         return h, n
 
     def _pull_state(self, h, n):

@@ -169,7 +169,7 @@ int main(int argc, char** argv) {
     m.nseg = nseg;
     const long long ngroups = (n + MV_GROUP - 1) / MV_GROUP;
     const unsigned nitems = (unsigned)(ngroups * MV_BPG * nseg);
-    const float ms_full = time_launches(reps / 2 + 1, [&]() { CK(svm_launch_chained(matvec_seg_kernel<false>, dim3(nitems), dim3(MV_NT), (cudaStream_t)0, m)); });
+    const float ms_full = time_launches(reps / 2 + 1, [&]() { CK(svm_launch_chained(matvec_seg_kernel, dim3(nitems), dim3(MV_NT), (cudaStream_t)0, m)); });
     printf("n = %lld  ld = %lld   full pass (K2): %8.4f ms  %7.1f GB/s\n", n, ld, ms_full, 8.0 * n * ld / ms_full / 1e6);
     run_shape<SymvDefault>(b, reps);
     if (argc > 3 && strcmp(argv[3], "one") == 0) return 0;   // profiling runs: the shipped shape only

@@ -36,12 +36,17 @@ def test_fits_are_bit_identical_with_and_without_the_exact_pass():
 
 
 def test_exact_pass_applies_only_where_it_is_exact(monkeypatch):
-    """one segment, a user-supplied matrix or the opt-in symmetric pass: the full pass"""
+    """one segment, a user-supplied matrix, the opt-in symmetric pass, a sharded matrix or SMO: the full pass; the
+    augmented-Lagrangian solvers take the exact pass like the box-constrained ones"""
+    import ctypes as C
     import numpy as np
-    from optiml_b200.ml.svm import DualSVC
+    from optiml_b200 import _native as N, runtime
+    from optiml_b200.ml.svm import SVC, DualSVC
     from optiml_b200.ml.svm.kernels import GaussianKernel
+    from optiml_b200.ml.svm.losses import hinge
     from optiml_b200.opti import Quadratic
     from optiml_b200.opti.constrained import ProjectedGradient
+    from optiml_b200.opti.unconstrained.stochastic import AdaGrad
     from symv_checks import symmetric_pass
     X, y = EX.data(600, 4)
     with emu_probe(defines=_SEG512), EX.exact_symv(True):
@@ -52,7 +57,38 @@ def test_exact_pass_applies_only_where_it_is_exact(monkeypatch):
             m = DualSVC(kernel=GaussianKernel(), max_iter=3).fit(X, y)
             assert m.optimizer.symmetric_pass and not m.optimizer.exact_symv_pass
             m.obj.release()
+        m = SVC(loss=hinge, kernel=GaussianKernel(), C=1, reg_intercept=False, dual=True, optimizer=AdaGrad, learning_rate=1.,
+                max_iter=3, random_state=5).fit(X, y)
+        assert m.optimizer.exact_symv_pass
+        m.obj.release()
         Q = np.eye(600) + 0.01
         pg = ProjectedGradient(quad=Quadratic(Q, np.ones(600)), ub=np.ones(600), max_iter=3).minimize()
         assert not pg.exact_symv_pass
         pg.f.release()
+        # SMO takes no products: svmb200_pg_set_self_gram leaves it alone
+        ctx = runtime.default_context()
+        ld = 608
+        Qp = np.zeros((600, ld))
+        Qp[:, :600] = Q
+        dQ = ctx.malloc(Qp.nbytes)
+        ctx.h2d(dQ, Qp)
+        ones = np.ones(600)
+        h, on = C.c_void_p(), C.c_int(1)
+        N.call('svmb200_smo_create', ctx.handle, C.c_void_p(dQ), 600, ld, 0, 600, N.HESSIAN_PLAIN, N.ptr(ones), N.ptr(-ones),
+               N.ptr(ones), 1e-3, 10, C.byref(h))
+        try:
+            N.call('svmb200_pg_set_self_gram', h, 1)
+            N.call('svmb200_pg_is_exact_symv', h, C.byref(on))
+            assert on.value == 0
+        finally:
+            N.load_library().svmb200_pg_destroy(h)
+            ctx.free(dQ)
+        # a matrix sharded over a single-process group of two GPUs
+        monkeypatch.setattr(runtime.DeviceGroup, 'MIN_ROWS_PER_GPU', 64)
+        runtime.use_devices([0, 1])
+        try:
+            m = DualSVC(kernel=GaussianKernel(), max_iter=3).fit(X, y)
+            assert len(m.obj.device_hessian().shards()) == 2 and not m.optimizer.exact_symv_pass
+            m.obj.release()
+        finally:
+            runtime.use_devices(None)
