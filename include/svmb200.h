@@ -206,9 +206,20 @@ int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld
 int svmb200_smo_create_signed(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
                               int hessian, const double* sign_host, const double* q_host, const double* ub_host,
                               double tol, int64_t max_iter, svmb200_pg** out);
-/* K14: `count` fresh resident or signed-view SMO solvers (svmb200_smo_create / _create_signed, not run yet, none twice)
- * on the same context, matrix, n, ld and layout, run to termination side by side: each problem gets its own range of
- * CTAs of one cooperative launch (at most one CTA per SM), keeps its own tol, max_iter, state and history, and ends
+/* The signed-view solver on a subset of the variables: active_host holds one byte per variable, and a variable whose
+ * byte is 0 is held at 0 (the solver sets its upper bound to 0; its ub_host and q_host entries are not used).  Such a
+ * variable is never selected and never changes m or M, and ties go to the larger index, so the active variables follow
+ * BIT FOR BIT the trajectory of the problem on them alone: with M from svmb200_gram over a subset of rows kept in index
+ * order, the problem of a cross-validation fold, whose training rows are some of M's rows.  Active variables must have
+ * finite upper bounds > 0, and both signs must occur among them (SVMB200_ERR_ARG otherwise).  Answers as for
+ * svmb200_smo_create_signed; svmb200_pg_state returns all n (SVR: 2n) variables, the inactive ones at alpha = 0.
+ * svmb200_smo_run_batch takes these solvers next to the plain signed-view ones on the same M. */
+int svmb200_smo_create_subset(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0, int64_t nrows,
+                              int hessian, const double* sign_host, const double* q_host, const double* ub_host,
+                              const unsigned char* active_host, double tol, int64_t max_iter, svmb200_pg** out);
+/* K14: `count` fresh resident or signed-view SMO solvers (svmb200_smo_create / _create_signed / _create_subset, not run
+ * yet, none twice) on the same context, matrix, n, ld and layout, run to termination side by side: each problem gets its
+ * own range of CTAs of one cooperative launch (at most one CTA per SM), keeps its own tol, max_iter, state and history, and ends
  * BIT-IDENTICAL to its own svmb200_pg_run.  Before every launch unfinished problems are admitted in index order while
  * their minimum grids (slices of at most 4 714 variables) fit the SMs, and the SMs are split evenly among them (no
  * problem above its own single-fit grid); a launch runs at most 4 096 iterations per problem; problems that finished give

@@ -69,6 +69,8 @@ PROTOTYPES = {
     'svmb200_smo_create': [c_vp, c_vp, i64, i64, i64, i64, C.c_int, c_vp, c_vp, c_vp, C.c_double, i64, C.POINTER(c_vp)],
     'svmb200_smo_create_signed': [c_vp, c_vp, i64, i64, i64, i64, C.c_int, c_vp, c_vp, c_vp, C.c_double, i64,
                                   C.POINTER(c_vp)],
+    'svmb200_smo_create_subset': [c_vp, c_vp, i64, i64, i64, i64, C.c_int, c_vp, c_vp, c_vp, c_vp, C.c_double, i64,
+                                  C.POINTER(c_vp)],
     'svmb200_smo_run_batch': [C.POINTER(c_vp), C.c_int, C.POINTER(i64), C.POINTER(C.c_int)],
     'svmb200_smo_create_rows': [c_vp, c_vp, i64, i64, i64, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, c_vp,
                                 c_vp, c_vp, C.c_double, i64, C.c_size_t, C.POINTER(c_vp)],

@@ -1813,10 +1813,11 @@ static int smo_setup(svmb200_ctx* ctx, int rows, int grid, size_t smem, bool* fi
                                      : cooperative_setup<smo_persistent_kernel<SMO_ROWS_RESIDENT>>(ctx, grid, SMO_NT, smem, fits);
 }
 
-// rows: the computed form (K12), else null; signed_view: dQ is an unsigned M read with the signs (SMO_ROWS_SIGNED)
+// rows: the computed form (K12), else null; signed_view: dQ is an unsigned M read with the signs (SMO_ROWS_SIGNED);
+// active: null, or one byte per variable of a signed view (svmb200_smo_create_subset): 0 holds the variable at 0
 static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int hessian, const double* sign_host,
                       const double* q_host, const double* ub_host, double tol, int64_t max_iter, const SmoRowsSpec* rows,
-                      bool signed_view, svmb200_pg** out) {
+                      bool signed_view, const unsigned char* active, svmb200_pg** out) {
     SVM_CHECK_ARG(max_iter > 0, "max_iter must be > 0");
     SVM_CHECK_ARG(tol >= 0.0, "tol must be >= 0");
     const int64_t nvars = hessian == SVMB200_HESSIAN_SVR ? 2 * n : n;
@@ -1830,9 +1831,23 @@ static int smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld,
             return SVMB200_ERR_ARG;
         }
     }
+    // an inactive variable gets ub = 0 (and alpha = 0, as every variable): it is then in neither I_up nor I_low, so it is
+    // never selected, never enters m or M, and the solve of the active variables is their own problem's solve
+    std::vector<double> ub_active;
+    bool side[2] = {false, false};
+    if (active) ub_active.assign(ub_host, ub_host + nvars);
     for (int64_t t = 0; t < nvars; ++t) {
         SVM_CHECK_ARG(sign_host[t] == 1.0 || sign_host[t] == -1.0, "signs must be +-1");
+        if (active && !active[t]) {
+            ub_active[(size_t)t] = 0.0;
+            continue;
+        }
         SVM_CHECK_ARG(ub_host[t] > 0.0 && ub_host[t] < INFINITY, "upper bounds must be finite and > 0");
+        side[sign_host[t] > 0.0] = true;
+    }
+    if (active) {
+        SVM_CHECK_ARG(side[0] && side[1], "the active variables must hold both signs of the equality constraint");
+        ub_host = ub_active.data();
     }
     int grid = ctx->sm_count > 0 ? ctx->sm_count : 1;
     if ((int64_t)grid * SMO_MIN_SLICE > nvars) grid = (int)((nvars + SMO_MIN_SLICE - 1) / SMO_MIN_SLICE);
@@ -1944,7 +1959,7 @@ extern "C" int svmb200_smo_create(svmb200_ctx* ctx, const double* dQ, int64_t n,
     SVM_TRY(check_create_args(__func__, ctx, out, dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr,
                               n, "Q is too small", ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
     SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
-    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, false, out);
+    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, false, nullptr, out);
 }
 
 extern "C" int svmb200_smo_create_signed(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0,
@@ -1953,7 +1968,18 @@ extern "C" int svmb200_smo_create_signed(svmb200_ctx* ctx, const double* dQ, int
     SVM_TRY(check_create_args(__func__, ctx, out, dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr,
                               n, "M is too small", ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
     SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
-    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, true, out);
+    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, true, nullptr, out);
+}
+
+extern "C" int svmb200_smo_create_subset(svmb200_ctx* ctx, const double* dQ, int64_t n, int64_t ld, int64_t row0,
+                                         int64_t nrows, int hessian, const double* sign_host, const double* q_host,
+                                         const double* ub_host, const unsigned char* active, double tol, int64_t max_iter,
+                                         svmb200_pg** out) {
+    SVM_TRY(check_create_args(__func__, ctx, out,
+                              dQ != nullptr && sign_host != nullptr && q_host != nullptr && ub_host != nullptr && active != nullptr,
+                              n, "M is too small", ld >= n && ld % 2 == 0, "ld must be >= n and even", hessian));
+    SVM_CHECK_ARG(row0 == 0 && nrows == n, "SMO needs the whole matrix on this rank (row0 = 0, nrows = n): it has no sharded form");
+    return smo_create(ctx, dQ, n, ld, hessian, sign_host, q_host, ub_host, tol, max_iter, nullptr, true, active, out);
 }
 
 extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel,
@@ -1979,7 +2005,7 @@ extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64
     rows.kf.degree = degree;
     rows.kf.int_degree = svm_gram_int_degree(degree);
     rows.cache_bytes = cache_bytes;
-    return smo_create(ctx, nullptr, n, 0, hessian, sign_host, q_host, ub_host, tol, max_iter, &rows, false, out);
+    return smo_create(ctx, nullptr, n, 0, hessian, sign_host, q_host, ub_host, tol, max_iter, &rows, false, nullptr, out);
 }
 
 extern "C" int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses) {
@@ -2059,8 +2085,8 @@ static int smo_run(svmb200_pg* pg, int64_t max_new) {
 }
 
 // ------------------------------------------------------------------------------------------ K14: SMO batch (k_smo.cuh)
-// Several resident or signed-view SMO problems on one matrix share the GPU: an SMO iteration is bound by the latency of
-// two grid barriers, not by bandwidth, and a smaller grid costs a problem little (profiles/smo_grid_sweep.jsonl).  So
+// Several resident or signed-view SMO problems (subsets included) on one matrix share the GPU: an SMO iteration is bound
+// by the latency of two grid barriers, not by bandwidth, and a smaller grid costs a problem little (profiles/smo_grid_sweep.jsonl).  So
 // problems run side by side on disjoint ranges of CTAs, at most one CTA per SM, in one cooperative launch of at most
 // SMO_BATCH_CHUNK iterations per problem.  Before every launch the scheduler admits unfinished problems in index order
 // while their minimum grids (slices of at most SMO_SLICE_MAX variables) fit the SMs, and splits the SMs evenly among

@@ -36,6 +36,19 @@ _SCOPE = ('optiml_b200 implements the dual formulation solved by a BoxConstraine
           'StochasticOptimizer (AdaGrad, ...); {} is outside that path')
 
 
+def _embed(nvars, cols, *vectors):
+    """A problem on the variables ``cols`` of a shared matrix with ``nvars`` variables: each vector spread to its
+    columns (1 elsewhere: a valid sign, never read as a bound or a linear term), and the mask of the active variables"""
+    out = []
+    for v in vectors:
+        full = np.ones(nvars)
+        full[cols] = v
+        out.append(full)
+    active = np.zeros(nvars, dtype=bool)
+    active[cols] = True
+    return out, active
+
+
 def _binarize(lb, y):
     """``lb.transform(y).ravel()`` for the labels ``lb`` was just fitted on (ml/svm/_base.py:440).  For a plain
     two-class 1-D target LabelBinarizer's answer is written down directly (int64, classes_[1] -> +1, classes_[0] -> -1):
@@ -141,14 +154,18 @@ class SVM(BaseEstimator):
             raise NotImplementedError
         return opt
 
-    def _make_solver(self, solver_cls, hessian, q, ub, eq_row):
+    def _make_solver(self, solver_cls, hessian, q, ub, eq_row, active=None):
         """The selected solver, ready to run, on  min x'Qx/2 + q'x : 0 <= x <= ub (, eq_row'x = 0 when the intercept
-        is not regularised); sets ``self.obj`` like ml/svm/_base.py:628-725."""
+        is not regularised); sets ``self.obj`` like ml/svm/_base.py:628-725.  ``active``: SMO on these variables only
+        (``_embed``)."""
         if solver_cls is SMO:
             # no callback: for a string optimizer there is no train_loss_history (SVM.__init__); the histories stay
             # on the solver
             self.obj = Quadratic(hessian, q)
-            return SMO(quad=self.obj, y=eq_row, C=ub, tol=self.tol, max_iter=self.max_iter, verbose=self.verbose)
+            return SMO(quad=self.obj, y=eq_row, C=ub, tol=self.tol, max_iter=self.max_iter, verbose=self.verbose,
+                       active=active)
+        if active is not None:
+            raise ValueError("a problem on a subset of a shared matrix's rows needs optimizer='smo'")
         if issubclass(solver_cls, BoxConstrainedQuadraticOptimizer):
             self.obj = Quadratic(hessian, q)
             solver = solver_cls(quad=self.obj, ub=ub, tol=self.tol, max_iter=self.max_iter,
@@ -271,12 +288,13 @@ class SVM(BaseEstimator):
     def support_vectors_(self, value):
         self._sv_host, self._sv_device = value, None
 
-    def _set_support_vectors(self, X):
+    def _set_support_vectors(self, X, rows=None):
+        """``rows``: the rows of the device copy of X that X's rows are (a fold's training rows in a shared matrix)"""
         dX, owned = getattr(self, '_train_X_device', None) or (None, False)
         self._train_X_device = None
         if dX is not None and dX.dptr and not isinstance(self.kernel, LinearKernel) and len(self.support_):
             ctx = dX.ctx
-            idx = np.ascontiguousarray(self.support_, dtype=np.int64)
+            idx = np.ascontiguousarray(self.support_ if rows is None else rows[self.support_], dtype=np.int64)
             sv = DeviceMatrix(ctx, len(idx), dX.cols, dX.ld)
             N.call('svmb200_gather_rows', ctx.handle, C.c_void_p(dX.dptr), dX.rows, dX.ld, dX.cols,
                    idx.ctypes.data_as(C.c_void_p), len(idx), C.c_void_p(sv.dptr), sv.ld)
@@ -369,10 +387,11 @@ class SVC(ClassifierMixin, SVM):
         self.fit_times_['solve_s'] = time.perf_counter() - t0
         return self._finish_fit(plan)
 
-    def _plan_fit(self, X, y, X_device=None, shared=None):
+    def _plan_fit(self, X, y, X_device=None, shared=None, rows=None):
         """Everything ``fit`` does before the solver runs.  ``shared``: an unsigned resident ``M = K + bias`` that other
         binary problems on the same X use too (one-vs-rest, ml/multiclass.py); the label signs are then applied by
-        the solver instead of being baked into a private copy of Q."""
+        the solver instead of being baked into a private copy of Q.  ``rows``: X and y are the rows ``rows`` (ascending)
+        of the set M was built on -- a cross-validation fold; the solver runs on those variables only (``_embed``)."""
         self.lb.fit(y)
         if len(self.lb.classes_) > 2:
             raise ValueError('use OneVsOneClassifier or OneVsRestClassifier from sklearn.multiclass '
@@ -390,16 +409,20 @@ class SVC(ClassifierMixin, SVM):
 
         # Q = K o yy' (+ yy' when the intercept is regularised)  (ml/svm/_base.py:552-554, 628), q = -1, 0 <= alpha <= C
         bias = self._bias()
+        ub, q, eq, active = np.ones(n) * self.C, -np.ones(n), y, None
         if shared is not None:
-            hessian = shared.with_signs(ys)
+            signs = ys
+            if rows is not None:
+                (signs, q, ub), active = _embed(shared.n, rows, ys, q, ub)
+                eq = signs
+            hessian = shared.with_signs(signs)
             self.fit_times_ = {}
         elif solver_cls is SMO:
             hessian = self._smo_hessian(X, ys, 'plain', X_device)
         else:
             hessian = self._build_hessian(X, ys, 'plain', X_device, bias)
-        ub = np.ones(n) * self.C
-        solver = self._make_solver(solver_cls, hessian, -np.ones(n), ub, y)
-        return dict(X=X, y=y, ys=ys, n=n, bias=bias, solver=solver)
+        solver = self._make_solver(solver_cls, hessian, q, ub, eq, active)
+        return dict(X=X, y=y, ys=ys, n=n, bias=bias, solver=solver, rows=rows)
 
     def _finish_fit(self, plan):
         """Everything ``fit`` does after the solver has run (ml/svm/_base.py:725, 867-880)."""
@@ -411,7 +434,7 @@ class SVC(ClassifierMixin, SVM):
         # support set, dual coefficients, intercept (ml/svm/_base.py:867-880)
         sv = self.alphas_ > 1e-6
         self.support_ = np.arange(n)[sv]
-        self._set_support_vectors(X)
+        self._set_support_vectors(X, plan['rows'])
         sv_y, alphas = y[sv], self.alphas_[sv]
         self.dual_coef_ = alphas * sv_y
         if isinstance(self.kernel, LinearKernel):
@@ -460,9 +483,10 @@ class SVR(RegressorMixin, SVM):
         self.fit_times_['solve_s'] = time.perf_counter() - t0
         return self._finish_fit(plan)
 
-    def _plan_fit(self, X, y, X_device=None, shared=None):
+    def _plan_fit(self, X, y, X_device=None, shared=None, rows=None):
         """Everything ``fit`` does before the solver runs.  ``shared``: the resident ``M = K + bias`` of another
-        regression on the same X (multi-target fits, ml/multiclass.py) -- targets only change q."""
+        regression on the same X (multi-target fits, ml/multiclass.py) -- targets only change q.  ``rows``: as for
+        ``SVC._plan_fit``."""
         y = np.asarray(y)
         targets = y.shape[1] if y.ndim > 1 else 1
         if targets > 1:
@@ -481,17 +505,20 @@ class SVR(RegressorMixin, SVM):
         # Q = [[K, -K], [-K, K]] (+ ee', e = [1, -1], when the intercept is regularised)  (ml/svm/_base.py:1098-1100,
         # 1126, 1178): only M = K + bias (n x n) is resident, the solver applies the block signs
         bias = self._bias()
+        ub, q, e, active = np.ones(2 * n) * self.C, np.hstack((-y, y)) + self.epsilon, np.repeat([1.0, -1.0], n), None
         if shared is not None:
+            if rows is not None:
+                m = shared.n
+                (q, ub), active = _embed(2 * m, np.concatenate((rows, rows + m)), q, ub)
+                e = np.repeat([1.0, -1.0], m)
             hessian = shared
             self.fit_times_ = {}
         elif solver_cls is SMO:
             hessian = self._smo_hessian(X, None, 'svr', X_device)
         else:
             hessian = self._build_hessian(X, None, 'svr', X_device, bias)
-        ub = np.ones(2 * n) * self.C
-        e = np.hstack((np.ones(n), -np.ones(n)))
-        solver = self._make_solver(solver_cls, hessian, np.hstack((-y, y)) + self.epsilon, ub, e)
-        return dict(X=X, y=y, n=n, bias=bias, solver=solver)
+        solver = self._make_solver(solver_cls, hessian, q, ub, e, active)
+        return dict(X=X, y=y, n=n, bias=bias, solver=solver, rows=rows)
 
     def _finish_fit(self, plan):
         """Everything ``fit`` does after the solver has run (ml/svm/_base.py:1275-1277, 1423-1437)."""
@@ -504,7 +531,7 @@ class SVR(RegressorMixin, SVM):
         # ml/svm/_base.py:1423-1437
         sv = np.logical_or(alphas_p > 1e-6, alphas_n > 1e-6)
         self.support_ = np.arange(n)[sv]
-        self._set_support_vectors(X)
+        self._set_support_vectors(X, plan['rows'])
         sv_y = y[sv]
         self.dual_coef_ = alphas_p[sv] - alphas_n[sv]
         if isinstance(self.kernel, LinearKernel):

@@ -74,11 +74,16 @@ class SMO(DeviceLoopMixin, Optimizer):
     upper bounds (a scalar or one per variable); ``tol``: stop when the maximal violating pair's gap m - M drops below it.
     After ``minimize``: ``x`` (alpha), ``g_x`` (G = Qx + q), ``f_x`` (= sum x_t (G_t + q_t) / 2), ``iter``, ``status``
     ('optimal' or 'stopped'), ``gap``, ``f_hist`` / ``gap_hist`` (one entry per evaluated state 0 .. iter) and ``rho``
-    (libsvm's; the intercept is -rho)."""
+    (libsvm's; the intercept is -rho).
+
+    ``active`` (one bool per variable, on a shared signed view only): solve the problem on the active variables alone,
+    every other one held at 0 (``svmb200_smo_create_subset``) -- a cross-validation fold on the matrix of a larger set of
+    rows.  ``x``, ``g_x``, ``f_x`` and ``rho`` then describe the active variables only, compacted in index order, and
+    ``f_x`` and ``rho`` come from the compacted arrays, exactly as a solve of the fold's own problem computes them."""
 
     _verbose_header = 'iter\t cost\t\t gap'
 
-    def __init__(self, quad, y, C, tol=1e-3, max_iter=1000, callback=None, callback_args=(), verbose=False):
+    def __init__(self, quad, y, C, tol=1e-3, max_iter=1000, callback=None, callback_args=(), verbose=False, active=None):
         if not isinstance(quad, Quadratic):
             raise TypeError(f'{quad} is not an allowed quadratic function')
         n = quad.ndim
@@ -92,7 +97,11 @@ class SMO(DeviceLoopMixin, Optimizer):
             raise ValueError('tol must be >= 0')
         super(SMO, self).__init__(f=quad, x=np.zeros(n), eps=tol, tol=tol, max_iter=max_iter, callback=callback,
                                   callback_args=callback_args, verbose=verbose)
-        self.y, self.ub = y, C
+        if active is not None:
+            active = np.asarray(active, dtype=bool).ravel()
+            if active.size != n:
+                raise ValueError('active must hold one flag per variable')
+        self.y, self.ub, self.active = y, C, active
         self.gap, self.rho = np.nan, np.nan
         self.row_source, self.cache_slots, self.cache_hits, self.cache_misses = None, 0, 0, 0
 
@@ -100,6 +109,8 @@ class SMO(DeviceLoopMixin, Optimizer):
         H = self.f.device_hessian()
         q, y, ub = (np.ascontiguousarray(v, dtype=np.float64) for v in (self.f.q, self.y, self.ub))
         self.symmetric_pass = False
+        if self.active is not None and (isinstance(H, KernelRowsHessian) or (H.signs is None and H.layout != 'svr')):
+            raise ValueError('an active subset needs a shared resident matrix read as a signed view')
         if isinstance(H, KernelRowsHessian):
             layout = N.HESSIAN_SVR if H.layout == 'svr' else N.HESSIAN_PLAIN
             if not np.array_equal(y, H.row_signs):
@@ -121,8 +132,17 @@ class SMO(DeviceLoopMixin, Optimizer):
                 raise ValueError('on a signed view the sign row y must be the signs of the view')
             symbol = 'svmb200_smo_create_signed'
         h = C.c_void_p()
-        N.call(symbol, H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows, layout,
-               N.ptr(y), N.ptr(q), N.ptr(ub), float(self.tol), int(self.max_iter), C.byref(h))
+        if self.active is not None:
+            # the SVR view reads M with the signs e, which is the plain SVR read (svmb200_smo_create_signed)
+            if H.layout == 'svr' and not np.array_equal(y, np.repeat([1.0, -1.0], H.n)):
+                raise ValueError('on an SVR matrix the sign row y must be e = [1, ..., -1, ...]')
+            active = np.ascontiguousarray(self.active, dtype=np.uint8)
+            N.call('svmb200_smo_create_subset', H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows,
+                   layout, N.ptr(y), N.ptr(q), N.ptr(ub), active.ctypes.data_as(C.c_void_p), float(self.tol),
+                   int(self.max_iter), C.byref(h))
+        else:
+            N.call(symbol, H.ctx.handle, C.c_void_p(H.matrix.dptr), H.n, H.ld, H.row0, H.nrows, layout,
+                   N.ptr(y), N.ptr(q), N.ptr(ub), float(self.tol), int(self.max_iter), C.byref(h))
         self.row_source = 'resident'
         return h, n
 
@@ -139,5 +159,10 @@ class SMO(DeviceLoopMixin, Optimizer):
         f_hist, gap_hist = np.empty(self.iter + 1), np.empty(self.iter + 1)
         N.call('svmb200_pg_history', h, N.ptr(f_hist), N.ptr(gap_hist), C.byref(cnt))
         self.f_hist, self.gap_hist = f_hist[:cnt.value], gap_hist[:cnt.value]
-        self.f_x = float(0.5 * np.dot(self.x, self.g_x + self.f.q))
-        self.rho = calculate_rho(self.x, self.g_x, self.y, self.ub)
+        q, y, ub = self.f.q, self.y, self.ub
+        if self.active is not None:
+            # zeros in a longer vector would change np.dot's rounding, and the held variables would enter rho's ub_set
+            keep = self.active
+            self.x, self.g_x, q, y, ub = self.x[keep], self.g_x[keep], q[keep], y[keep], ub[keep]
+        self.f_x = float(0.5 * np.dot(self.x, self.g_x + q))
+        self.rho = calculate_rho(self.x, self.g_x, y, ub)
