@@ -245,6 +245,15 @@ int64_t svmb200_smo_max_vars(int sm_count);
 /* row source of an SMO solver (computed = 1: svmb200_smo_create_rows), cache slots, hits and misses so far (every row
  * computed without a cache counts as a miss); any output pointer may be NULL */
 int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses);
+/* Shrinking (libsvm's, on by default in libsvm and sklearn) for any SMO solver (all row sources, subsets, batches),
+ * before its first run; SVMB200_ERR_ARG once a run has started.  on = 0 turns it off again.  Variables at a bound that
+ * cannot enter the maximal violating pair are set aside every min(l, 1000) states (l: the variables not held at 0);
+ * their G is rebuilt from q and alpha before the solver stops, so svmb200_pg_state returns the full G.  A run with
+ * shrinking follows its own trajectory (k_smo.cuh documents the rule); it does not depend on the grid or the batch. */
+int svmb200_smo_set_shrinking(svmb200_pg* pg, int on);
+/* active variables after the last shrink check (all variables without shrinking), shrink checks and gradient
+ * reconstructions so far; any output pointer may be NULL */
+int svmb200_smo_shrink_stats(svmb200_pg* pg, int64_t* active, int64_t* checks, int64_t* reconstructions);
 /* dout[r][t] = k(X_{rows[r]}, X_t) for t < n (0 for t in [n, ldo)), unsigned, no bias: the values SMO's computed rows use */
 int svmb200_kernel_rows(svmb200_ctx* ctx, const double* dX, int64_t n, int64_t ldx, int64_t d, int kernel, double gamma,
                         double coef0, double degree, const int64_t* rows_host, int64_t nrows, double* dout, int64_t ldo);

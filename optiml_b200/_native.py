@@ -75,6 +75,8 @@ PROTOTYPES = {
     'svmb200_smo_create_rows': [c_vp, c_vp, i64, i64, i64, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, c_vp,
                                 c_vp, c_vp, C.c_double, i64, C.c_size_t, C.POINTER(c_vp)],
     'svmb200_smo_cache_stats': [c_vp, C.POINTER(C.c_int), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)],
+    'svmb200_smo_set_shrinking': [c_vp, C.c_int],
+    'svmb200_smo_shrink_stats': [c_vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)],
     'svmb200_kernel_rows': [c_vp, c_vp, i64, i64, i64, C.c_int, C.c_double, C.c_double, C.c_double, c_vp, i64, c_vp, i64],
     'svmb200_pg_run_batch': [C.POINTER(c_vp), C.c_int, C.POINTER(i64), C.POINTER(C.c_int)],
     'svmb200_matvec_multi': [c_vp, c_vp, i64, i64, C.POINTER(c_vp), C.POINTER(c_vp), C.c_int],

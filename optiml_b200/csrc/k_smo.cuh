@@ -53,6 +53,26 @@
 // CTA's index and grid size inside its problem instead of blockIdx.x / gridDim.x.  A solve does not depend on its grid
 // (total-order reductions), so every problem follows the same bits whatever grid it is given, launch after launch.  The
 // computed form stays single-problem: its per-CTA cache tags assume one problem owns the CTA's slice.
+//
+// Shrinking (libsvm's do_shrinking / be_shrunk / reconstruct_gradient; the SHRINK instantiations smo_shrink_kernel and
+// smo_batch_shrink_kernel, the plain kernels are the SHRINK = false ones).  One active flag per variable (a bit per owned
+// variable in shared memory, a byte per variable in HBM between launches: K14 changes slices between launches); held
+// variables (ub = 0) are never active.  Selection, step and G update run over the active variables only: an inactive
+// variable's G is not updated and its row entries are neither read nor computed.  l = the non-held variables, P = min(l,
+// 1000); a counter that starts at P + 1 is decremented before the selection of every state, and at 0 (set back to P) the
+// state is a shrink check:
+//   phase 1 also carries the slice's min over the active I_low in `mlow`; after the barrier every CTA knows m and M;
+//   the first time m - M <= 10 tol the solver reconstructs and reactivates everything (`unshrunk`);
+//   every CTA deactivates its own variables at a bound that are only in I_low with -y_t G_t > m, or only in I_up with
+//   -y_t G_t < M (free variables never), publishes a fresh i candidate (in the i slots of the other parity, free until
+//   phase 1 of state k + 1) and its active count, and one more grid barrier follows.
+// When the stopping test fires with inactive variables the solver reconstructs, reactivates everything, sets the counter
+// to 1 and selects again at the same state (the history of state k is the evaluation that decided it); a max_iter stop
+// reconstructs before G is written back.  Reconstruct: every CTA writes its alpha to HBM, grid barrier, then
+// G_t = q_t + sum_{j ascending, alpha_j > 0} Q_jt alpha_j (one rounding per product and per sum) for its inactive, non-held
+// t, with Q_jt read from row j (resident, signed) or computed by kfn_value; a computed-row CTA then clears its copy of the
+// cache tags, so no cached row holds an entry skipped while its variable was inactive.  Every decision that adds a barrier
+// (counter, m, M, gap, status, the grid's active count) is grid-uniform.  SmoShrink::on = 0 follows the plain bits.
 #pragma once
 #include "k_persistent.cuh"   // pk_grid_barrier
 #include "kernel_fn.cuh"      // kfn_value
@@ -62,6 +82,8 @@ constexpr int SMO_ARRAYS = 6;        // doubles of shared memory per owned varia
 constexpr double SMO_TAU = 1e-12;
 constexpr int SMO_ROWS_RESIDENT = 0, SMO_ROWS_COMPUTED = 1, SMO_ROWS_SIGNED = 2;
 constexpr int SMO_CACHE_WAYS = 8;
+constexpr int SMO_ACT_WORDS = 148;   // shrinking: one bit per owned variable (pg.cu asserts the largest slice fits)
+constexpr long long SMO_SHRINK_EVERY = 1000;
 
 struct SmoCand {      // the winner of one CTA's slice (64 bytes)
     double key;       // i pass: -y_t G_t;  j pass: b_t^2 / a_t  (the larger wins, ties to the larger index)
@@ -94,6 +116,25 @@ struct SmoArgs {
     long long* stamps;      // [grid][slots] stamp of the last use
     long long sets, ways;
     unsigned long long* stats;  // hits, misses (CTA 0)
+};
+
+// shrinking: the grid-uniform state carried across launches (every CTA reads it at the start, CTA 0 writes it at the end)
+struct SmoShrinkState {
+    long long counter;          // decremented before the selection of every state: a check at 0
+    long long unshrunk;         // the gap came within 10 tol once and everything was reactivated
+    long long shrunk;           // some non-held variable is inactive
+    long long prepared;         // the last state whose counter step ran: a launch that ends on its budget evaluates
+                                // its last state, and the next launch evaluates it again without a second step
+    long long checks, reconstructions;
+    long long active;           // active variables after the last check
+};
+
+struct SmoShrink {
+    const double* q;            // linear term (nvars): G of an inactive variable is rebuilt from it
+    unsigned char* act;         // active flags (nvars): read at the start of a launch, written back at its end
+    SmoShrinkState* st;
+    long long l;                // variables that are not held (ub > 0)
+    int on;                     // 0: no shrinking, the plain kernel's trajectory
 };
 
 // Q[s][t] as read from row s
@@ -223,9 +264,88 @@ __device__ __forceinline__ void smo_grid_reduce(const SmoCand* slots, unsigned g
     __syncthreads();
 }
 
-// the solve of one problem by CTA `cta` of the `grid` CTAs that run it
+__device__ __forceinline__ bool smo_is_active(const unsigned* act, int l) { return (act[l >> 5] >> (l & 31)) & 1u; }
+
+// block-wide sum of v (exact for counts); the result is returned to every thread
+__device__ __forceinline__ double smo_block_sum(double v, double (*red)[SMO_NT / 32]) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    __syncthreads();   // red may still be read by the previous reduction
+    if ((threadIdx.x & 31) == 0) red[0][threadIdx.x >> 5] = v;
+    __syncthreads();
+    double sum = 0.0;
+    for (int w = 0; w < SMO_NT / 32; ++w) sum += red[0][w];
+    __syncthreads();
+    return sum;
+}
+
+// shrinking: G_t = q_t + sum_{j ascending, alpha_j > 0} Q_jt alpha_j for the slice's inactive, non-held variables, which
+// then become active (with every other non-held one).  Every CTA calls it (it holds a grid barrier).
 template <int ROWS>
-__device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, const unsigned grid) {
+__device__ __forceinline__ void smo_reconstruct(const SmoArgs& a, const SmoShrink& s, const unsigned cta, const unsigned grid,
+                                                const long long t0, const int len, unsigned* act, const double* s_alpha,
+                                                double* s_g, const double* s_y, const double* s_c) {
+    __shared__ double s_ya[SMO_NT];   // y_j alpha_j of one chunk of j (alpha_j >= 0: the sign is y_j where alpha_j > 0)
+    const int tid = threadIdx.x, nwords = (len + 31) >> 5;
+    for (int l = tid; l < len; l += SMO_NT) a.x[t0 + l] = s_alpha[l];
+    pk_grid_barrier(a.gbar, grid);
+    bool mine = false;   // this thread owns a variable to rebuild
+    for (int l = tid; l < len; l += SMO_NT) {
+        if (!smo_is_active(act, l) && s_c[l] > 0.0) {
+            s_g[l] = __ldg(s.q + t0 + l);
+            mine = true;
+        }
+    }
+    for (long long j0 = 0; j0 < a.nvars; j0 += SMO_NT) {
+        __syncthreads();
+        const long long jt = j0 + tid;
+        s_ya[tid] = jt < a.nvars ? __dmul_rn(__ldg(a.sgn + jt), __ldcg(a.x + jt)) : 0.0;
+        __syncthreads();
+        if (!mine) continue;
+        const int cnt = a.nvars - j0 < SMO_NT ? (int)(a.nvars - j0) : SMO_NT;
+        for (int b = 0; b < cnt; ++b) {
+            const double v = s_ya[b];
+            if (v == 0.0) continue;
+            const long long j = j0 + b;
+            const double aj = fabs(v), yj = v > 0.0 ? 1.0 : -1.0;
+            for (int l = tid; l < len; l += SMO_NT) {
+                if (smo_is_active(act, l) || !(s_c[l] > 0.0)) continue;
+                const long long t = t0 + l;
+                double qjt;
+                if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+                    const double w = kfn_value(a.kf, j < a.n ? j : j - a.n, t < a.n ? t : t - a.n);
+                    qjt = yj == s_y[l] ? w : -w;
+                } else if constexpr (ROWS == SMO_ROWS_SIGNED) {
+                    qjt = smo_q_signed(a, j, t, yj, s_y[l]);
+                } else {
+                    qjt = smo_q(a, j, t);
+                }
+                s_g[l] = __dadd_rn(s_g[l], __dmul_rn(qjt, aj));
+            }
+        }
+    }
+    __syncthreads();
+    for (int w = tid; w < nwords; w += SMO_NT) {
+        unsigned bits = 0u;
+        for (int b = 0; b < 32 && 32 * w + b < len; ++b)
+            if (s_c[32 * w + b] > 0.0) bits |= 1u << b;
+        act[w] = bits;
+    }
+    if constexpr (ROWS == SMO_ROWS_COMPUTED) {
+        // the CTA's copy of the tags, cleared identically everywhere: a cached row may lack the entries of variables
+        // that were inactive when it was computed
+        const long long slots = a.sets * a.ways;
+        for (long long r = tid; r < slots; r += SMO_NT) {
+            a.tags[(size_t)cta * slots + r] = -1;
+            a.stamps[(size_t)cta * slots + r] = -1;
+        }
+    }
+    __syncthreads();
+}
+
+// the solve of one problem by CTA `cta` of the `grid` CTAs that run it; SHRINK: with shrinking when s.on
+template <int ROWS, bool SHRINK>
+__device__ __forceinline__ void smo_solve(const SmoArgs& a, const SmoShrink& s, const unsigned cta, const unsigned grid) {
 #ifndef SVMB200_HOST_EMULATION
     extern __shared__ __align__(16) unsigned char smo_smem_raw[];
     double* sm = reinterpret_cast<double*>(smo_smem_raw);
@@ -259,6 +379,27 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
         s_qi[l] = 0.0;
     }
     double f = a.st->f;   // objective at state k0 (CTA 0 rewrites it only after the first grid barrier)
+    // shrinking: the slice's active flags and the grid-uniform state (identical in every CTA)
+    __shared__ unsigned s_act[SHRINK ? SMO_ACT_WORDS : 1];
+    long long counter = 0, checks = 0, recons = 0, nact = 0, prepared = -1;
+    bool unshrunk = false, shrunk = false, reselect = false;
+    if constexpr (SHRINK) {
+        for (int w = tid; w < (len + 31) >> 5; w += SMO_NT) {
+            unsigned bits = 0u;
+            for (int b = 0; b < 32 && 32 * w + b < len; ++b)
+                if (!s.on || s.act[t0 + 32 * w + b]) bits |= 1u << b;
+            s_act[w] = bits;
+        }
+        if (s.on) {
+            counter = s.st->counter;
+            unshrunk = s.st->unshrunk != 0;
+            shrunk = s.st->shrunk != 0;
+            prepared = s.st->prepared;
+            checks = s.st->checks;
+            recons = s.st->reconstructions;
+            nact = s.st->active;
+        }
+    }
     __syncthreads();
 
     bool pending = false;          // a step whose G update phase 1 still has to apply
@@ -268,9 +409,21 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
         const long long k = a.k0 + e;
         SmoCand* slots_i = a.cand + (size_t)((k & 1) * 2) * grid;
         SmoCand* slots_j = slots_i + grid;
+        bool check = false;   // shrinking: this state is a shrink check
+        if constexpr (SHRINK) {
+            if (s.on && !reselect && k != prepared && --counter == 0) {
+                counter = s.l < SMO_SHRINK_EVERY ? s.l : SMO_SHRINK_EVERY;
+                check = true;
+            }
+            prepared = k;
+            reselect = false;
+        }
         // ================= phase 1: previous step on the own G, local candidate for i
         double key = -INFINITY, idx = -1.0, low = INFINITY;
         for (int l = tid; l < len; l += SMO_NT) {
+            if constexpr (SHRINK) {
+                if (!smo_is_active(s_act, l)) continue;
+            }
             const long long t = t0 + l;
             double gt = s_g[l];
             if (pending) {
@@ -293,10 +446,13 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
                 key = v;
                 idx = (double)t;
             }
+            if constexpr (SHRINK) {
+                if (check && (y > 0.0 ? al > 0.0 : al < s_c[l])) low = fmin(low, v);
+            }
         }
         smo_block_reduce(key, idx, low, red);
         if (tid == 0) {
-            SmoCand c = {key, idx, 0.0, 0.0, 0.0, 0.0, 0.0, INFINITY};
+            SmoCand c = {key, idx, 0.0, 0.0, 0.0, 0.0, 0.0, SHRINK ? low : INFINITY};
             if (idx >= 0.0) {
                 const int l = (int)((long long)idx - t0);
                 c.alpha = s_alpha[l];
@@ -309,8 +465,70 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
         }
         pk_grid_barrier(a.gbar, grid);
 
+        const SmoCand* src_i = slots_i;
+        if constexpr (SHRINK) {
+            if (check) {   // ================= shrink check
+                smo_grid_reduce(slots_i, grid, S, red, &win_i);
+                const double cm = win_i.key, cM = win_i.mlow;
+                ++checks;
+                if (!unshrunk && __dsub_rn(cm, cM) <= __dmul_rn(10.0, a.tol)) {
+                    unshrunk = true;
+                    smo_reconstruct<ROWS>(a, s, cta, grid, t0, len, s_act, s_alpha, s_g, s_y, s_c);
+                    ++recons;
+                }
+                double cnt = 0.0;
+                for (int w = tid; w < (len + 31) >> 5; w += SMO_NT) {
+                    unsigned bits = s_act[w];
+                    for (int b = 0; b < 32 && 32 * w + b < len; ++b) {
+                        if (!((bits >> b) & 1u)) continue;
+                        const int l = 32 * w + b;
+                        const double y = s_y[l], al = s_alpha[l], c = s_c[l];
+                        const bool up = y > 0.0 ? al < c : al > 0.0, lo = y > 0.0 ? al > 0.0 : al < c;
+                        const double v = -__dmul_rn(y, s_g[l]);
+                        if ((lo && !up && v > cm) || (up && !lo && v < cM)) bits &= ~(1u << b);
+                        else cnt += 1.0;
+                    }
+                    s_act[w] = bits;
+                }
+                cnt = smo_block_sum(cnt, red);   // (its barriers also publish s_act)
+                key = -INFINITY;
+                idx = -1.0;
+                low = INFINITY;
+                for (int l = tid; l < len; l += SMO_NT) {
+                    if (!smo_is_active(s_act, l)) continue;
+                    const double y = s_y[l], al = s_alpha[l];
+                    const bool up = y > 0.0 ? al < s_c[l] : al > 0.0;
+                    const double v = -__dmul_rn(y, s_g[l]);
+                    if (up && v >= key) {
+                        key = v;
+                        idx = (double)(t0 + l);
+                    }
+                }
+                smo_block_reduce(key, idx, low, red);
+                SmoCand* fresh = a.cand + (size_t)(((k + 1) & 1) * 2) * grid;
+                if (tid == 0) {
+                    SmoCand c = {key, idx, 0.0, 0.0, 0.0, 0.0, 0.0, cnt};   // mlow carries the slice's active count
+                    if (idx >= 0.0) {
+                        const int l = (int)((long long)idx - t0);
+                        c.alpha = s_alpha[l];
+                        c.g = s_g[l];
+                        c.y = s_y[l];
+                        c.qd = s_qd[l];
+                        c.c = s_c[l];
+                    }
+                    fresh[cta] = c;
+                }
+                pk_grid_barrier(a.gbar, grid);
+                double total = 0.0;
+                for (unsigned b = 0; b < grid; ++b) total += __ldcg(&fresh[b].mlow);
+                nact = (long long)total;
+                shrunk = nact < s.l;
+                src_i = fresh;
+            }
+        }
+
         // ================= phase 2: i and m; own part of row i; local candidate for j, local M
-        smo_grid_reduce(slots_i, grid, S, red, &win_i);
+        smo_grid_reduce(src_i, grid, S, red, &win_i);
         const double m = win_i.key, yi = win_i.y, qii = win_i.qd;
         const long long i = (long long)win_i.idx;
         if constexpr (ROWS == SMO_ROWS_COMPUTED) {
@@ -321,6 +539,9 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
         idx = -1.0;
         low = INFINITY;
         for (int l = tid; l < len; l += SMO_NT) {
+            if constexpr (SHRINK) {
+                if (!smo_is_active(s_act, l)) continue;
+            }
             const long long t = t0 + l;
             double qit = 0.0;
             if constexpr (ROWS == SMO_ROWS_COMPUTED) {
@@ -384,6 +605,20 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
         if (j < 0 || gap < a.tol) stop = SVMB200_STATUS_OPTIMAL;
         else if (k >= a.max_iter) stop = SVMB200_STATUS_STOPPED;
         if (stop) {
+            if constexpr (SHRINK) {
+                if (shrunk) {   // the full problem decides: rebuild G, reactivate everything
+                    smo_reconstruct<ROWS>(a, s, cta, grid, t0, len, s_act, s_alpha, s_g, s_y, s_c);
+                    ++recons;
+                    shrunk = false;
+                    if (stop == SVMB200_STATUS_OPTIMAL) {   // select again at the same state, check at the next
+                        counter = 1;
+                        reselect = true;
+                        pending = false;
+                        --e;
+                        continue;
+                    }
+                }
+            }
             if (cta == 0 && tid == 0) {
                 a.st->status = stop;
                 __threadfence();
@@ -458,17 +693,43 @@ __device__ __forceinline__ void smo_solve(const SmoArgs& a, const unsigned cta, 
         a.x[t0 + l] = s_alpha[l];
         a.g[t0 + l] = s_g[l];
     }
+    if constexpr (SHRINK) {
+        if (s.on) {
+            for (int l = tid; l < len; l += SMO_NT) s.act[t0 + l] = smo_is_active(s_act, l) ? 1 : 0;
+            if (cta == 0 && tid == 0) {
+                s.st->counter = counter;
+                s.st->unshrunk = unshrunk;
+                s.st->shrunk = shrunk;
+                s.st->prepared = prepared;
+                s.st->checks = checks;
+                s.st->reconstructions = recons;
+                s.st->active = nact;
+            }
+        }
+    }
 }
 
 template <int ROWS>
 __global__ void __launch_bounds__(SMO_NT, 1) smo_persistent_kernel(const SmoArgs a) {
-    smo_solve<ROWS>(a, blockIdx.x, gridDim.x);
+    smo_solve<ROWS, false>(a, SmoShrink{}, blockIdx.x, gridDim.x);
+}
+
+// the solver's arguments and its shrinking state (one launch argument)
+struct SmoShrinkArgs {
+    SmoArgs a;
+    SmoShrink s;
+};
+
+template <int ROWS>
+__global__ void __launch_bounds__(SMO_NT, 1) smo_shrink_kernel(const SmoShrinkArgs p) {
+    smo_solve<ROWS, true>(p.a, p.s, blockIdx.x, gridDim.x);
 }
 
 // K14: one problem of a batch -- its arguments and its CTAs [cta0, cta0 + grid) of the launch
 struct SmoBatchProblem {
     SmoArgs a;
     int cta0, grid;
+    SmoShrink s;      // smo_batch_shrink_kernel only (s.on = 0: the problem does not shrink)
 };
 
 struct SmoBatchArgs {
@@ -476,17 +737,30 @@ struct SmoBatchArgs {
     int count;
 };
 
-template <int ROWS>
-__global__ void __launch_bounds__(SMO_NT, 1) smo_batch_kernel(const SmoBatchArgs b) {
+template <int ROWS, bool SHRINK>
+__device__ __forceinline__ void smo_batch(const SmoBatchArgs& b) {
     __shared__ SmoArgs pa;   // the problem's arguments, read once per launch
+    __shared__ SmoShrink ps;
     __shared__ unsigned p_cta, p_grid;
     if (threadIdx.x == 0) {
         int p = 0;
         while (p + 1 < b.count && (int)blockIdx.x >= b.probs[p + 1].cta0) ++p;
         pa = b.probs[p].a;
+        if constexpr (SHRINK) ps = b.probs[p].s;
         p_cta = blockIdx.x - (unsigned)b.probs[p].cta0;
         p_grid = (unsigned)b.probs[p].grid;
     }
     __syncthreads();
-    smo_solve<ROWS>(pa, p_cta, p_grid);
+    smo_solve<ROWS, SHRINK>(pa, ps, p_cta, p_grid);
+}
+
+template <int ROWS>
+__global__ void __launch_bounds__(SMO_NT, 1) smo_batch_kernel(const SmoBatchArgs b) {
+    smo_batch<ROWS, false>(b);
+}
+
+// K14 with shrinking: each problem's SmoShrink::on says whether it shrinks
+template <int ROWS>
+__global__ void __launch_bounds__(SMO_NT, 1) smo_batch_shrink_kernel(const SmoBatchArgs b) {
+    smo_batch<ROWS, true>(b);
 }

@@ -590,6 +590,8 @@ struct SmoSolver {
     int grid = 0;
     int rows = SMO_ROWS_RESIDENT;   // SMO_ROWS_RESIDENT, _SIGNED (svmb200_smo_create_signed) or _COMPUTED
     void* rows_buf = nullptr;  // |x|^2 | Q_ij slots | tags | stamps | stats | cache
+    SmoShrink shrink = {};     // shrinking (svmb200_smo_set_shrinking): on, and its buffer at shrink.q
+    bool started = false;      // a run has started
 };
 
 struct svmb200_pg {
@@ -786,6 +788,7 @@ extern "C" int svmb200_pg_destroy(svmb200_pg* pg) {
         cudaStreamSynchronize(pg->ctx->stream);
         if (pg->solver == SOLVER_SMO && pg->hist_f) cudaFree(pg->hist_f);
         if (pg->smo.rows_buf) cudaFree(pg->smo.rows_buf);
+        if (pg->smo.shrink.q) cudaFree(const_cast<double*>(pg->smo.shrink.q));
         if (pg->slab_private) {
             if (pg->slab) cudaFree(pg->slab);
             if (pg->pinned) cudaFreeHost(pg->pinned);
@@ -1789,6 +1792,7 @@ extern "C" int svmb200_al_multipliers(svmb200_pg* pg, double* mu, double* lam_lb
 constexpr int64_t SMO_CHUNK = 65536;
 constexpr int64_t SMO_MIN_SLICE = 128;
 constexpr int64_t SMO_SLICE_MAX = (int64_t)(COOP_SMEM_MAX / (SMO_ARRAYS * sizeof(double)));
+static_assert(SMO_SLICE_MAX <= 32 * SMO_ACT_WORDS, "the shrinking flags of a slice do not fit SMO_ACT_WORDS");
 
 static size_t smo_smem_bytes(const svmb200_pg* pg) { return (size_t)pg->smo.a.slice * SMO_ARRAYS * sizeof(double); }
 
@@ -1811,6 +1815,19 @@ static int smo_setup(svmb200_ctx* ctx, int rows, int grid, size_t smem, bool* fi
     return rows == SMO_ROWS_COMPUTED ? cooperative_setup<smo_persistent_kernel<SMO_ROWS_COMPUTED>>(ctx, grid, SMO_NT, smem, fits)
          : rows == SMO_ROWS_SIGNED   ? cooperative_setup<smo_persistent_kernel<SMO_ROWS_SIGNED>>(ctx, grid, SMO_NT, smem, fits)
                                      : cooperative_setup<smo_persistent_kernel<SMO_ROWS_RESIDENT>>(ctx, grid, SMO_NT, smem, fits);
+}
+
+// the same with shrinking
+static void (*smo_shrink_kernel_of(int rows))(SmoShrinkArgs) {
+    return rows == SMO_ROWS_COMPUTED ? smo_shrink_kernel<SMO_ROWS_COMPUTED>
+         : rows == SMO_ROWS_SIGNED   ? smo_shrink_kernel<SMO_ROWS_SIGNED>
+                                     : smo_shrink_kernel<SMO_ROWS_RESIDENT>;
+}
+
+static int smo_shrink_setup(svmb200_ctx* ctx, int rows, int grid, size_t smem, bool* fits) {
+    return rows == SMO_ROWS_COMPUTED ? cooperative_setup<smo_shrink_kernel<SMO_ROWS_COMPUTED>>(ctx, grid, SMO_NT, smem, fits)
+         : rows == SMO_ROWS_SIGNED   ? cooperative_setup<smo_shrink_kernel<SMO_ROWS_SIGNED>>(ctx, grid, SMO_NT, smem, fits)
+                                     : cooperative_setup<smo_shrink_kernel<SMO_ROWS_RESIDENT>>(ctx, grid, SMO_NT, smem, fits);
 }
 
 // rows: the computed form (K12), else null; signed_view: dQ is an unsigned M read with the signs (SMO_ROWS_SIGNED);
@@ -2008,6 +2025,69 @@ extern "C" int svmb200_smo_create_rows(svmb200_ctx* ctx, const double* dX, int64
     return smo_create(ctx, nullptr, n, 0, hessian, sign_host, q_host, ub_host, tol, max_iter, &rows, false, nullptr, out);
 }
 
+// Shrinking: q (nvars), the state, the active flags (nvars bytes) in one allocation at shrink.q.  Flags start set for
+// every variable that is not held (ub > 0); the counter at min(l, 1000) + 1 puts the first check at state min(l, 1000).
+extern "C" int svmb200_smo_set_shrinking(svmb200_pg* pg, int on) {
+    SVM_CHECK_ARG(pg != nullptr && pg->solver == SOLVER_SMO, "not an SMO solver");
+    SVM_CHECK_ARG(!pg->smo.started, "svmb200_smo_set_shrinking: the solver has already run");
+    SVM_TRY(svm_use(pg->ctx));
+    SmoShrink& sh = pg->smo.shrink;
+    if (!on) {
+        if (sh.q) SVM_CUDA(cudaFree(const_cast<double*>(sh.q)));
+        sh = {};
+        return SVMB200_OK;
+    }
+    if (sh.on) return SVMB200_OK;
+    bool fits = false;
+    SVM_TRY(smo_shrink_setup(pg->ctx, pg->smo.rows, pg->smo.grid, smo_smem_bytes(pg), &fits));
+    if (!fits) {
+        svmb200_set_error("SMO: %d CTAs of %zu bytes of shared memory cannot be co-resident", pg->smo.grid, smo_smem_bytes(pg));
+        return SVMB200_ERR_ARG;
+    }
+    const size_t nv = (size_t)pg->nvars * sizeof(double);
+    std::vector<double> ub((size_t)pg->nvars);
+    std::vector<unsigned char> act((size_t)pg->nvars);
+    cudaStream_t s = pg->ctx->stream;
+    SVM_CUDA(cudaMemcpyAsync(ub.data(), pg->ub, nv, cudaMemcpyDeviceToHost, s));
+    SVM_CUDA(cudaStreamSynchronize(s));
+    long long l = 0;
+    for (size_t t = 0; t < act.size(); ++t) l += act[t] = ub[t] > 0.0;
+    SmoShrinkState st = {};
+    st.counter = (l < SMO_SHRINK_EVERY ? l : SMO_SHRINK_EVERY) + 1;
+    st.active = l;
+    st.prepared = -1;
+    const size_t st_off = nv, act_off = st_off + ((sizeof(SmoShrinkState) + 255) & ~size_t(255));
+    unsigned char* buf = nullptr;
+    SVM_CUDA(cudaMalloc(&buf, act_off + (size_t)pg->nvars));
+    sh.q = reinterpret_cast<double*>(buf);
+    sh.st = reinterpret_cast<SmoShrinkState*>(buf + st_off);
+    sh.act = buf + act_off;
+    sh.l = l;
+    sh.on = 1;
+    // before the first run G = q
+    SVM_CUDA(cudaMemcpyAsync(buf, pg->g, nv, cudaMemcpyDeviceToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(sh.st, &st, sizeof(st), cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaMemcpyAsync(sh.act, act.data(), act.size(), cudaMemcpyHostToDevice, s));
+    SVM_CUDA(cudaStreamSynchronize(s));
+    return SVMB200_OK;
+}
+
+extern "C" int svmb200_smo_shrink_stats(svmb200_pg* pg, int64_t* active, int64_t* checks, int64_t* reconstructions) {
+    SVM_CHECK_ARG(pg != nullptr && pg->solver == SOLVER_SMO, "not an SMO solver");
+    SVM_TRY(svm_use(pg->ctx));
+    SmoShrinkState st = {};
+    if (pg->smo.shrink.on) {
+        SVM_CUDA(cudaMemcpyAsync(&st, pg->smo.shrink.st, sizeof(st), cudaMemcpyDeviceToHost, pg->ctx->stream));
+        SVM_CUDA(cudaStreamSynchronize(pg->ctx->stream));
+    } else {
+        st.active = pg->nvars;
+    }
+    if (active) *active = st.active;
+    if (checks) *checks = st.checks;
+    if (reconstructions) *reconstructions = st.reconstructions;
+    return SVMB200_OK;
+}
+
 extern "C" int svmb200_smo_cache_stats(svmb200_pg* pg, int* computed, int64_t* slots, int64_t* hits, int64_t* misses) {
     SVM_CHECK_ARG(pg != nullptr && pg->solver == SOLVER_SMO, "not an SMO solver");
     SVM_TRY(svm_use(pg->ctx));
@@ -2054,8 +2134,12 @@ static int smo_launch(svmb200_pg* pg, int64_t niter) {
     a.hist_cap = pg->hist_cap;
     a.k0 = pg->k_next;
     a.niter = niter;
-    SVM_CUDA(svm_launch_cooperative(smo_kernel(pg->smo.rows), dim3((unsigned)pg->smo.grid), dim3(SMO_NT), smo_smem_bytes(pg),
-                                    pg->ctx->stream, a));
+    if (pg->smo.shrink.on)
+        SVM_CUDA(svm_launch_cooperative(smo_shrink_kernel_of(pg->smo.rows), dim3((unsigned)pg->smo.grid), dim3(SMO_NT),
+                                        smo_smem_bytes(pg), pg->ctx->stream, SmoShrinkArgs{a, pg->smo.shrink}));
+    else
+        SVM_CUDA(svm_launch_cooperative(smo_kernel(pg->smo.rows), dim3((unsigned)pg->smo.grid), dim3(SMO_NT), smo_smem_bytes(pg),
+                                        pg->ctx->stream, a));
     pg->ctx->launches++;
     return SVMB200_OK;
 }
@@ -2064,6 +2148,7 @@ static int smo_run(svmb200_pg* pg, int64_t max_new) {
     svmb200_ctx* ctx = pg->ctx;
     SVM_TRY(svm_use(ctx));
     reset_run_stats(pg);   // last_passes stays 0: an iteration reads two rows, never a full pass over Q
+    pg->smo.started = true;
     SVM_CUDA(cudaEventRecord(pg->ev0, ctx->stream));
     if (!pg->finished) {
         int64_t budget = pg->max_iter - pg->k_next;
@@ -2139,7 +2224,12 @@ extern "C" int svmb200_smo_run_batch(svmb200_pg* const* pgs, int count, int64_t*
     SmoBatchProblem* dprobs = static_cast<SmoBatchProblem*>(ctx->batch_buf);
     unsigned* bars = reinterpret_cast<unsigned*>(static_cast<unsigned char*>(ctx->batch_buf) + probs_bytes);
     SVM_CUDA(cudaMemsetAsync(bars, 0, (size_t)slots * 256, ctx->stream));
-    for (int b = 0; b < count; ++b) reset_run_stats(pgs[b]);
+    bool shrink = false;   // one problem shrinks: the launches take smo_batch_shrink_kernel (a flag per problem)
+    for (int b = 0; b < count; ++b) {
+        reset_run_stats(pgs[b]);
+        pgs[b]->smo.started = true;
+        shrink = shrink || pgs[b]->smo.shrink.on;
+    }
     SVM_CUDA(cudaEventRecord(p0->ev0, ctx->stream));
     std::vector<SmoBatchProblem> hp((size_t)slots);
     std::vector<int> admitted((size_t)slots);
@@ -2169,6 +2259,7 @@ extern "C" int svmb200_smo_run_batch(svmb200_pg* const* pgs, int count, int64_t*
             p.a.hist_cap = pg->hist_cap;
             p.a.k0 = pg->k_next;
             p.a.niter = nb[r];
+            p.s = pg->smo.shrink;
             p.cta0 = cta0;
             p.grid = (int)((nvars + slice - 1) / slice);
             cta0 += p.grid;
@@ -2176,8 +2267,12 @@ extern "C" int svmb200_smo_run_batch(svmb200_pg* const* pgs, int count, int64_t*
         }
         bool fits = false;
         const bool sgn = p0->smo.rows == SMO_ROWS_SIGNED;
-        SVM_TRY(sgn ? cooperative_setup<smo_batch_kernel<SMO_ROWS_SIGNED>>(ctx, cta0, SMO_NT, smem, &fits)
-                    : cooperative_setup<smo_batch_kernel<SMO_ROWS_RESIDENT>>(ctx, cta0, SMO_NT, smem, &fits));
+        void (*kernel)(SmoBatchArgs) = shrink ? (sgn ? smo_batch_shrink_kernel<SMO_ROWS_SIGNED> : smo_batch_shrink_kernel<SMO_ROWS_RESIDENT>)
+                                              : (sgn ? smo_batch_kernel<SMO_ROWS_SIGNED> : smo_batch_kernel<SMO_ROWS_RESIDENT>);
+        SVM_TRY(shrink ? (sgn ? cooperative_setup<smo_batch_shrink_kernel<SMO_ROWS_SIGNED>>(ctx, cta0, SMO_NT, smem, &fits)
+                              : cooperative_setup<smo_batch_shrink_kernel<SMO_ROWS_RESIDENT>>(ctx, cta0, SMO_NT, smem, &fits))
+                       : (sgn ? cooperative_setup<smo_batch_kernel<SMO_ROWS_SIGNED>>(ctx, cta0, SMO_NT, smem, &fits)
+                              : cooperative_setup<smo_batch_kernel<SMO_ROWS_RESIDENT>>(ctx, cta0, SMO_NT, smem, &fits)));
         if (!fits) {
             svmb200_set_error("SMO batch: %d CTAs of %zu bytes of shared memory cannot be co-resident", cta0, smem);
             return SVMB200_ERR_STATE;
@@ -2186,8 +2281,7 @@ extern "C" int svmb200_smo_run_batch(svmb200_pg* const* pgs, int count, int64_t*
         SmoBatchArgs ba;
         ba.probs = dprobs;
         ba.count = k;
-        SVM_CUDA(svm_launch_cooperative(sgn ? smo_batch_kernel<SMO_ROWS_SIGNED> : smo_batch_kernel<SMO_ROWS_RESIDENT>,
-                                        dim3((unsigned)cta0), dim3(SMO_NT), smem, ctx->stream, ba));
+        SVM_CUDA(svm_launch_cooperative(kernel, dim3((unsigned)cta0), dim3(SMO_NT), smem, ctx->stream, ba));
         ctx->launches++;
         for (int r = 0; r < k; ++r) {
             svmb200_pg* pg = pgs[admitted[r]];

@@ -147,7 +147,7 @@ def _smo_batch_capable(estimator):
         return False
     try:
         return estimator._bcqp_solver_class() is SMO
-    except (NotImplementedError, TypeError):
+    except (NotImplementedError, TypeError, ValueError):   # (ValueError: shrinking without SMO, refused at fit)
         return False
 
 
@@ -163,7 +163,7 @@ def _lockstep_capable(estimator, n_samples=None):
             return False
     try:
         solver_cls = estimator._bcqp_solver_class()
-    except (NotImplementedError, TypeError):
+    except (NotImplementedError, TypeError, ValueError):   # (ValueError: shrinking without SMO, refused at fit)
         return False
     return solver_cls is not SMO   # SMO batches are not lockstep ones: _smo_batch_capable
 

@@ -68,7 +68,7 @@ class SVM(BaseEstimator):
                  reg_intercept=False, dual=False, optimizer=None, master_solver='clarabel', learning_rate='auto',
                  momentum_type='none', momentum=0.9, max_iter=1000, max_f_eval=15000, tol=1e-4, batch_size=None,
                  shuffle=True, random_state=None, early_stopping=False, validation_split=0., patience=5,
-                 verbose=False, master_verbose=False):
+                 verbose=False, master_verbose=False, shrinking=False):
         self.loss = loss
         if not isinstance(kernel, Kernel):
             raise TypeError(f'{kernel} is not an allowed kernel function')
@@ -113,6 +113,7 @@ class SVM(BaseEstimator):
         self.patience = patience
         self.verbose = verbose
         self.master_verbose = master_verbose
+        self.shrinking = shrinking   # libsvm's shrinking heuristic (optimizer='smo' only; checked at fit)
         if not self.dual or isinstance(self.kernel, LinearKernel):
             self.coef_ = np.zeros(0)
         self.intercept_ = 0.
@@ -127,6 +128,12 @@ class SVM(BaseEstimator):
 
     # ------------------------------------------------------------------ shared pieces of fit
     def _bcqp_solver_class(self):
+        solver_cls = self._bcqp_solver_class_of_optimizer()
+        if getattr(self, 'shrinking', False) and solver_cls is not SMO:
+            raise ValueError("shrinking=True is libsvm's heuristic for the SMO solver: it needs optimizer='smo'")
+        return solver_cls
+
+    def _bcqp_solver_class_of_optimizer(self):
         """The solver class to instantiate; mirrors the dispatch of ml/svm/_base.py:559-725.  A
         ``StochasticOptimizer`` subclass selects the augmented-Lagrangian relaxation (:638-723), ``'smo'`` the SMO
         solver of the problem with its equality constraint (ml/svm/smo.py)."""
@@ -163,7 +170,7 @@ class SVM(BaseEstimator):
             # on the solver
             self.obj = Quadratic(hessian, q)
             return SMO(quad=self.obj, y=eq_row, C=ub, tol=self.tol, max_iter=self.max_iter, verbose=self.verbose,
-                       active=active)
+                       active=active, shrinking=bool(getattr(self, 'shrinking', False)))
         if active is not None:
             raise ValueError("a problem on a subset of a shared matrix's rows needs optimizer='smo'")
         if issubclass(solver_cls, BoxConstrainedQuadraticOptimizer):
@@ -366,7 +373,7 @@ class SVC(ClassifierMixin, SVM):
                  intercept_scaling=1, reg_intercept=False, dual=False, optimizer=None, master_solver='clarabel',
                  learning_rate='auto', momentum_type='none', momentum=0.9, max_iter=1000, max_f_eval=15000, tol=1e-4,
                  batch_size=None, shuffle=True, random_state=None, early_stopping=False, validation_split=0.,
-                 patience=5, verbose=False, master_verbose=False):
+                 patience=5, verbose=False, master_verbose=False, shrinking=False):
         super(SVC, self).__init__(loss=loss, kernel=kernel, C=C, rho=rho, mu=mu, fit_intercept=fit_intercept,
                                   intercept_scaling=intercept_scaling, reg_intercept=reg_intercept, dual=dual,
                                   optimizer=optimizer, master_solver=master_solver, learning_rate=learning_rate,
@@ -374,7 +381,7 @@ class SVC(ClassifierMixin, SVM):
                                   max_f_eval=max_f_eval, tol=tol, batch_size=batch_size, shuffle=shuffle,
                                   random_state=random_state, early_stopping=early_stopping,
                                   validation_split=validation_split, patience=patience, verbose=verbose,
-                                  master_verbose=master_verbose)
+                                  master_verbose=master_verbose, shrinking=shrinking)
         if not getattr(loss, '_loss_type', None) == 'classifier':
             raise TypeError(f'{loss} is not an allowed SVC loss function')
         self.lb = LabelBinarizer(neg_label=-1)
@@ -460,7 +467,7 @@ class SVR(RegressorMixin, SVM):
                  fit_intercept=True, intercept_scaling=1, reg_intercept=False, dual=False, optimizer=None,
                  master_solver='clarabel', learning_rate='auto', momentum_type='none', momentum=0.9, max_iter=1000,
                  max_f_eval=15000, tol=1e-4, batch_size=None, shuffle=True, random_state=None, early_stopping=False,
-                 validation_split=0., patience=5, verbose=False, master_verbose=False):
+                 validation_split=0., patience=5, verbose=False, master_verbose=False, shrinking=False):
         super(SVR, self).__init__(loss=loss, kernel=kernel, C=C, rho=rho, mu=mu, fit_intercept=fit_intercept,
                                   intercept_scaling=intercept_scaling, reg_intercept=reg_intercept, dual=dual,
                                   optimizer=optimizer, master_solver=master_solver, learning_rate=learning_rate,
@@ -468,7 +475,7 @@ class SVR(RegressorMixin, SVM):
                                   max_f_eval=max_f_eval, tol=tol, batch_size=batch_size, shuffle=shuffle,
                                   random_state=random_state, early_stopping=early_stopping,
                                   validation_split=validation_split, patience=patience, verbose=verbose,
-                                  master_verbose=master_verbose)
+                                  master_verbose=master_verbose, shrinking=shrinking)
         if not getattr(loss, '_loss_type', None) == 'regressor':
             raise TypeError(f'{loss} is not an allowed SVR loss function')
         if not epsilon >= 0:
@@ -557,7 +564,7 @@ class DualSVC(SVC):
                  reg_intercept=True, dual=True, optimizer=ProjectedGradient, master_solver='clarabel',
                  learning_rate='auto', momentum_type='none', momentum=0.9, max_iter=1000, max_f_eval=15000, tol=1e-4,
                  batch_size=None, shuffle=True, random_state=None, early_stopping=False, validation_split=0.,
-                 patience=5, verbose=False, master_verbose=False):
+                 patience=5, verbose=False, master_verbose=False, shrinking=False):
         super(DualSVC, self).__init__(loss=loss, kernel=kernel, C=C, rho=rho, mu=mu, fit_intercept=fit_intercept,
                                       intercept_scaling=intercept_scaling, reg_intercept=reg_intercept, dual=dual,
                                       optimizer=optimizer, master_solver=master_solver, learning_rate=learning_rate,
@@ -565,7 +572,7 @@ class DualSVC(SVC):
                                       max_f_eval=max_f_eval, tol=tol, batch_size=batch_size, shuffle=shuffle,
                                       random_state=random_state, early_stopping=early_stopping,
                                       validation_split=validation_split, patience=patience, verbose=verbose,
-                                      master_verbose=master_verbose)
+                                      master_verbose=master_verbose, shrinking=shrinking)
 
 
 class DualSVR(SVR):
@@ -575,7 +582,7 @@ class DualSVR(SVR):
                  intercept_scaling=1, reg_intercept=True, dual=True, optimizer=ProjectedGradient,
                  master_solver='clarabel', learning_rate='auto', momentum_type='none', momentum=0.9, max_iter=1000,
                  max_f_eval=15000, tol=1e-4, batch_size=None, shuffle=True, random_state=None, early_stopping=False,
-                 validation_split=0., patience=5, verbose=False, master_verbose=False):
+                 validation_split=0., patience=5, verbose=False, master_verbose=False, shrinking=False):
         super(DualSVR, self).__init__(loss=loss, epsilon=epsilon, kernel=kernel, C=C, rho=rho, mu=mu,
                                       fit_intercept=fit_intercept, intercept_scaling=intercept_scaling,
                                       reg_intercept=reg_intercept, dual=dual, optimizer=optimizer,
@@ -584,4 +591,4 @@ class DualSVR(SVR):
                                       max_f_eval=max_f_eval, tol=tol, batch_size=batch_size, shuffle=shuffle,
                                       random_state=random_state, early_stopping=early_stopping,
                                       validation_split=validation_split, patience=patience, verbose=verbose,
-                                      master_verbose=master_verbose)
+                                      master_verbose=master_verbose, shrinking=shrinking)

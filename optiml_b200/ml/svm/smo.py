@@ -79,11 +79,17 @@ class SMO(DeviceLoopMixin, Optimizer):
     ``active`` (one bool per variable, on a shared signed view only): solve the problem on the active variables alone,
     every other one held at 0 (``svmb200_smo_create_subset``) -- a cross-validation fold on the matrix of a larger set of
     rows.  ``x``, ``g_x``, ``f_x`` and ``rho`` then describe the active variables only, compacted in index order, and
-    ``f_x`` and ``rho`` come from the compacted arrays, exactly as a solve of the fold's own problem computes them."""
+    ``f_x`` and ``rho`` come from the compacted arrays, exactly as a solve of the fold's own problem computes them.
+
+    ``shrinking``: libsvm's shrinking heuristic (``svmb200_smo_set_shrinking``): every min(l, 1000) states the variables
+    at a bound that cannot enter the maximal violating pair are set aside, and their G is rebuilt before the solver
+    stops.  It follows its own trajectory (csrc/k_smo.cuh).  After a run: ``active_`` (active variables after the last
+    shrink check), ``shrink_checks`` and ``reconstructions``."""
 
     _verbose_header = 'iter\t cost\t\t gap'
 
-    def __init__(self, quad, y, C, tol=1e-3, max_iter=1000, callback=None, callback_args=(), verbose=False, active=None):
+    def __init__(self, quad, y, C, tol=1e-3, max_iter=1000, callback=None, callback_args=(), verbose=False, active=None,
+                 shrinking=False):
         if not isinstance(quad, Quadratic):
             raise TypeError(f'{quad} is not an allowed quadratic function')
         n = quad.ndim
@@ -101,11 +107,22 @@ class SMO(DeviceLoopMixin, Optimizer):
             active = np.asarray(active, dtype=bool).ravel()
             if active.size != n:
                 raise ValueError('active must hold one flag per variable')
-        self.y, self.ub, self.active = y, C, active
+        self.y, self.ub, self.active, self.shrinking = y, C, active, bool(shrinking)
+        self.active_, self.shrink_checks, self.reconstructions = n, 0, 0
         self.gap, self.rho = np.nan, np.nan
         self.row_source, self.cache_slots, self.cache_hits, self.cache_misses = None, 0, 0, 0
 
     def _create(self, profile=False):
+        h, n = self._create_solver()
+        if self.shrinking:
+            try:
+                N.call('svmb200_smo_set_shrinking', h, 1)
+            except Exception:
+                N.load_library().svmb200_pg_destroy(h)
+                raise
+        return h, n
+
+    def _create_solver(self):
         H = self.f.device_hessian()
         q, y, ub = (np.ascontiguousarray(v, dtype=np.float64) for v in (self.f.q, self.y, self.ub))
         self.symmetric_pass = False
@@ -154,6 +171,9 @@ class SMO(DeviceLoopMixin, Optimizer):
         slots, hits, misses = C.c_int64(0), C.c_int64(0), C.c_int64(0)
         N.call('svmb200_smo_cache_stats', h, None, C.byref(slots), C.byref(hits), C.byref(misses))
         self.cache_slots, self.cache_hits, self.cache_misses = slots.value, hits.value, misses.value
+        active, checks, recons = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        N.call('svmb200_smo_shrink_stats', h, C.byref(active), C.byref(checks), C.byref(recons))
+        self.active_, self.shrink_checks, self.reconstructions = active.value, checks.value, recons.value
         self.gap = self._pull_state(h, n)
         cnt = C.c_int64(0)
         f_hist, gap_hist = np.empty(self.iter + 1), np.empty(self.iter + 1)
